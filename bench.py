@@ -55,6 +55,9 @@ def parse():
     ap.add_argument("--kernel", default="auto", choices=["auto", "staged", "gather", "compact"])
     ap.add_argument("--nan", default="none", choices=["none", "land", "random"],
                     help="missing values in the synthetic slab: none | land (static smooth land mask, ~35%%) | random (30%% of points)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the result of the last timed step to DIR/y.npy (rank 0; a fixed sample of its rows "
+                         "when larger than 48 MiB), so that two builds can be compared output for output")
     return ap.parse_args()
 
 
@@ -183,13 +186,30 @@ class ClockSampler:
                 "reasons": sorted(reasons), "samples": len(sm)}
 
 
+DUMP_BYTES = 48 << 20
+
+
+def dump_output(out_dir, y):
+    """--dump-outputs: ``y`` (torch tensor or numpy array) as ``out_dir/y.npy``.  An output larger
+    than DUMP_BYTES is viewed as rows of its last axis and a fixed sample of those rows (seed 0,
+    kept in order) is written as a 2-D array."""
+    import numpy as np
+    rows = y.reshape(-1, y.shape[-1])
+    k = DUMP_BYTES // (rows.shape[1] * rows.dtype.itemsize)
+    out = y
+    if k < rows.shape[0]:
+        out = rows[np.sort(np.random.default_rng(0).choice(rows.shape[0], max(1, k), replace=False))]
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "y.npy"), out.cpu().numpy() if hasattr(out, "cpu") else out)
+
+
 def cpu_port_throughput(w, n_threads, rows, reps, seed=99):
     """The reference's CPU algorithm (oracle C port: fill + COO-order loop + 3 where passes,
-    one pthread per batch chunk like dask's threaded scheduler) on `rows` batch rows."""
+    one pthread per batch chunk like dask's threaded scheduler) on `rows` batch rows.
+    Returns (points/s of the best rep, seconds of every rep, the last rep's result)."""
     import numpy as np
     from oracle import oracle as orc
     from smmregrid_b200 import synth
-    orc.build()
     n_src, n_dst = w.sizes["src_grid_size"], w.sizes["dst_grid_size"]
     mat = orc.compute_weights_matrix_c(w["src_address"], w["dst_address"], w["remap_matrix"], n_src, n_dst)
     x = synth.synthetic_field((rows, n_src), np.float32, seed=seed)
@@ -203,7 +223,7 @@ def cpu_port_throughput(w, n_threads, rows, reps, seed=99):
         dt = time.perf_counter() - t0
         times.append(dt)
         best = min(best, dt)
-    return rows * n_src / best, times
+    return rows * n_src / best, times, y
 
 
 def run_reference(args):
@@ -218,7 +238,9 @@ def run_reference(args):
     rows = max(cores, min(4 * cores, 512))
     for _ in range(args.warmup):
         cpu_port_throughput(w, cores, min(rows, cores), 1)
-    tput, times = cpu_port_throughput(w, cores, rows, max(1, args.steps))
+    tput, times, y = cpu_port_throughput(w, cores, rows, max(1, args.steps))
+    if args.dump_outputs:
+        dump_output(args.dump_outputs, y)
     n_src = w.sizes["src_grid_size"]
     ms = 1e3 * sum(times) / len(times)
     val = rows * n_src / (sum(times) / len(times))
@@ -258,6 +280,8 @@ def run_3d(args, rg, w, T, xdt, ydt, sx, sy, area_min, dev, g, world, rank, desc
     e1.record()
     torch.cuda.synchronize(dev)
     ms = e0.elapsed_time(e1) / args.steps
+    if args.dump_outputs:
+        dump_output(args.dump_outputs, y)
     infos = [rg.weights_matrix.info(l) for l in range(L)]
     nnz = sum(i["nnz"] for i in infos)
     abytes = nnz * 12 + L * ((n_dst + 1) * 4 + n_dst * 9) + T * L * (n_src * sx + n_dst * sy)
@@ -353,7 +377,7 @@ def main():
     import torch
     import torch.distributed as dist
 
-    from smmregrid_b200 import Regridder, _build, _lib
+    from smmregrid_b200 import Regridder, _lib
 
     world = int(os.environ.get("WORLD_SIZE", "1"))
     rank = int(os.environ.get("RANK", "0"))
@@ -366,10 +390,7 @@ def main():
     dev = torch.device("cuda", local)
     from smmregrid_b200.shard import bind_to_gpu_numa
     numa = bind_to_gpu_numa(local) if world > 1 else None      # host staging stays on the GPU's socket
-    if rank == 0:
-        _build.build()
-    if world > 1:
-        dist.barrier()
+    # the library is the one build() left in the tree: a run compiles nothing (the tree may be read-only)
 
     w, B_default, desc = workload(args.workload)
     B = args.batch or B_default
@@ -443,6 +464,8 @@ def main():
         dist.all_reduce(tt, op=dist.ReduceOp.MAX)
     total_ms_max = float(tt.item())
     clocks = sampler.stop(t0, t1) if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_output(args.dump_outputs, y)
 
     # ---- e2e: public API from HOST memory, H2D + D2H inside the timed region
     def all_max(v):
@@ -614,7 +637,7 @@ def main():
     if world == 1 and not args.no_cpu:
         cores = len(os.sched_getaffinity(0))
         rows = max(cores, min(2 * cores, 256))
-        tput, times = cpu_port_throughput(w, cores, rows, 3)
+        tput, times, _ = cpu_port_throughput(w, cores, rows, 3)
         cpu = {"value": tput, "unit": UNIT, "cores": cores, "kind": "port",
                "sample": f"{rows} batch rows of the same workload, best of 3 ({min(times) * 1e3:.0f} ms)"}
 
