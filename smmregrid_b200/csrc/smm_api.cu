@@ -70,6 +70,7 @@ struct smm_handle {
     size_t smem_optin = 0;
     bool ref_order = false;              // rows are summed in the reference's order (SMM_SUM_REFERENCE)
     bool cache_hit = false;              // CSR + plans were read from the on-disk plan cache
+    int gather_lanes[2] = {1, 1};        // lanes per row of fast-sum gather launches: whole levels | row lists
     std::vector<LevelDev> levels;
     // stream-ordered pool for the compact path's transposed buffer; keeps its memory between
     // applies (re-mapping ~1 GB per call cost 8 ms against 1.9 ms of kernels), freed with the handle
@@ -274,6 +275,7 @@ void plan_levels(const std::vector<HostCsr> &csrs, int64_t n_dst, int sm_count, 
         auto work = [&]() {
             for (size_t i = next.fetch_add(1); i < csrs.size() && !retry.load(); i = next.fetch_add(1)) {
                 plans[i] = HostPlan{};
+                plans[i].ref_order = ref_order;
                 if (!pc.cfg) { plans[i].why = "a destination row has more than 512 links"; continue; }
                 if (mode == kSplit) {
                     std::vector<int32_t> lrows, srows;
@@ -340,11 +342,8 @@ int build_host_operator(int32_t n_levels, const int64_t *link_length, int64_t nl
     if (use_cache) {
         cache_key = plan_cache_key(n_levels, link_length, nl_max, n_src, n_dst, src_address, dst_address,
                                    remap_matrix, num_wgts, index_base, summation, sm_count);
-        cache_hit = plan_cache_load(cache_dir, cache_key, n_levels, n_src, n_dst, csrs, plans);
-        if (cache_hit) {
-            ref_order = !plans.empty() && plans[0].ref_order;
-            return SMM_OK;
-        }
+        cache_hit = plan_cache_load(cache_dir, cache_key, n_levels, n_src, n_dst, csrs, plans, ref_order);
+        if (cache_hit) return SMM_OK;
         csrs.assign(static_cast<size_t>(n_levels), HostCsr{});
     }
     {
@@ -374,7 +373,7 @@ int build_host_operator(int32_t n_levels, const int64_t *link_length, int64_t nl
     }
     ref_order = resolve_ref_order(summation, csrs);
     plan_levels(csrs, n_dst, sm_count, ref_order, plans);
-    if (use_cache) plan_cache_store(cache_dir, cache_key, csrs, plans);   // best effort
+    if (use_cache) plan_cache_store(cache_dir, cache_key, csrs, plans, ref_order);   // best effort
     return SMM_OK;
 }
 
@@ -644,6 +643,8 @@ int launch_jobs(const smm_handle *h, const std::vector<JobSpec> &specs, int32_t 
     for (int pass = 0; pass < 2; ++pass) {
     const std::vector<JobSpec> &list = pass == 0 ? gather : gather_lists;
     const bool lists = pass == 1;
+    // reference order: one thread walks a row's links in sequence
+    const int lpr = ord ? 1 : h->gather_lanes[pass];
     for (size_t g0 = 0; g0 < list.size(); g0 += kMaxJobs) {
         const size_t g1 = std::min(list.size(), g0 + kMaxJobs);
         JobBatch jb{};
@@ -654,9 +655,6 @@ int launch_jobs(const smm_handle *h, const std::vector<JobSpec> &specs, int32_t 
             rows += lists ? L.n_gather_rows : L.n_dst;
             a.n_src = L.n_src; a.n_dst = L.n_dst;
         }
-        const double avg = rows ? static_cast<double>(nnz) / rows : 0.0;
-        // reference order: one thread walks a row's links in sequence
-        const int lpr = ord ? 1 : (avg <= 2.0 ? 1 : (avg <= 24.0 ? 4 : 32));
         const int rpb = kGatherThreads / lpr;
         auto rows_of = [&](const LevelDev &L) -> int64_t { return lists ? L.n_gather_rows : L.n_dst; };
         int64_t blocks_total = 0;
@@ -978,6 +976,19 @@ int smm_create_levels(int32_t n_levels, const int64_t *link_length, int64_t nl_m
         csrs[i] = HostCsr{};
         plans[i] = HostPlan{};
     }
+    // Lanes per row of the gather kernel, from the mean row length of the weight set's gather-family
+    // levels (of all levels when every one has a staged plan) and of the split plans' row lists.
+    // The lanes split a row's fast sum: chosen once per handle, a level's bits do not depend on
+    // which other levels share a call.
+    int64_t nnz[3] = {0, 0, 0}, rows[3] = {0, 0, 0};      // gather-family levels | staged levels | row lists
+    for (const LevelDev &L : h->levels) {
+        nnz[L.staged ? 1 : 0] += L.nnz; rows[L.staged ? 1 : 0] += L.n_dst;
+        nnz[2] += L.gather_nnz; rows[2] += L.n_gather_rows;
+    }
+    auto lanes = [](int64_t n, int64_t r) { const double avg = r ? static_cast<double>(n) / r : 0.0;
+                                            return avg <= 2.0 ? 1 : (avg <= 24.0 ? 4 : 32); };
+    h->gather_lanes[0] = rows[0] ? lanes(nnz[0], rows[0]) : lanes(nnz[1], rows[1]);
+    h->gather_lanes[1] = lanes(nnz[2], rows[2]);
     *out = h;
     return SMM_OK;
 }

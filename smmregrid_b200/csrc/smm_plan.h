@@ -99,10 +99,11 @@ PlanCacheKey plan_cache_key(int32_t n_levels, const int64_t *link_length, int64_
                             int64_t n_dst, const int32_t *src_address, const int32_t *dst_address,
                             const double *remap_matrix, int32_t num_wgts, int32_t index_base,
                             int32_t summation, int32_t sm_count);
-// false = miss (absent, stale or damaged file): build as usual
+// false = miss (absent, stale or damaged file): build as usual.  ref_order = the summation order of
+// the weight set, stored in the file as the handle's own value
 bool plan_cache_load(const std::string &dir, const PlanCacheKey &key, int32_t n_levels, int64_t n_src,
-                     int64_t n_dst, std::vector<HostCsr> &csrs, std::vector<HostPlan> &plans);
+                     int64_t n_dst, std::vector<HostCsr> &csrs, std::vector<HostPlan> &plans, bool &ref_order);
 bool plan_cache_store(const std::string &dir, const PlanCacheKey &key, std::vector<HostCsr> &csrs,
-                      std::vector<HostPlan> &plans);
+                      std::vector<HostPlan> &plans, bool ref_order);
 
 }  // namespace smm

@@ -20,7 +20,7 @@ namespace smm {
 
 namespace {
 
-constexpr char kMagic[8] = {'S', 'M', 'M', 'P', 'L', 'A', 'N', '5'};
+constexpr char kMagic[8] = {'S', 'M', 'M', 'P', 'L', 'A', 'N', '6'};
 
 // 4 interleaved 64-bit multiply-xorshift lanes over 8-byte words (a few GB/s on one core)
 struct Hasher {
@@ -137,7 +137,9 @@ PlanCacheKey plan_cache_key(int32_t n_levels, const int64_t *link_length, int64_
     hs.pod(n_levels); hs.pod(nl_max); hs.pod(n_src); hs.pod(n_dst); hs.pod(num_wgts); hs.pod(index_base);
     hs.pod(summation); hs.pod(sm_count);
     // plan-shaping experiment switches are part of the key
-    for (const char *env : {"SMM_CONSUMER_THREADS", "SMM_PACKED", "SMM_FORCE_LANES"}) hs.str(std::getenv(env));
+    for (const char *env : {"SMM_CONSUMER_THREADS", "SMM_PACKED", "SMM_FORCE_LANES", "SMM_SPLIT", "SMM_ORDLONG",
+                            "SMM_ORD_ROWS", "SMM_SUMMATION"})
+        hs.str(std::getenv(env));
     for (int32_t i = 0; i < n_levels; ++i) {
         const int64_t nl = link_length[i], o = static_cast<int64_t>(i) * nl_max;
         hs.pod(nl);
@@ -152,7 +154,7 @@ PlanCacheKey plan_cache_key(int32_t n_levels, const int64_t *link_length, int64_
 }
 
 bool plan_cache_load(const std::string &dir, const PlanCacheKey &key, int32_t n_levels, int64_t n_src,
-                     int64_t n_dst, std::vector<HostCsr> &csrs, std::vector<HostPlan> &plans)
+                     int64_t n_dst, std::vector<HostCsr> &csrs, std::vector<HostPlan> &plans, bool &ref_order)
 {
     const std::string path = cache_file(dir, key);
     FILE *f = std::fopen(path.c_str(), "rb");
@@ -163,7 +165,8 @@ bool plan_cache_load(const std::string &dir, const PlanCacheKey &key, int32_t n_
     char magic[8] = {0};
     uint64_t k0 = 0, k1 = 0;
     int32_t nl = 0;
-    rd.raw(magic, 8); rd.pod(k0); rd.pod(k1); rd.pod(nl);
+    uint8_t ord = 0;
+    rd.raw(magic, 8); rd.pod(k0); rd.pod(k1); rd.pod(nl); rd.pod(ord);
     bool good = rd.ok && std::memcmp(magic, kMagic, 8) == 0 && k0 == key.h[0] && k1 == key.h[1] && nl == n_levels;
     if (good) {
         csrs.assign(static_cast<size_t>(n_levels), HostCsr{});
@@ -186,11 +189,12 @@ bool plan_cache_load(const std::string &dir, const PlanCacheKey &key, int32_t n_
     }
     std::fclose(f);
     if (!good) { csrs.clear(); plans.clear(); }
+    else ref_order = ord != 0;
     return good;
 }
 
 bool plan_cache_store(const std::string &dir, const PlanCacheKey &key, std::vector<HostCsr> &csrs,
-                      std::vector<HostPlan> &plans)
+                      std::vector<HostPlan> &plans, bool ref_order)
 {
     ::mkdir(dir.c_str(), 0777);            // best effort; an existing directory is fine
     const std::string path = cache_file(dir, key);
@@ -201,7 +205,8 @@ bool plan_cache_store(const std::string &dir, const PlanCacheKey &key, std::vect
     wr.raw(kMagic, 8);
     wr.pod(key.h[0]); wr.pod(key.h[1]);
     const int32_t nl = static_cast<int32_t>(csrs.size());
-    wr.pod(nl);
+    const uint8_t ord = ref_order ? 1 : 0;
+    wr.pod(nl); wr.pod(ord);
     for (size_t i = 0; i < csrs.size(); ++i) {
         io_csr(wr, csrs[i]);
         io_plan(wr, plans[i]);
