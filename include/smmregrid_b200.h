@@ -37,6 +37,8 @@ extern "C" {
 
 #define SMM_F32 0
 #define SMM_F64 1
+#define SMM_I16 2           /* x_dtype only (smm_apply*): CF-packed 16-bit integers, decoded inside the */
+                            /* kernels as smm_apply_opts.decode says (smm_decode)                       */
 
 /* Which kernel family serves a level (smm_info.kernel). */
 #define SMM_KERNEL_STAGED 1 /* TMA-staged source footprint, register-resident weights     */
@@ -74,6 +76,41 @@ typedef struct smm_create_opts {
                                 /* arrays: a hit skips the host-side build (C4: 1.6 s -> 0.2 s) */
 } smm_create_opts;
 
+/*
+ * CF-packed 16-bit source data (x_dtype SMM_I16): the semantics of xarray's CF decoding
+ * (CFMaskCoder + CFScaleOffsetCoder, _choose_float_dtype) followed by the reference's apply.
+ * For a raw element r:
+ *   1. v = r read as int16, or as uint16 when is_unsigned != 0;
+ *   2. v equal to one of fill[0 .. n_fill) (_FillValue and every entry of missing_value, given in
+ *      the raw type's range; a value outside it matches nothing) -> NaN;
+ *   3. else x = D(D(v) * scale_factor) + add_offset: both operations in the decoded dtype D
+ *      (`dtype`), each rounded once, no FMA contraction.  Absent attributes: scale_factor = 1.0,
+ *      add_offset = -0.0 (x + -0.0 leaves every value, -0.0 included, unchanged, as numpy does
+ *      when it skips the addition);
+ *   4. then the reference: non-finite (including a decode that overflowed to +-inf) -> 1e20 in D,
+ *      float64 products and sums, imask / frac / `> 1e19 -> NaN`.
+ * D follows xarray's _choose_float_dtype for 16-bit integers: scale_factor and add_offset of the
+ * same type (float32 or float64): that type; only scale_factor: its type; add_offset present and
+ * types differ or scale_factor missing: float64; neither (fill values only): float32.  A Python
+ * float counts as float64; valid_min / valid_max / valid_range are ignored.
+ * smm_apply* return SMM_ERR_INVALID for SMM_I16 without decode, decode with a float x_dtype,
+ * n_fill outside [0, 4], a non-finite scale_factor or add_offset, and (dtype SMM_F32) a
+ * scale_factor or add_offset float32 cannot hold exactly.  Results are bit-identical to
+ * decoding as above on the host and applying the float path (x of dtype D) with reference-order
+ * sums (SMM_SUM_REFERENCE, or automatic with a negative weight), or when both calls run the same
+ * kernel family.  With fast sums and automatic kernel choice the two may pick different families
+ * -- 2-byte rows stage only when n_src % 8 == 0 (float32: n_src % 4 == 0), and the compact
+ * path's cost model counts the element size -- and then differ in the last bits of the sums.
+ */
+typedef struct smm_decode {
+    int32_t dtype;              /* SMM_F32 | SMM_F64: the decoded dtype D                       */
+    int32_t is_unsigned;        /* != 0: raw values are uint16 (_Unsigned = "true")             */
+    double scale_factor;        /* 1.0 when absent                                              */
+    double add_offset;          /* -0.0 when absent                                             */
+    int32_t n_fill;             /* 0..4                                                         */
+    int32_t fill[4];            /* raw values that decode to NaN                                */
+} smm_decode;
+
 /* Per-call options of smm_apply* (NULL = all defaults = zero-initialised). */
 typedef struct smm_apply_opts {
     int32_t kernel;             /* 0 = automatic, else force SMM_KERNEL_STAGED (fails if the    */
@@ -88,6 +125,7 @@ typedef struct smm_apply_opts {
                                 /* dst_grid_frac masking are unchanged and the `> 1e19 -> NaN`   */
                                 /* rule is not used (the reference has no counterpart: README.md:40) */
     double min_valid_fraction;  /* within [0, 1]; read only when renormalize != 0                */
+    const smm_decode *decode;   /* x_dtype SMM_I16 only (required there), else NULL              */
 } smm_apply_opts;
 
 typedef struct smm_info {
@@ -168,7 +206,8 @@ int smm_set_dst_mask(smm_handle *h, int32_t level, const int32_t *dst_grid_imask
 
 /*
  * Numeric core of Regridder.apply_weights (smmregrid/regrid.py:536-570) on one level:
- *   x [B, n_src] row-major with row stride ldx (elements), dtype x_dtype;
+ *   x [B, n_src] row-major with row stride ldx (elements), dtype x_dtype (SMM_I16: decoded
+ *   to its dtype D first, see smm_decode);
  *   non-finite -> 1e20 (in x's dtype), Y = X.W accumulated in float64,
  *   masked != 0:            Y[:, d] = NaN where dst_grid_imask[d] == 0     (:553-559)
  *   remap_area_min > 0:     Y[:, d] = NaN where dst_grid_frac[d] < min     (:562-565)

@@ -26,9 +26,13 @@ KERNELS = [
     ("smm_inst_f32_f64.o", "gather_kernel<float, double, 4, false>", "C5dis, few batch rows"),
     ("smm_inst_f32_f64.o", "compact_kernel<float>", "C5dis pass 1"),
     ("smm_inst_f32_f64.o", "compact_apply_kernel<float, double>", "C5dis pass 2"),
+    # CF-packed int16 sources decoded to float32 (per link: LDS.U16 + decode instead of LDS.32)
+    ("smm_inst_i16f32_f64.o", "staged_kernel<smm::I16F32, double, 8, 14, 512, false, false>", "C4, int16 -> float32"),
+    ("smm_inst_i16f32_f64.o", "staged_kernel<smm::I16F32, double, 2, 14, 512, false, false>", "C2, int16 -> float32"),
+    ("smm_inst_i16f32_f64.o", "staged_kernel<smm::I16F32, double, 1, 16, 256, true, false>", "C3, int16 -> float32"),
 ]
 MNEMONICS = ["UBLKCP", "UTMALDG", "UTMASTG", "SYNCS", "LDGSTS", "LDS", "F2F", "DFMA", "DMUL", "DADD", "IMAD", "LEA", "SHFL",
-             "STG", "LDG", "USETMAXREG"]
+             "STG", "LDG", "USETMAXREG", "FMUL", "FADD", "ISETP", "FSEL", "LOP3", "I2F"]
 
 
 def main():

@@ -14,9 +14,11 @@ _PKG = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(_PKG, "csrc")
 LIB_DIR = os.path.join(_PKG, "lib")
 LIB_PATH = os.path.join(LIB_DIR, "libsmmregrid_b200.so")
-# one translation unit per (x, y) element-type pair of the kernels, compiled in parallel
+# one translation unit per (x, y) element-type pair of the kernels (x: float32, float64, or CF-packed
+# 16 bits decoding to either), compiled in parallel
 SOURCES = ["smm_api.cu", "smm_plan.cpp", "smm_plan_cache.cpp",
-           "smm_inst_f32_f32.cu", "smm_inst_f32_f64.cu", "smm_inst_f64_f32.cu", "smm_inst_f64_f64.cu"]
+           "smm_inst_f32_f32.cu", "smm_inst_f32_f64.cu", "smm_inst_f64_f32.cu", "smm_inst_f64_f64.cu",
+           "smm_inst_i16f32_f32.cu", "smm_inst_i16f32_f64.cu", "smm_inst_i16f64_f32.cu", "smm_inst_i16f64_f64.cu"]
 HEADERS = ["smm_common.h", "smm_internal.h", "smm_kernels.cuh", "smm_launch.cuh", "smm_plan.h",
            os.path.join("..", "..", "include", "smmregrid_b200.h")]
 OBJ_DIR = os.path.join(_PKG, "build")

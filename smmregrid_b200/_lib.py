@@ -11,7 +11,7 @@ import os
 from . import _build
 
 SMM_OK, SMM_ERR_INVALID, SMM_ERR_RANGE, SMM_ERR_CUDA, SMM_ERR_ALLOC, SMM_ERR_DTYPE = range(6)
-SMM_F32, SMM_F64 = 0, 1
+SMM_F32, SMM_F64, SMM_I16 = 0, 1, 2
 SMM_KERNEL_STAGED, SMM_KERNEL_GATHER, SMM_KERNEL_COMPACT = 1, 2, 3
 KERNEL_NAMES = {SMM_KERNEL_STAGED: "staged", SMM_KERNEL_GATHER: "gather"}
 KERNEL_CODES = {None: 0, "auto": 0, "staged": SMM_KERNEL_STAGED, "gather": SMM_KERNEL_GATHER,
@@ -47,9 +47,15 @@ class SmmCreateOpts(ctypes.Structure):
     _fields_ = [("summation", i32), ("reserved", i32), ("plan_cache_dir", ctypes.c_char_p)]
 
 
+class SmmDecode(ctypes.Structure):
+    """``smm_decode``: CF unpacking of 16-bit source data (x_dtype ``SMM_I16``)."""
+    _fields_ = [("dtype", i32), ("is_unsigned", i32), ("scale_factor", f64), ("add_offset", f64),
+                ("n_fill", i32), ("fill", i32 * 4)]
+
+
 class SmmApplyOpts(ctypes.Structure):
     """``smm_apply_opts``: zero-initialised = defaults (automatic kernel, reference semantics)."""
-    _fields_ = [("kernel", i32), ("renormalize", i32), ("min_valid_fraction", f64)]
+    _fields_ = [("kernel", i32), ("renormalize", i32), ("min_valid_fraction", f64), ("decode", P(SmmDecode))]
 
 
 def create_opts(summation=None, plan_cache_dir=None):
@@ -60,14 +66,18 @@ def create_opts(summation=None, plan_cache_dir=None):
     return SmmCreateOpts(code, 0, os.fsencode(plan_cache_dir) if plan_cache_dir else None)
 
 
-def apply_opts(kernel=None, renormalize=None):
+def apply_opts(kernel=None, renormalize=None, decode=None):
     """``smm_apply_opts`` for one call (None when everything is default).  ``kernel``: None |
     'auto' | 'staged' | 'gather' | 'compact' (or the SMM_KERNEL_* code); ``renormalize``: None
-    (reference semantics) or the minimum valid weight fraction of the opt-in extension."""
+    (reference semantics) or the minimum valid weight fraction of the opt-in extension;
+    ``decode``: an ``SmmDecode`` for x_dtype ``SMM_I16`` (the options keep it alive)."""
     code = kernel if isinstance(kernel, int) else KERNEL_CODES[kernel]
-    if code == 0 and renormalize is None:
+    if code == 0 and renormalize is None and decode is None:
         return None
-    return SmmApplyOpts(code, 0 if renormalize is None else 1, 0.0 if renormalize is None else float(renormalize))
+    o = SmmApplyOpts(code, 0 if renormalize is None else 1, 0.0 if renormalize is None else float(renormalize),
+                     ctypes.pointer(decode) if decode is not None else None)
+    o._decode = decode
+    return o
 
 
 # name -> (restype, argtypes): every symbol the header declares

@@ -32,6 +32,10 @@ SMM_DECLARE_LAUNCHERS(extern, float, float)
 SMM_DECLARE_LAUNCHERS(extern, float, double)
 SMM_DECLARE_LAUNCHERS(extern, double, float)
 SMM_DECLARE_LAUNCHERS(extern, double, double)
+SMM_DECLARE_LAUNCHERS(extern, I16F32, float)
+SMM_DECLARE_LAUNCHERS(extern, I16F32, double)
+SMM_DECLARE_LAUNCHERS(extern, I16F64, float)
+SMM_DECLARE_LAUNCHERS(extern, I16F64, double)
 
 namespace {
 thread_local std::string g_err;
@@ -385,11 +389,19 @@ int env_int(const char *name, int dflt)
     return e ? std::atoi(e) : dflt;
 }
 
-#define SMM_DTYPE_DISPATCH(FN, ...)                                                    \
-    ((x_dtype == SMM_F32 && y_dtype == SMM_F32)   ? FN<float, float>(__VA_ARGS__)      \
-     : (x_dtype == SMM_F32 && y_dtype == SMM_F64) ? FN<float, double>(__VA_ARGS__)     \
-     : (x_dtype == SMM_F64 && y_dtype == SMM_F32) ? FN<double, float>(__VA_ARGS__)     \
+// (packed 16-bit x: the element type follows the decoded dtype, opt.dec_dtype)
+#define SMM_DTYPE_DISPATCH(FN, ...)                                                                           \
+    ((x_dtype == SMM_I16)                                                                                     \
+         ? ((opt.dec_dtype == SMM_F32)                                                                        \
+                ? (y_dtype == SMM_F32 ? FN<I16F32, float>(__VA_ARGS__) : FN<I16F32, double>(__VA_ARGS__))     \
+                : (y_dtype == SMM_F32 ? FN<I16F64, float>(__VA_ARGS__) : FN<I16F64, double>(__VA_ARGS__)))    \
+     : (x_dtype == SMM_F32 && y_dtype == SMM_F32) ? FN<float, float>(__VA_ARGS__)                             \
+     : (x_dtype == SMM_F32 && y_dtype == SMM_F64) ? FN<float, double>(__VA_ARGS__)                            \
+     : (x_dtype == SMM_F64 && y_dtype == SMM_F32) ? FN<double, float>(__VA_ARGS__)                            \
                                                   : FN<double, double>(__VA_ARGS__))
+
+// bytes of one x element as it sits in memory (SMM_I16: the raw 16 bits)
+size_t x_elem_bytes(int32_t x_dtype) { return x_dtype == SMM_I16 ? 2 : x_dtype == SMM_F32 ? 4 : 8; }
 
 // Batch rows per work item.  A work item pays a fixed prologue (its tile's register image,
 // barriers: `prologue_us`) and the launch pays about half an item of tail per wave, so with an
@@ -419,11 +431,40 @@ constexpr int kCompactUnavailable = -1;   // launch_compact: nothing was launche
 struct ApplyOpts {
     int kernel = 0;                 // 0 automatic | SMM_KERNEL_*
     double renorm_min_valid = -1.0; // < 0: reference semantics (fill 1e20)
+    int32_t dec_dtype = SMM_F64;    // SMM_I16 x: the decoded dtype D
+    Decode dec{};                   // SMM_I16 x: the decode parameters as the kernels read them
 };
 
-int resolve_opts(const smm_apply_opts *o, ApplyOpts &out)
+// smm_decode -> Decode, after checking it against x_dtype
+int resolve_decode(const smm_decode *d, int32_t x_dtype, ApplyOpts &out)
+{
+    if (x_dtype == SMM_I16 && !d) return fail(SMM_ERR_INVALID, "x_dtype SMM_I16 needs smm_apply_opts.decode");
+    if (!d) return SMM_OK;
+    if (x_dtype != SMM_I16) return fail(SMM_ERR_INVALID, "smm_apply_opts.decode is only valid with x_dtype SMM_I16");
+    if (d->dtype != SMM_F32 && d->dtype != SMM_F64)
+        return fail(SMM_ERR_INVALID, "smm_decode.dtype must be SMM_F32 or SMM_F64");
+    if (d->n_fill < 0 || d->n_fill > 4) return fail(SMM_ERR_INVALID, "smm_decode.n_fill must be within [0, 4]");
+    if (!std::isfinite(d->scale_factor) || !std::isfinite(d->add_offset))
+        return fail(SMM_ERR_INVALID, "smm_decode.scale_factor and add_offset must be finite");
+    const float sf = static_cast<float>(d->scale_factor), of = static_cast<float>(d->add_offset);
+    if (d->dtype == SMM_F32 && (static_cast<double>(sf) != d->scale_factor || static_cast<double>(of) != d->add_offset))
+        return fail(SMM_ERR_INVALID, "smm_decode: scale_factor and add_offset must be exact float32 values when dtype is SMM_F32");
+    out.dec_dtype = d->dtype;
+    out.dec.scale = d->scale_factor; out.dec.offset = d->add_offset;
+    out.dec.scale_f = sf; out.dec.offset_f = of;
+    out.dec.sign_xor = d->is_unsigned ? 0u : 0x8000u;
+    out.dec.bias_f = d->is_unsigned ? 8388608.0f : 8421376.0f;
+    // compared on the raw 16 bits; a value outside the raw type's range matches nothing
+    const int32_t lo = d->is_unsigned ? 0 : -32768, hi = d->is_unsigned ? 65535 : 32767;
+    for (int i = 0; i < 4; ++i)
+        out.dec.fill[i] = (i < d->n_fill && d->fill[i] >= lo && d->fill[i] <= hi) ? (d->fill[i] & 0xffff) : -1;
+    return SMM_OK;
+}
+
+int resolve_opts(const smm_apply_opts *o, int32_t x_dtype, ApplyOpts &out)
 {
     out = ApplyOpts{};
+    if (int rc = resolve_decode(o ? o->decode : nullptr, x_dtype, out)) return rc;
     if (!o) return SMM_OK;
     if (o->kernel != 0 && o->kernel != SMM_KERNEL_STAGED && o->kernel != SMM_KERNEL_GATHER &&
         o->kernel != SMM_KERNEL_COMPACT)
@@ -440,7 +481,7 @@ int resolve_opts(const smm_apply_opts *o, ApplyOpts &out)
 // Two-pass apply of one gather-family level (see compact_kernel).  The transposed buffer XT comes
 // from the handle's stream-ordered pool, so concurrent applies on other streams stay independent.
 int launch_compact(const smm_handle *h, const LevelDev &L, const JobSpec &sp, int32_t x_dtype, int32_t y_dtype,
-                   int64_t B, int64_t xbs, int64_t ybs, double area_min, cudaStream_t st)
+                   int64_t B, int64_t xbs, int64_t ybs, double area_min, const ApplyOpts &opt, cudaStream_t st)
 {
     {
         std::lock_guard<std::mutex> lock(h->pool_mu);
@@ -459,13 +500,13 @@ int launch_compact(const smm_handle *h, const LevelDev &L, const JobSpec &sp, in
         }
     }
     void *xt = nullptr;
-    const size_t sx = x_dtype == SMM_F32 ? 4 : 8;
+    const size_t sx = x_elem_bytes(x_dtype);
     const size_t xt_bytes = std::max<size_t>(static_cast<size_t>(L.touched), 1) * kCompactBC * sx;
     if (cudaMallocFromPoolAsync(&xt, xt_bytes, h->pool, st) != cudaSuccess) {
         cudaGetLastError();
         return kCompactUnavailable;                  // not enough memory for the transposed buffer
     }
-    const int rc = SMM_DTYPE_DISPATCH(launch_compact_t, h->device, L, sp, xt, B, xbs, ybs, area_min, st);
+    const int rc = SMM_DTYPE_DISPATCH(launch_compact_t, h->device, L, sp, xt, B, xbs, ybs, area_min, opt.dec, st);
     cudaFreeAsync(xt, st);
     return rc;
 }
@@ -475,7 +516,7 @@ int launch_jobs(const smm_handle *h, const std::vector<JobSpec> &specs, int32_t 
                 const ApplyOpts &opt, cudaStream_t st)
 {
     if (B == 0 || specs.empty()) return SMM_OK;
-    const size_t sx = x_dtype == SMM_F32 ? 4 : 8;
+    const size_t sx = x_elem_bytes(x_dtype);
     const bool ord = h->ref_order;
     // shared memory a staged launch needs for `nstages` stages of one batch row each (`image` = the
     // link image of ordered-long plans: kpl x nct x (8 + 4) bytes)
@@ -514,6 +555,7 @@ int launch_jobs(const smm_handle *h, const std::vector<JobSpec> &specs, int32_t 
     ApplyArgs a{};
     a.B = B; a.x_bstride = xbs; a.y_bstride = ybs; a.remap_area_min = area_min;
     a.renorm_min_valid = opt.renorm_min_valid;
+    a.dec = opt.dec;
     // experiment switches are read once per process, not per launch
     static const uint32_t k_debug_flags = static_cast<uint32_t>(env_int("SMM_DEBUG_STREAM_ONLY", 0)) & 3u;
     static const int k_max_stages = std::max(2, env_int("SMM_MAX_STAGES", kMaxStages));
@@ -632,7 +674,7 @@ int launch_jobs(const smm_handle *h, const std::vector<JobSpec> &specs, int32_t 
             bool use = L.rcol && opt.renorm_min_valid < 0.0 && opt.kernel != SMM_KERNEL_GATHER;
             if (opt.kernel != SMM_KERNEL_COMPACT) use = use && B >= 16 && gather_cost > compact_cost;
             if (!use) { plain.push_back(sp); continue; }
-            const int rc = launch_compact(h, L, sp, x_dtype, y_dtype, B, xbs, ybs, area_min, st);
+            const int rc = launch_compact(h, L, sp, x_dtype, y_dtype, B, xbs, ybs, area_min, opt, st);
             if (rc == kCompactUnavailable) { plain.push_back(sp); continue; }
             if (rc) return rc;
         }
@@ -760,8 +802,8 @@ void parallel_copy_rows(char *dst, size_t dst_stride, const char *src, size_t sr
 
 int check_dtypes(int32_t x_dtype, int32_t y_dtype)
 {
-    if ((x_dtype != SMM_F32 && x_dtype != SMM_F64) || (y_dtype != SMM_F32 && y_dtype != SMM_F64))
-        return fail(SMM_ERR_DTYPE, "dtype must be SMM_F32 (0) or SMM_F64 (1)");
+    if ((x_dtype != SMM_F32 && x_dtype != SMM_F64 && x_dtype != SMM_I16) || (y_dtype != SMM_F32 && y_dtype != SMM_F64))
+        return fail(SMM_ERR_DTYPE, "x_dtype must be SMM_F32 (0), SMM_F64 (1) or SMM_I16 (2), y_dtype SMM_F32 or SMM_F64");
     return SMM_OK;
 }
 
@@ -1133,7 +1175,7 @@ int smm_apply(const smm_handle *h, int32_t level, const void *x, int32_t x_dtype
     if (rc) return rc;
     if ((rc = check_dtypes(x_dtype, y_dtype))) return rc;
     ApplyOpts opt;
-    if ((rc = resolve_opts(opts, opt))) return rc;
+    if ((rc = resolve_opts(opts, x_dtype, opt))) return rc;
     if (B < 0) return fail(SMM_ERR_INVALID, "B must be >= 0");
     if (B == 0) return SMM_OK;
     const LevelDev &L = h->levels[level];
@@ -1157,13 +1199,13 @@ int smm_apply_levels(const smm_handle *h, int32_t n_sel, const int32_t *level_in
     int rc;
     if ((rc = check_dtypes(x_dtype, y_dtype))) return rc;
     ApplyOpts opt;
-    if ((rc = resolve_opts(opts, opt))) return rc;
+    if ((rc = resolve_opts(opts, x_dtype, opt))) return rc;
     if (n_sel < 0 || B < 0) return fail(SMM_ERR_INVALID, "n_sel and B must be >= 0");
     if (n_sel == 0 || B == 0) return SMM_OK;
     if (!level_index || !x || !y) return fail(SMM_ERR_INVALID, "null level_index, x or y");
     if (!(remap_area_min >= 0.0 && remap_area_min <= 1.0))
         return fail(SMM_ERR_INVALID, "The remap_area_min provided must be between 0.0 and 1.0");
-    const size_t sx = x_dtype == SMM_F32 ? 4 : 8, sy = y_dtype == SMM_F32 ? 4 : 8;
+    const size_t sx = x_elem_bytes(x_dtype), sy = y_dtype == SMM_F32 ? 4 : 8;
     std::vector<JobSpec> specs;
     specs.reserve(static_cast<size_t>(n_sel));
     for (int32_t i = 0; i < n_sel; ++i) {
@@ -1188,7 +1230,7 @@ int smm_apply_host(const smm_handle *hc, int32_t level, const void *x, int32_t x
     if (rc) return rc;
     if ((rc = check_dtypes(x_dtype, y_dtype))) return rc;
     ApplyOpts opt;
-    if ((rc = resolve_opts(opts, opt))) return rc;
+    if ((rc = resolve_opts(opts, x_dtype, opt))) return rc;
     if (B < 0) return fail(SMM_ERR_INVALID, "B must be >= 0");
     if (B == 0) return SMM_OK;
     if (!x || !y) return fail(SMM_ERR_INVALID, "null x or y");
@@ -1197,7 +1239,7 @@ int smm_apply_host(const smm_handle *hc, int32_t level, const void *x, int32_t x
     smm_handle *h = const_cast<smm_handle *>(hc);
     const LevelDev &L = h->levels[level];
     if (ldx < L.n_src || ldy < L.n_dst) return fail(SMM_ERR_INVALID, "ldx < n_src or ldy < n_dst");
-    const size_t sx = x_dtype == SMM_F32 ? 4 : 8, sy = y_dtype == SMM_F32 ? 4 : 8;
+    const size_t sx = x_elem_bytes(x_dtype), sy = y_dtype == SMM_F32 ? 4 : 8;
     return host_pipeline(h, x, L.n_src * sx, ldx * sx, y, L.n_dst * sy, ldy * sy, B, chunk_rows,
                          [&](void *dx, void *dy, int64_t nb, cudaStream_t st) -> int {
                              std::vector<JobSpec> specs{JobSpec{level, dx, dy, masked ? 1 : 0}};
@@ -1213,7 +1255,7 @@ int smm_apply_levels_host(const smm_handle *hc, int32_t n_sel, const int32_t *le
     int rc;
     if ((rc = check_dtypes(x_dtype, y_dtype))) return rc;
     ApplyOpts opt;
-    if ((rc = resolve_opts(opts, opt))) return rc;
+    if ((rc = resolve_opts(opts, x_dtype, opt))) return rc;
     if (n_sel < 0 || B < 0) return fail(SMM_ERR_INVALID, "n_sel and B must be >= 0");
     if (n_sel == 0 || B == 0) return SMM_OK;
     if (!level_index || !x || !y) return fail(SMM_ERR_INVALID, "null level_index, x or y");
@@ -1223,7 +1265,7 @@ int smm_apply_levels_host(const smm_handle *hc, int32_t n_sel, const int32_t *le
         if ((rc = check_level(hc, level_index[i]))) return rc;
     smm_handle *h = const_cast<smm_handle *>(hc);
     const int64_t n_src = h->levels[0].n_src, n_dst = h->levels[0].n_dst;
-    const size_t sx = x_dtype == SMM_F32 ? 4 : 8, sy = y_dtype == SMM_F32 ? 4 : 8;
+    const size_t sx = x_elem_bytes(x_dtype), sy = y_dtype == SMM_F32 ? 4 : 8;
     const size_t row_x = static_cast<size_t>(n_sel) * n_src * sx, row_y = static_cast<size_t>(n_sel) * n_dst * sy;
     return host_pipeline(h, x, row_x, row_x, y, row_y, row_y, B, chunk_rows,
                          [&](void *dx, void *dy, int64_t nb, cudaStream_t st) -> int {

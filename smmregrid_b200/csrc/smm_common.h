@@ -75,6 +75,18 @@ struct JobBatch {
     int32_t pad;
 };
 
+// CF unpacking of 16-bit raw source values (smm_decode; read by the packed element types only).
+// Raw r -> NaN if r is one of fill[] (compared on the raw 16 bits; unused slots hold -1, which no
+// zero-extended 16-bit value equals), else D(D(v) * scale) + offset with v = r as int16 (sign_xor =
+// 0x8000) or uint16 (sign_xor = 0), each operation rounded once in the decoded type D.
+struct Decode {
+    double scale, offset;       // D = float64
+    float scale_f, offset_f;    // D = float32 (exactly the doubles above)
+    int32_t fill[4];
+    uint32_t sign_xor;
+    float bias_f;               // 2^23 + (int16: 2^15 | uint16: 0), see decode16
+};
+
 struct ApplyArgs {
     int64_t B;            // batch rows per level
     int64_t x_bstride;    // elements between consecutive batch rows of x
@@ -92,6 +104,7 @@ struct ApplyArgs {
     uint32_t debug_flags; // bit 0: stream only (profiling aid: consumers skip the arithmetic)
     int32_t ord_k;        // ordered_kernel: links per row of the shared-memory image (= the plan's links per lane)
     uint32_t wimg_off, oimg_off;   // ordered_kernel: byte offsets of the weight / offset images in shared memory
+    Decode dec;           // packed 16-bit sources only (appended: the offsets of the fields above do not move)
 };
 
 }  // namespace smm

@@ -1,7 +1,7 @@
 // smm_internal.h -- declarations shared by the translation units of the library (not part of
-// the ABI).  The kernel launchers are templates over the (x, y) element types; each of the four
-// type pairs is instantiated in its own translation unit (smm_inst_*.cu) so the library builds
-// in parallel.
+// the ABI).  The kernel launchers are templates over the (x, y) element types; each of the eight
+// type pairs (x: float, double, I16F32, I16F64; y: float, double) is instantiated in its own
+// translation unit (smm_inst_*.cu) so the library builds in parallel.
 #pragma once
 #include <cuda_runtime.h>
 
@@ -54,6 +54,10 @@ struct LevelDev {
     int64_t device_bytes = 0;
 };
 
+// packed element types (smm_kernels.cuh): raw 16-bit sources decoding to float / double
+struct I16F32;
+struct I16F64;
+
 struct JobSpec {
     int32_t level;
     const void *x;
@@ -75,10 +79,11 @@ int launch_ordered_t(int dev, int rows_per_tile, int threads_per_row, dim3 grid,
 template <typename TX, typename TY>
 int launch_gather_t(int lpr, bool ord, dim3 grid, cudaStream_t st, const JobBatch &jb, const ApplyArgs &a);
 
-// the two passes of the compact path over B batch rows; `xt` holds touched x kCompactBC elements of TX
+// the two passes of the compact path over B batch rows; `xt` holds touched x kCompactBC elements of
+// what x holds (xs_t<TX>: raw 16 bits for packed sources, decoded in pass 2 with `dec`)
 template <typename TX, typename TY>
 int launch_compact_t(int dev, const LevelDev &L, const JobSpec &sp, void *xt, int64_t B, int64_t xbs,
-                     int64_t ybs, double area_min, cudaStream_t st);
+                     int64_t ybs, double area_min, const Decode &dec, cudaStream_t st);
 
 #define SMM_DECLARE_LAUNCHERS(EXTERN, TX, TY)                                                              \
     EXTERN template int launch_staged_t<TX, TY>(int, int, int, int, bool, bool, dim3, size_t, cudaStream_t, \
@@ -88,6 +93,6 @@ int launch_compact_t(int dev, const LevelDev &L, const JobSpec &sp, void *xt, in
     EXTERN template int launch_ordered_t<TX, TY>(int, int, int, dim3, size_t, cudaStream_t,                \
                                                  const JobBatch &, const ApplyArgs &);                     \
     EXTERN template int launch_compact_t<TX, TY>(int, const LevelDev &, const JobSpec &, void *, int64_t,  \
-                                                 int64_t, int64_t, double, cudaStream_t);
+                                                 int64_t, int64_t, double, const Decode &, cudaStream_t);
 
 }  // namespace smm

@@ -102,6 +102,48 @@ __device__ __forceinline__ void tma_bulk_g2s(uint32_t dst, const void *src, uint
 __device__ __forceinline__ float fill_invalid(float v) { return (fabsf(v) <= 3.402823466e+38f) ? v : 1e20f; }
 __device__ __forceinline__ double fill_invalid(double v) { return (fabs(v) <= 1.7976931348623157e+308) ? v : 1e20; }
 
+// ------------------------------------------------------------------ source element types
+//
+// TX is float, double, or a PACKED type: raw 16-bit CF-packed values (smm_decode) that every read
+// of x decodes to float (I16F32) or double (I16F64).  xs_t<TX> is what x holds in memory (staged,
+// gathered, transposed into XT), xv_t<TX> what the arithmetic sees.  For float / double every
+// helper below is exactly the plain load.
+struct I16F32 {};
+struct I16F64 {};
+template <typename TX> struct XElem { using S = TX; using V = TX; static constexpr bool kPacked = false; };
+template <> struct XElem<I16F32> { using S = uint16_t; using V = float; static constexpr bool kPacked = true; };
+template <> struct XElem<I16F64> { using S = uint16_t; using V = double; static constexpr bool kPacked = true; };
+template <typename TX> using xs_t = typename XElem<TX>::S;
+template <typename TX> using xv_t = typename XElem<TX>::V;
+
+// CF decode of one raw value (see Decode): fill values -> NaN, else (v * scale) + offset in V, each
+// operation rounded once (no FMA contraction), as numpy does it in the decoded dtype.
+template <typename V>
+__device__ __forceinline__ V decode16(uint32_t r, const Decode &d)
+{
+    // v exactly, without the (quarter-rate) integer conversion: 2^23 + (r ^ sign_xor) as float bits,
+    // minus 2^23 (+ 2^15 for int16: the xor moved the sign bit into a bias)
+    const float v = __fsub_rn(__int_as_float(static_cast<int>(0x4B000000u | (r ^ d.sign_xor))), d.bias_f);
+    V x;
+    if constexpr (sizeof(V) == 4) x = __fadd_rn(__fmul_rn(v, d.scale_f), d.offset_f);
+    else x = __dadd_rn(__dmul_rn(static_cast<double>(v), d.scale), d.offset);
+    // one predicate for the four compares (bitwise: no short-circuit, so one select below)
+    const int ri = static_cast<int>(r);
+    const bool fill = (ri == d.fill[0]) | (ri == d.fill[1]) | (ri == d.fill[2]) | (ri == d.fill[3]);
+    if constexpr (sizeof(V) == 4) return fill ? CUDART_NAN_F : x;
+    else return fill ? CUDART_NAN : x;
+}
+
+// plain (generic) read of one source element; packed types pass their Decode
+template <typename TX>
+__device__ __forceinline__ xv_t<TX> ldx_g(const xs_t<TX> *p) { return *p; }
+template <typename TX>
+__device__ __forceinline__ xv_t<TX> ldx_g(const xs_t<TX> *p, const Decode &d)
+{
+    if constexpr (XElem<TX>::kPacked) return decode16<xv_t<TX>>(*p, d);
+    else return *p;
+}
+
 // Gather load of one source element, with the smallest L2 prefetch-size hint (SASS LDG.E.LTC64B):
 // a random 4-byte gather was measured to pull 128 bytes from DRAM without it.  B200, B = 64:
 // C5dis 5.59 -> 4.98 ms, C5nn 1.43 -> 1.29 ms; the 256-byte hint costs 7 %.  SMM_GATHER_L2 = 0
@@ -134,22 +176,50 @@ template <> __device__ __forceinline__ double ld_nc<double>(const double *p)
     return __ldg(p);
 #endif
 }
+template <> __device__ __forceinline__ uint16_t ld_nc<uint16_t>(const uint16_t *p)
+{
+#if SMM_GATHER_L2 == 64
+    uint16_t v; asm volatile("ld.global.nc.L2::64B.u16 %0, [%1];" : "=h"(v) : "l"(p)); return v;
+#elif SMM_GATHER_L2 == 128
+    uint16_t v; asm volatile("ld.global.nc.L2::128B.u16 %0, [%1];" : "=h"(v) : "l"(p)); return v;
+#elif SMM_GATHER_L2 == 256
+    uint16_t v; asm volatile("ld.global.nc.L2::256B.u16 %0, [%1];" : "=h"(v) : "l"(p)); return v;
+#else
+    return __ldg(p);
+#endif
+}
+
+// gather read of one source element, decoded for packed types
+template <typename TX>
+__device__ __forceinline__ xv_t<TX> ld_nc_x(const xs_t<TX> *p, const Decode &d)
+{
+    if constexpr (XElem<TX>::kPacked) return decode16<xv_t<TX>>(ld_nc(p), d);
+    else return ld_nc(p);
+}
 
 // Reference-order evaluation of one destination row: links in ascending-src order, separate
-// multiply and add in float64 (pydata/sparse ndarray.COO loop; no FMA contraction).
-template <typename TX>
+// multiply and add in float64 (pydata/sparse ndarray.COO loop; no FMA contraction).  Packed
+// sources pass their Decode (`d`: empty for float / double).
+template <typename TX, typename... D>
 __device__ __noinline__ double replay_row(const int32_t *__restrict__ rowptr,
                                           const int32_t *__restrict__ col,
                                           const double *__restrict__ val, int row,
-                                          const TX *__restrict__ xrow)
+                                          const xs_t<TX> *__restrict__ xrow, const D &...d)
 {
     double acc = 0.0;
     const int j1 = rowptr[row + 1];
     for (int j = rowptr[row]; j < j1; ++j) {
-        const TX v = fill_invalid(xrow[col[j]]);
+        const xv_t<TX> v = fill_invalid(ldx_g<TX>(xrow + col[j], d...));
         acc = __dadd_rn(acc, __dmul_rn(static_cast<double>(v), val[j]));
     }
     return acc;
+}
+template <typename TX>
+__device__ __forceinline__ double replay(const int32_t *rowptr, const int32_t *col, const double *val, int row,
+                                         const xs_t<TX> *xrow, const Decode &d)
+{
+    if constexpr (XElem<TX>::kPacked) return replay_row<TX>(rowptr, col, val, row, xrow, d);
+    else return replay_row<TX>(rowptr, col, val, row, xrow);
 }
 
 __device__ __forceinline__ bool near_threshold(double acc) { return fabs(acc - 1e19) <= 1e10; }
@@ -214,6 +284,31 @@ template <> __device__ __forceinline__ double lds<double>(uint32_t addr)
     asm volatile("ld.shared.f64 %0, [%1];" : "=d"(v) : "r"(addr));
     return v;
 }
+template <> __device__ __forceinline__ uint16_t lds<uint16_t>(uint32_t addr)
+{
+    uint16_t v;
+    asm volatile("ld.shared.u16 %0, [%1];" : "=h"(v) : "r"(addr));
+    return v;
+}
+// an already loaded source element, decoded for packed types
+template <typename TX>
+__device__ __forceinline__ xv_t<TX> ldx_v(xs_t<TX> v) { return v; }
+template <typename TX>
+__device__ __forceinline__ xv_t<TX> ldx_v(xs_t<TX> v, const Decode &d)
+{
+    if constexpr (XElem<TX>::kPacked) return decode16<xv_t<TX>>(v, d);
+    else return v;
+}
+
+// shared-memory read of one staged source element, decoded for packed types
+template <typename TX>
+__device__ __forceinline__ xv_t<TX> ldx_s(uint32_t addr) { return lds<TX>(addr); }
+template <typename TX>
+__device__ __forceinline__ xv_t<TX> ldx_s(uint32_t addr, const Decode &d)
+{
+    if constexpr (XElem<TX>::kPacked) return decode16<xv_t<TX>>(lds<uint16_t>(addr), d);
+    else return lds<TX>(addr);
+}
 
 // Sum of one lane's register-resident links against the staged footprint at shared address
 // `sb`.  kFill = false is the fast path: raw values, no non-finite test (any NaN/inf input
@@ -238,14 +333,14 @@ __device__ __forceinline__ uint32_t pin_reg(uint32_t v)
 // `sb`.  kFill = false is the fast path: raw values, no non-finite test (any NaN/inf input
 // makes the sum non-finite, which the caller detects and redoes with kFill = true).
 template <typename TX, int KPL, bool kFill>
-__device__ __forceinline__ double lane_sum(uint32_t sb, const uint32_t (&off)[KPL], const double (&w)[KPL])
+__device__ __forceinline__ double lane_sum(uint32_t sb, const uint32_t (&off)[KPL], const double (&w)[KPL], const Decode &d)
 {
     static_assert(KPL % 2 == 0, "links per lane come in pairs");
     double acc[4] = {0.0, 0.0, 0.0, 0.0};
 #pragma unroll
     for (int k = 0; k < KPL; k += 2) {
-        TX v0 = lds<TX>(sb + off[k + 0]);
-        TX v1 = lds<TX>(sb + off[k + 1]);
+        xv_t<TX> v0 = ldx_s<TX>(sb + off[k + 0], d);
+        xv_t<TX> v1 = ldx_s<TX>(sb + off[k + 1], d);
         if (kFill) { v0 = fill_invalid(v0); v1 = fill_invalid(v1); }
         acc[k % 4 + 0] = fma(static_cast<double>(v0), w[k + 0], acc[k % 4 + 0]);
         acc[k % 4 + 1] = fma(static_cast<double>(v1), w[k + 1], acc[k % 4 + 1]);
@@ -255,14 +350,15 @@ __device__ __forceinline__ double lane_sum(uint32_t sb, const uint32_t (&off)[KP
 
 // Packed rows: a thread's 16 links are four sub-rows of four; one partial sum per sub-row.
 template <typename TX, bool kFill>
-__device__ __forceinline__ void lane_sum4(uint32_t sb, const uint32_t (&off)[16], const double (&w)[16], double (&s4)[4])
+__device__ __forceinline__ void lane_sum4(uint32_t sb, const uint32_t (&off)[16], const double (&w)[16], double (&s4)[4],
+                                          const Decode &d)
 {
 #pragma unroll
     for (int u = 0; u < 4; ++u) {
-        TX v0 = lds<TX>(sb + off[4 * u + 0]);
-        TX v1 = lds<TX>(sb + off[4 * u + 1]);
-        TX v2 = lds<TX>(sb + off[4 * u + 2]);
-        TX v3 = lds<TX>(sb + off[4 * u + 3]);
+        xv_t<TX> v0 = ldx_s<TX>(sb + off[4 * u + 0], d);
+        xv_t<TX> v1 = ldx_s<TX>(sb + off[4 * u + 1], d);
+        xv_t<TX> v2 = ldx_s<TX>(sb + off[4 * u + 2], d);
+        xv_t<TX> v3 = ldx_s<TX>(sb + off[4 * u + 3], d);
         if (kFill) { v0 = fill_invalid(v0); v1 = fill_invalid(v1); v2 = fill_invalid(v2); v3 = fill_invalid(v3); }
         const double e = fma(static_cast<double>(v1), w[4 * u + 1], static_cast<double>(v0) * w[4 * u + 0]);
         const double o = fma(static_cast<double>(v3), w[4 * u + 3], static_cast<double>(v2) * w[4 * u + 2]);
@@ -276,11 +372,11 @@ __device__ __forceinline__ void lane_sum4(uint32_t sb, const uint32_t (&off)[16]
 // products of one lane's links, each rounded once (no FMA contraction)
 template <typename TX, int KPL, bool kFill>
 __device__ __forceinline__ void lane_products(uint32_t sb, const uint32_t (&off)[KPL], const double (&w)[KPL],
-                                              double (&p)[KPL])
+                                              double (&p)[KPL], const Decode &d)
 {
 #pragma unroll
     for (int k = 0; k < KPL; ++k) {
-        TX v = lds<TX>(sb + off[k]);
+        xv_t<TX> v = ldx_s<TX>(sb + off[k], d);
         if (kFill) v = fill_invalid(v);
         p[k] = __dmul_rn(static_cast<double>(v), w[k]);
     }
@@ -311,10 +407,11 @@ __device__ __forceinline__ double ordered_group_sum(const double (&p)[KPL], int 
 }
 
 template <typename TX, int LPR, int KPL, bool kFill>
-__device__ __forceinline__ double lane_sum_ordered(uint32_t sb, const uint32_t (&off)[KPL], const double (&w)[KPL], int l_in)
+__device__ __forceinline__ double lane_sum_ordered(uint32_t sb, const uint32_t (&off)[KPL], const double (&w)[KPL], int l_in,
+                                                   const Decode &d)
 {
     double p[KPL];
-    lane_products<TX, KPL, kFill>(sb, off, w, p);
+    lane_products<TX, KPL, kFill>(sb, off, w, p, d);
     return ordered_group_sum<LPR, KPL>(p, l_in);
 }
 
@@ -322,7 +419,7 @@ __device__ __forceinline__ double lane_sum_ordered(uint32_t sb, const uint32_t (
 // (`cont` bit u: sub-row u continues the row of sub-row u-1); s4[u] = the chain after sub-row u.
 template <typename TX, bool kFill>
 __device__ __forceinline__ void lane_chain4(uint32_t sb, const uint32_t (&off)[16], const double (&w)[16], uint32_t cont,
-                                            double (&s4)[4])
+                                            double (&s4)[4], const Decode &d)
 {
     double c = 0.0;
 #pragma unroll
@@ -330,7 +427,7 @@ __device__ __forceinline__ void lane_chain4(uint32_t sb, const uint32_t (&off)[1
         c = (cont & (1u << u)) ? c : 0.0;
 #pragma unroll
         for (int j = 0; j < 4; ++j) {
-            TX v = lds<TX>(sb + off[4 * u + j]);
+            xv_t<TX> v = ldx_s<TX>(sb + off[4 * u + j], d);
             if (kFill) v = fill_invalid(v);
             c = __dadd_rn(c, __dmul_rn(static_cast<double>(v), w[4 * u + j]));
         }
@@ -343,17 +440,17 @@ __device__ __forceinline__ void lane_chain4(uint32_t sb, const uint32_t (&off)[1
 // finite x, sum of all w.
 // Kept out of line and fed from the plan arrays (not from the caller's register image) so that
 // this cold path costs the hot loop no registers.
-template <typename TX, int KPL, int NCT>
+template <typename TX, int KPL, int NCT, typename... D>
 __device__ __noinline__ void lane_sum_valid(const double *__restrict__ wplan, const uint16_t *__restrict__ iplan,
-                                            size_t base, uint32_t sb, double *out3)
+                                            size_t base, uint32_t sb, double *out3, const D &...d)
 {
     double wx = 0.0, wv = 0.0, wa = 0.0;
 #pragma unroll 2
     for (int k = 0; k < KPL; ++k) {
         const double wk = __ldg(wplan + base + static_cast<size_t>(k) * NCT);
         const uint32_t o = static_cast<uint32_t>(__ldg(iplan + base + static_cast<size_t>(k) * NCT)) *
-                           static_cast<uint32_t>(sizeof(TX));
-        const TX v = lds<TX>(sb + o);
+                           static_cast<uint32_t>(sizeof(xs_t<TX>));
+        const xv_t<TX> v = ldx_s<TX>(sb + o, d...);
         wa += wk;
         if (fill_invalid(v) == v) { wx = fma(static_cast<double>(v), wk, wx); wv += wk; }   // false for NaN, +-inf
     }
@@ -413,10 +510,10 @@ __device__ __forceinline__ void produce_stages(const LevelJob &job, const ApplyA
     if (p >= active) return;
     const uint64_t policy = l2_evict_first_policy();
     const char *xbase = static_cast<const char *>(job.x);
-    const uint32_t tile_bytes = static_cast<uint32_t>(td.elems) * sizeof(TX);
+    const uint32_t tile_bytes = static_cast<uint32_t>(td.elems) * sizeof(xs_t<TX>);
     const int NB = a.rows_per_stage;
     const int S = a.nstages;
-    const int64_t xrow_stride = a.x_bstride * static_cast<int64_t>(sizeof(TX));
+    const int64_t xrow_stride = a.x_bstride * static_cast<int64_t>(sizeof(xs_t<TX>));
     int s = 0;
     uint32_t ph = 0;
     for (int64_t g = b0; g < b1; g += NB) {          // one stage = up to NB consecutive batch rows
@@ -474,8 +571,8 @@ staged_kernel(const __grid_constant__ JobBatch jb, const __grid_constant__ Apply
 
     for (int i = tid; i < td.nseg; i += kThreads) {
         const Seg sg = job.segs[td.seg0 + i];
-        ssegs[i] = SegB{sg.dst * static_cast<uint32_t>(sizeof(TX)), sg.len * static_cast<uint32_t>(sizeof(TX)),
-                        static_cast<uint64_t>(sg.src) * sizeof(TX)};
+        ssegs[i] = SegB{sg.dst * static_cast<uint32_t>(sizeof(xs_t<TX>)), sg.len * static_cast<uint32_t>(sizeof(xs_t<TX>)),
+                        static_cast<uint64_t>(sg.src) * sizeof(xs_t<TX>)};
     }
     if (tid == 0) {
         for (int s = 0; s < S; ++s) {
@@ -509,7 +606,7 @@ staged_kernel(const __grid_constant__ JobBatch jb, const __grid_constant__ Apply
             for (int k = 0; k < KPL; ++k) {
                 w[k] = __ldg(job.wplan + base + static_cast<size_t>(k) * NCT);
                 off[k] = stages_addr + static_cast<uint32_t>(__ldg(job.iplan + base + static_cast<size_t>(k) * NCT)) *
-                                           static_cast<uint32_t>(sizeof(TX));      // address of the link in stage 0, row 0
+                                           static_cast<uint32_t>(sizeof(xs_t<TX>));      // address of the link in stage 0, row 0
             }
         }
         if constexpr (PACKED) {
@@ -534,7 +631,7 @@ staged_kernel(const __grid_constant__ JobBatch jb, const __grid_constant__ Apply
                 asm volatile("" : "+r"(dm[u]));          // opaque: kept in a register, not re-derived from `flags` per batch row
             }
             TY *yb = static_cast<TY *>(job.y) + b0 * a.y_bstride;
-            const TX *xp = static_cast<const TX *>(job.x) + b0 * a.x_bstride;
+            const xs_t<TX> *xp = static_cast<const xs_t<TX> *>(job.x) + b0 * a.x_bstride;
             const bool stream_only = (a.debug_flags & 1u) != 0;
             const int NB = a.rows_per_stage;
             bool prefer_fill = false;
@@ -553,13 +650,13 @@ staged_kernel(const __grid_constant__ JobBatch jb, const __grid_constant__ Apply
                         const bool probe = !prefer_fill || (n_done & 15u) == 0;
                         ++n_done;
                         if (probe) {
-                            if constexpr (ORD) lane_chain4<TX, false>(sb, off, w, flags, s4);
-                            else lane_sum4<TX, false>(sb, off, w, s4);
+                            if constexpr (ORD) lane_chain4<TX, false>(sb, off, w, flags, s4, a.dec);
+                            else lane_sum4<TX, false>(sb, off, w, s4, a.dec);
                             prefer_fill = __any_sync(0xffffffffu, not_finite((s4[0] + s4[1]) + (s4[2] + s4[3])));
                         }
                         if (prefer_fill) {                                          // one copy of the filled sum
-                            if constexpr (ORD) lane_chain4<TX, true>(sb, off, w, flags, s4);
-                            else lane_sum4<TX, true>(sb, off, w, s4);
+                            if constexpr (ORD) lane_chain4<TX, true>(sb, off, w, flags, s4, a.dec);
+                            else lane_sum4<TX, true>(sb, off, w, s4, a.dec);
                         }
                     }
                     if (n == nb - 1) {
@@ -590,7 +687,7 @@ staged_kernel(const __grid_constant__ JobBatch jb, const __grid_constant__ Apply
                         for (int u = 0; u < 4; ++u) {
                             if (rs[u] >= 0)
                                 store_y(yb + rs[u], finish<TY, ORD>(acc[u], (flags & (16u << u)) != 0,
-                                                                    [&]() { return replay_row<TX>(job.rowptr, job.col, job.val, rs[u], xp); }));
+                                                                    [&]() { return replay<TX>(job.rowptr, job.col, job.val, rs[u], xp, a.dec); }));
                         }
                     } else {
 #pragma unroll
@@ -613,7 +710,7 @@ staged_kernel(const __grid_constant__ JobBatch jb, const __grid_constant__ Apply
             if (a.remap_area_min > 0.0 && job.frac[row] < a.remap_area_min) dead = true;
         }
         TY *yp = static_cast<TY *>(job.y) + row + b0 * a.y_bstride;      // this row's output, batch row b
-        const TX *xp = static_cast<const TX *>(job.x) + b0 * a.x_bstride;    // source row b (replay only)
+        const xs_t<TX> *xp = static_cast<const xs_t<TX> *>(job.x) + b0 * a.x_bstride;    // source row b (replay only)
         const bool stream_only = (a.debug_flags & 1u) != 0;
 
         const int NB = a.rows_per_stage;
@@ -639,8 +736,8 @@ staged_kernel(const __grid_constant__ JobBatch jb, const __grid_constant__ Apply
                     const bool probe = !prefer_fill || (n_done & 15u) == 0;
                     ++n_done;
                     auto row_sum = [&](auto fill) -> double {        // ORD: already the whole row's sum
-                        if constexpr (ORD) return lane_sum_ordered<TX, LPR, KPL, decltype(fill)::value>(sb, off, w, l_in);
-                        else return lane_sum<TX, KPL, decltype(fill)::value>(sb, off, w);
+                        if constexpr (ORD) return lane_sum_ordered<TX, LPR, KPL, decltype(fill)::value>(sb, off, w, l_in, a.dec);
+                        else return lane_sum<TX, KPL, decltype(fill)::value>(sb, off, w, a.dec);
                     };
                     if (!probe) {
                         acc = row_sum(cuda::std::true_type{});
@@ -653,8 +750,11 @@ staged_kernel(const __grid_constant__ JobBatch jb, const __grid_constant__ Apply
                                 prefer_fill = true;
                             } else {
                                 double s3[3];
-                                lane_sum_valid<TX, KPL, NCT>(job.wplan, job.iplan,
-                                                             static_cast<size_t>(tile) * KPL * NCT + tid, stages_addr + sb, s3);
+                                const size_t base = static_cast<size_t>(tile) * KPL * NCT + tid;
+                                if constexpr (XElem<TX>::kPacked)
+                                    lane_sum_valid<TX, KPL, NCT>(job.wplan, job.iplan, base, stages_addr + sb, s3, a.dec);
+                                else
+                                    lane_sum_valid<TX, KPL, NCT>(job.wplan, job.iplan, base, stages_addr + sb, s3);
                                 acc = renormalise(group_sum<LPR>(s3[0]), group_sum<LPR>(s3[1]), group_sum<LPR>(s3[2]),
                                                   a.renorm_min_valid);
                                 renormed = true;
@@ -662,7 +762,7 @@ staged_kernel(const __grid_constant__ JobBatch jb, const __grid_constant__ Apply
                         }
                     }
                 }
-                if (n == nb - 1) {                           // last row read: the stage may be refilled
+                if (n == nb - 1) {                   // last row read: the stage may be refilled
                     __syncwarp();
                     if (lane == 0) mbar_arrive(empty_addr + 8 * s);
                 }
@@ -672,7 +772,7 @@ staged_kernel(const __grid_constant__ JobBatch jb, const __grid_constant__ Apply
                     if constexpr (!ORD) acc = group_sum<LPR>(acc);
                     if (l_in == 0 && valid && !(a.debug_flags & 2u)) {       // bit 1 (profiling aid): no stores
                         if (a.renorm_min_valid < 0.0)
-                            store_y(yp, finish<TY, ORD>(acc, dead, [&]() { return replay_row<TX>(job.rowptr, job.col, job.val, row, xp); }));
+                            store_y(yp, finish<TY, ORD>(acc, dead, [&]() { return replay<TX>(job.rowptr, job.col, job.val, row, xp, a.dec); }));
                         else
                             store_y(yp, static_cast<TY>(dead ? CUDART_NAN : acc));      // no fill, so no 1e19 rule
                     }
@@ -718,7 +818,8 @@ __device__ __forceinline__ uint32_t lds_u32(uint32_t addr)
 constexpr int kOrdUnroll = SMM_ORD_UNROLL;
 
 template <typename TX, int R, bool kFill>
-__device__ __forceinline__ void chain_pair(uint32_t wa, uint32_t oa, int K, uint32_t s0, uint32_t s1, double &a0, double &a1)
+__device__ __forceinline__ void chain_pair(uint32_t wa, uint32_t oa, int K, uint32_t s0, uint32_t s1, double &a0, double &a1,
+                                           const Decode &d)
 {
     a0 = 0.0;
     a1 = 0.0;
@@ -726,8 +827,8 @@ __device__ __forceinline__ void chain_pair(uint32_t wa, uint32_t oa, int K, uint
     for (int k = 0; k < K; ++k, wa += R * 8, oa += R * 4) {
         const double w = lds_f64(wa);
         const uint32_t o = lds_u32(oa);
-        TX v0 = lds<TX>(s0 + o);
-        TX v1 = lds<TX>(s1 + o);
+        xv_t<TX> v0 = ldx_s<TX>(s0 + o, d);
+        xv_t<TX> v1 = ldx_s<TX>(s1 + o, d);
         if (kFill) { v0 = fill_invalid(v0); v1 = fill_invalid(v1); }
         a0 = __dadd_rn(a0, __dmul_rn(static_cast<double>(v0), w));
         a1 = __dadd_rn(a1, __dmul_rn(static_cast<double>(v1), w));
@@ -735,13 +836,13 @@ __device__ __forceinline__ void chain_pair(uint32_t wa, uint32_t oa, int K, uint
 }
 
 template <typename TX, int R, bool kFill>
-__device__ __forceinline__ double chain_one(uint32_t wa, uint32_t oa, int K, uint32_t s0)
+__device__ __forceinline__ double chain_one(uint32_t wa, uint32_t oa, int K, uint32_t s0, const Decode &d)
 {
     double acc = 0.0;
 #pragma unroll kOrdUnroll
     for (int k = 0; k < K; ++k, wa += R * 8, oa += R * 4) {
         const double w = lds_f64(wa);
-        TX v = lds<TX>(s0 + lds_u32(oa));
+        xv_t<TX> v = ldx_s<TX>(s0 + lds_u32(oa), d);
         if (kFill) v = fill_invalid(v);
         acc = __dadd_rn(acc, __dmul_rn(static_cast<double>(v), w));
     }
@@ -787,12 +888,12 @@ __device__ __forceinline__ void ordered_consume_half(const LevelJob &job, const 
                 const bool probe = !prefer_fill || (n_done & 15u) == 0;
                 ++n_done;
                 if (!probe) {
-                    acc = chain_one<TX, R, true>(wa, oa, K, sb);
+                    acc = chain_one<TX, R, true>(wa, oa, K, sb, a.dec);
                 } else {
                     prefer_fill = false;
-                    acc = chain_one<TX, R, false>(wa, oa, K, sb);
+                    acc = chain_one<TX, R, false>(wa, oa, K, sb, a.dec);
                     if (__any_sync(0xffffffffu, not_finite(acc))) {
-                        acc = chain_one<TX, R, true>(wa, oa, K, sb);
+                        acc = chain_one<TX, R, true>(wa, oa, K, sb, a.dec);
                         prefer_fill = true;
                     }
                 }
@@ -837,8 +938,8 @@ ordered_kernel(const __grid_constant__ JobBatch jb, const __grid_constant__ Appl
 
     for (int i = tid; i < td.nseg; i += kThreads) {
         const Seg sg = job.segs[td.seg0 + i];
-        ssegs[i] = SegB{sg.dst * static_cast<uint32_t>(sizeof(TX)), sg.len * static_cast<uint32_t>(sizeof(TX)),
-                        static_cast<uint64_t>(sg.src) * sizeof(TX)};
+        ssegs[i] = SegB{sg.dst * static_cast<uint32_t>(sizeof(xs_t<TX>)), sg.len * static_cast<uint32_t>(sizeof(xs_t<TX>)),
+                        static_cast<uint64_t>(sg.src) * sizeof(xs_t<TX>)};
     }
     {   // the tile's link image: [K][R] weights and stage byte offsets
         const size_t ibase = static_cast<size_t>(tile) * K * R;
@@ -846,7 +947,7 @@ ordered_kernel(const __grid_constant__ JobBatch jb, const __grid_constant__ Appl
             wimg[i] = __ldg(job.wplan + ibase + i);
             // absolute shared address of the link in stage 0, row 0: what is added per batch row is a
             // pure function of the stage and row counters and stays in a uniform register
-            oimg[i] = stages_addr + static_cast<uint32_t>(__ldg(job.iplan + ibase + i)) * static_cast<uint32_t>(sizeof(TX));
+            oimg[i] = stages_addr + static_cast<uint32_t>(__ldg(job.iplan + ibase + i)) * static_cast<uint32_t>(sizeof(xs_t<TX>));
         }
     }
     if (tid == 0) {
@@ -906,12 +1007,12 @@ ordered_kernel(const __grid_constant__ JobBatch jb, const __grid_constant__ Appl
             const bool probe = !prefer_fill || (n_done & 15u) == 0;
             ++n_done;
             if (!probe) {
-                chain_pair<TX, R, true>(wa, oa, K, sb, s1, a0, a1);
+                chain_pair<TX, R, true>(wa, oa, K, sb, s1, a0, a1, a.dec);
             } else {
                 prefer_fill = false;
-                chain_pair<TX, R, false>(wa, oa, K, sb, s1, a0, a1);
+                chain_pair<TX, R, false>(wa, oa, K, sb, s1, a0, a1, a.dec);
                 if (__any_sync(0xffffffffu, not_finite(a0) || not_finite(a1))) {
-                    chain_pair<TX, R, true>(wa, oa, K, sb, s1, a0, a1);
+                    chain_pair<TX, R, true>(wa, oa, K, sb, s1, a0, a1, a.dec);
                     prefer_fill = true;
                 }
             }
@@ -962,12 +1063,12 @@ gather_kernel(const __grid_constant__ JobBatch jb, const __grid_constant__ Apply
         if (job.masked && job.imask[row] == 0) dead = true;
         if (a.remap_area_min > 0.0 && job.frac[row] < a.remap_area_min) dead = true;
     }
-    const TX *xbase = static_cast<const TX *>(job.x);
+    const xs_t<TX> *xbase = static_cast<const xs_t<TX> *>(job.x);
     TY *yrow = static_cast<TY *>(job.y) + row;
     const bool do_fill = a.renorm_min_valid < 0.0;
 
     for (int64_t b = b0; b < b1; b += BT) {
-        const TX *xr[BT];
+        const xs_t<TX> *xr[BT];
 #pragma unroll
         for (int t = 0; t < BT; ++t) {
             const int64_t bb = (b + t < b1) ? b + t : b1 - 1;
@@ -979,9 +1080,9 @@ gather_kernel(const __grid_constant__ JobBatch jb, const __grid_constant__ Apply
         for (int j = j0 + l_in; j < j1; j += LPR) {
             const int c = __ldg(job.col + j);
             const double wv = __ldg(job.val + j);
-            TX v[BT];
+            xv_t<TX> v[BT];
 #pragma unroll
-            for (int t = 0; t < BT; ++t) v[t] = ld_nc(xr[t] + c);
+            for (int t = 0; t < BT; ++t) v[t] = ld_nc_x<TX>(xr[t] + c, a.dec);
 #pragma unroll
             for (int t = 0; t < BT; ++t) {  // renormalising mode keeps raw values: a non-finite sum flags the row
                 const double xv = static_cast<double>(do_fill ? fill_invalid(v[t]) : v[t]);
@@ -1005,7 +1106,7 @@ gather_kernel(const __grid_constant__ JobBatch jb, const __grid_constant__ Apply
                     if (not_finite(r)) {
                         double wx = 0.0, wv = 0.0, wa = 0.0;
                         for (int j = j0; j < j1; ++j) {
-                            const TX v = xr[t][job.col[j]];
+                            const xv_t<TX> v = ldx_g<TX>(xr[t] + job.col[j], a.dec);
                             const double wj = job.val[j];
                             wa += wj;
                             if (fill_invalid(v) == v) { wx = fma(static_cast<double>(v), wj, wx); wv += wj; }
@@ -1022,7 +1123,7 @@ gather_kernel(const __grid_constant__ JobBatch jb, const __grid_constant__ Apply
             for (int t = 0; t < BT; ++t) {
                 if (b + t < b1)
                     yrow[(b + t) * a.y_bstride] = finish<TY, ORD>(acc[t], dead, [&]() {
-                        return replay_row<TX>(job.rowptr, job.col, job.val, row, xr[t]);
+                        return replay<TX>(job.rowptr, job.col, job.val, row, xr[t], a.dec);
                     });
             }
         }
@@ -1047,8 +1148,12 @@ constexpr int kCompactRows = 32;        // destination rows per pass-2 block
 // tcols[blk_ptr[i] .. blk_ptr[i+1]) (ascending; their rank in tcols is the row of XT).
 // The block's [bc][W] piece of the slab comes in as bc 1-D TMA bulk copies (one per batch row,
 // W * sizeof(TX) bytes each, all in flight at once, completion counted on one mbarrier) when the
-// rows are 16-byte aligned (`bulk`), else as 4-byte asynchronous element copies (LDGSTS).
+// rows are 16-byte aligned (`bulk`), else as 4-byte asynchronous element copies (LDGSTS).  Packed
+// 16-bit sources are transposed RAW (XT holds the 16-bit values; pass 2 decodes them); their
+// element copies are plain loads and stores, as cp.async has no 2-byte form.
 constexpr int kCompactStride = kCompactW + 4;       // tile row stride in elements: a multiple of 16 bytes
+// (2-byte elements: kCompactW + 8, the next stride that keeps the rows 16-byte aligned)
+__host__ __device__ constexpr int compact_stride(size_t elem_bytes) { return elem_bytes == 2 ? kCompactW + 8 : kCompactStride; }
 
 template <typename TX>
 __global__ void __launch_bounds__(kCompactThreads)
@@ -1060,7 +1165,8 @@ compact_kernel(const TX *__restrict__ x, int64_t x_bstride, int64_t n_src, int b
     __shared__ __align__(8) uint64_t bar;
     __shared__ int16_t tcol_s[kCompactW];
     static_assert(kCompactW <= 32768, "touched columns of a block are kept as 16-bit offsets");
-    TX *tile = reinterpret_cast<TX *>(smem_raw);                 // [bc][kCompactStride]
+    constexpr int kStride = compact_stride(sizeof(TX));
+    TX *tile = reinterpret_cast<TX *>(smem_raw);                 // [bc][kStride]
     const int t0 = blk_ptr[blockIdx.x], t1 = blk_ptr[blockIdx.x + 1];
     if (t0 == t1) return;                                        // nothing touched here: not read at all
     const int64_t c0 = static_cast<int64_t>(blockIdx.x) * kCompactW;
@@ -1078,7 +1184,7 @@ compact_kernel(const TX *__restrict__ x, int64_t x_bstride, int64_t n_src, int b
             if (tid == 0) mbar_arrive_expect_tx(bar_addr, static_cast<uint32_t>(bc) * w * sizeof(TX));
             const uint64_t pol = l2_evict_first_policy();
             for (int b = tid; b < bc; b += 32)
-                tma_bulk_g2s(smem_u32(tile + b * kCompactStride), x + c0 + b * x_bstride,
+                tma_bulk_g2s(smem_u32(tile + b * kStride), x + c0 + b * x_bstride,
                              static_cast<uint32_t>(w * sizeof(TX)), bar_addr, pol);
         }
     }
@@ -1093,25 +1199,34 @@ compact_kernel(const TX *__restrict__ x, int64_t x_bstride, int64_t n_src, int b
         // row (one 128-byte line per LDGSTS instruction); with fewer than 256 columns per block the
         // remaining threads take every (256 / W)-th batch row
         constexpr int kRowGroups = kCompactThreads / kCompactW > 0 ? kCompactThreads / kCompactW : 1;
-        for (int col = tid % kCompactW; col < w; col += kCompactThreads) {
-            const TX *xc = x + c0 + col;
-            const uint32_t dst0 = smem_u32(tile + col);
+        if constexpr (sizeof(TX) == 2) {
+            for (int col = tid % kCompactW; col < w; col += kCompactThreads) {
+                const TX *xc = x + c0 + col;
 #pragma unroll 8
-            for (int b = (kCompactW < kCompactThreads ? tid / kCompactW : 0); b < bc; b += kRowGroups)
-                asm volatile("cp.async.ca.shared.global [%0], [%1], %2;" ::"r"(dst0 + static_cast<uint32_t>(b * kCompactStride * sizeof(TX))),
-                             "l"(xc + b * x_bstride), "n"(sizeof(TX))
-                             : "memory");
+                for (int b = (kCompactW < kCompactThreads ? tid / kCompactW : 0); b < bc; b += kRowGroups)
+                    tile[b * kStride + col] = __ldg(xc + b * x_bstride);
+            }
+        } else {
+            for (int col = tid % kCompactW; col < w; col += kCompactThreads) {
+                const TX *xc = x + c0 + col;
+                const uint32_t dst0 = smem_u32(tile + col);
+#pragma unroll 8
+                for (int b = (kCompactW < kCompactThreads ? tid / kCompactW : 0); b < bc; b += kRowGroups)
+                    asm volatile("cp.async.ca.shared.global [%0], [%1], %2;" ::"r"(dst0 + static_cast<uint32_t>(b * kStride * sizeof(TX))),
+                                 "l"(xc + b * x_bstride), "n"(sizeof(TX))
+                                 : "memory");
+            }
+            asm volatile("cp.async.commit_group;" ::: "memory");
+            asm volatile("cp.async.wait_group 0;" ::: "memory");
         }
-        asm volatile("cp.async.commit_group;" ::: "memory");
-        asm volatile("cp.async.wait_group 0;" ::: "memory");
         __syncthreads();
     }
     const int warp = tid >> 5, lane = tid & 31;
     for (int t = t0 + warp; t < t1; t += kCompactThreads / 32) {
         const int c = tcol_s[t - t0];
         TX *dst = xt + static_cast<int64_t>(t) * kCompactBC;
-        if (lane < bc) dst[lane] = tile[lane * kCompactStride + c];
-        if (kCompactBC > 32 && lane + 32 < bc) dst[lane + 32] = tile[(lane + 32) * kCompactStride + c];
+        if (lane < bc) dst[lane] = tile[lane * kStride + c];
+        if (kCompactBC > 32 && lane + 32 < bc) dst[lane + 32] = tile[(lane + 32) * kStride + c];
     }
 }
 
@@ -1131,21 +1246,22 @@ constexpr int kCompactLinks = 1024;
 // compiler puts each value's non-finite test right behind its load and the links go one round trip
 // to memory at a time.  (XT rows are kCompactBC wide whatever bc is, slots behind the last link
 // re-read it; what lanes >= bc compute is never stored.)
-template <typename TX>
-__device__ __noinline__ double2 compact_row_filled(const TX *__restrict__ xt, const int32_t *rc, const double *vl,
-                                                   int j0, int j1, int lane)
+template <typename TX, typename... D>
+__device__ __noinline__ double2 compact_row_filled(const xs_t<TX> *__restrict__ xt, const int32_t *rc, const double *vl,
+                                                   int j0, int j1, int lane, const D &...d)
 {
+    using XS = xs_t<TX>;
     double a0 = 0.0, a1 = 0.0;
     for (int j = j0; j < j1; j += 4) {
-        TX v0[4], v1[4];
+        xv_t<TX> v0[4], v1[4];
         double w[4];
 #pragma unroll
         for (int u = 0; u < 4; ++u) {
             const int jj = j + u < j1 ? j + u : j1 - 1;
-            const TX *src = xt + static_cast<int64_t>(rc[jj]) * kCompactBC + lane;
+            const XS *src = xt + static_cast<int64_t>(rc[jj]) * kCompactBC + lane;
             w[u] = vl[jj];
-            v0[u] = __ldg(src);
-            v1[u] = kCompactBC > 32 ? __ldg(src + 32) : TX(0);
+            v0[u] = ldx_v<TX>(__ldg(src), d...);
+            v1[u] = ldx_v<TX>(kCompactBC > 32 ? __ldg(src + 32) : XS(0), d...);
         }
 #pragma unroll
         for (int u = 0; u < 4; ++u) {
@@ -1159,24 +1275,25 @@ __device__ __noinline__ double2 compact_row_filled(const TX *__restrict__ xt, co
 }
 
 template <typename TX, typename TY, bool FULL, bool STAGED, bool RAW>
-__device__ __forceinline__ void compact_rows(const TX *__restrict__ xt, int bc, const int32_t *rp, const int32_t *rc,
+__device__ __forceinline__ void compact_rows(const xs_t<TX> *__restrict__ xt, int bc, const int32_t *rp, const int32_t *rc,
                                              const double *vl, const uint8_t *dead_s, int nrows, int warp, int lane,
-                                             TY (*out)[kCompactRows + 1])
+                                             TY (*out)[kCompactRows + 1], const Decode &d)
 {
+    using XS = xs_t<TX>;
     for (int rl = warp; rl < nrows; rl += kCompactThreads / 32) {
         double a0 = 0.0, a1 = 0.0;
         const int j0 = rp[rl], j1 = rp[rl + 1];
 #pragma unroll 4
         for (int j = j0; j < j1; ++j) {
-            const TX *src = xt + static_cast<int64_t>(rc[j]) * kCompactBC + lane;
+            const XS *src = xt + static_cast<int64_t>(rc[j]) * kCompactBC + lane;
             const double wj = vl[j];
-            TX v0, v1;
+            xv_t<TX> v0, v1;
             if (FULL) {
-                v0 = __ldg(src);
-                v1 = kCompactBC > 32 ? __ldg(src + 32) : TX(0);
+                v0 = ldx_v<TX>(__ldg(src), d);
+                v1 = ldx_v<TX>(kCompactBC > 32 ? __ldg(src + 32) : XS(0), d);
             } else {
-                v0 = lane < bc ? __ldg(src) : TX(0);
-                v1 = lane + 32 < bc ? __ldg(src + 32) : TX(0);
+                v0 = ldx_v<TX>(lane < bc ? __ldg(src) : XS(0), d);
+                v1 = ldx_v<TX>(lane + 32 < bc ? __ldg(src + 32) : XS(0), d);
             }
             if (!RAW) { v0 = fill_invalid(v0); v1 = fill_invalid(v1); }
             a0 = __dadd_rn(a0, __dmul_rn(static_cast<double>(v0), wj));      // reference order, no FMA
@@ -1185,7 +1302,9 @@ __device__ __forceinline__ void compact_rows(const TX *__restrict__ xt, int bc, 
         // (a warp that remembers "the last row needed the fill" and skips the raw pass was measured:
         // it costs the clean case more than it saves the other)
         if (RAW && __any_sync(0xffffffffu, not_finite(a0) || not_finite(a1))) {
-            const double2 f = compact_row_filled<TX>(xt, rc, vl, j0, j1, lane);
+            double2 f;
+            if constexpr (XElem<TX>::kPacked) f = compact_row_filled<TX>(xt, rc, vl, j0, j1, lane, d);
+            else f = compact_row_filled<TX>(xt, rc, vl, j0, j1, lane);
             a0 = f.x;
             a1 = f.y;
         }
@@ -1199,10 +1318,11 @@ __device__ __forceinline__ void compact_rows(const TX *__restrict__ xt, int bc, 
 
 template <typename TX, typename TY>
 __global__ void __launch_bounds__(kCompactThreads, 6)       // 6 blocks per SM: the out-of-line filled row must not raise the register count
-compact_apply_kernel(const TX *__restrict__ xt, int bc, const int32_t *__restrict__ rowptr,
+compact_apply_kernel(const xs_t<TX> *__restrict__ xt, int bc, const int32_t *__restrict__ rowptr,
                      const int32_t *__restrict__ rcol, const double *__restrict__ val,
                      const int32_t *__restrict__ imask, const double *__restrict__ frac, int masked,
-                     double remap_area_min, int64_t n_dst, TY *__restrict__ y, int64_t y_bstride, int raw_first)
+                     double remap_area_min, int64_t n_dst, TY *__restrict__ y, int64_t y_bstride, int raw_first,
+                     const __grid_constant__ Decode dec)
 {
     __shared__ TY out[kCompactBC][kCompactRows + 1];
     __shared__ double val_s[kCompactLinks];
@@ -1233,13 +1353,13 @@ compact_apply_kernel(const TX *__restrict__ xt, int bc, const int32_t *__restric
     // raw_first (rows of two or more links on average): sum raw values and redo the rows that came
     // out non-finite; with one link per row the per-row work dominates and the fill stays in line
     if (staged && full && raw_first)
-        compact_rows<TX, TY, true, true, true>(xt, bc, rp, rcol_s - jb0, val_s - jb0, dead_s, nrows, warp, lane, out);
+        compact_rows<TX, TY, true, true, true>(xt, bc, rp, rcol_s - jb0, val_s - jb0, dead_s, nrows, warp, lane, out, dec);
     else if (staged && full)
-        compact_rows<TX, TY, true, true, false>(xt, bc, rp, rcol_s - jb0, val_s - jb0, dead_s, nrows, warp, lane, out);
+        compact_rows<TX, TY, true, true, false>(xt, bc, rp, rcol_s - jb0, val_s - jb0, dead_s, nrows, warp, lane, out, dec);
     else if (staged)
-        compact_rows<TX, TY, false, true, false>(xt, bc, rp, rcol_s - jb0, val_s - jb0, dead_s, nrows, warp, lane, out);
+        compact_rows<TX, TY, false, true, false>(xt, bc, rp, rcol_s - jb0, val_s - jb0, dead_s, nrows, warp, lane, out, dec);
     else
-        compact_rows<TX, TY, false, false, false>(xt, bc, rp, rcol, val, dead_s, nrows, warp, lane, out);
+        compact_rows<TX, TY, false, false, false>(xt, bc, rp, rcol, val, dead_s, nrows, warp, lane, out, dec);
     __syncthreads();
     for (int b = warp; b < bc; b += kCompactThreads / 32)
         if (lane < nrows) y[b * y_bstride + row0 + lane] = out[b][lane];

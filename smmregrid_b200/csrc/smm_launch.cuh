@@ -1,5 +1,6 @@
 // smm_launch.cuh -- definitions of the kernel launchers declared in smm_internal.h.  Included by
-// the four smm_inst_*.cu translation units only, each of which instantiates one (x, y) type pair.
+// the eight smm_inst_*.cu translation units only, each of which instantiates one (x, y) type pair
+// (x: float, double, or packed 16-bit decoding to float / double; see XElem).
 #pragma once
 #include <atomic>
 #include <cstdlib>
@@ -81,33 +82,34 @@ int launch_gather_t(int lpr, bool ord, dim3 grid, cudaStream_t st, const JobBatc
 // transpose the touched source columns into XT, then apply the links from XT.
 template <typename TX, typename TY>
 int launch_compact_t(int dev, const LevelDev &L, const JobSpec &sp, void *xt_raw, int64_t B, int64_t xbs,
-                     int64_t ybs, double area_min, cudaStream_t st)
+                     int64_t ybs, double area_min, const Decode &dec, cudaStream_t st)
 {
-    TX *xt = static_cast<TX *>(xt_raw);
-    const size_t smem = static_cast<size_t>(kCompactBC) * kCompactStride * sizeof(TX);
+    using XS = xs_t<TX>;          // pass 1 copies what x holds: packed sources stay raw in XT
+    XS *xt = static_cast<XS *>(xt_raw);
+    const size_t smem = static_cast<size_t>(kCompactBC) * compact_stride(sizeof(XS)) * sizeof(XS);
     static std::atomic<bool> optin[kMaxDevices];
     if (dev < 0 || dev >= kMaxDevices || !optin[dev].load(std::memory_order_relaxed)) {
-        CUDA_TRY(cudaFuncSetAttribute(compact_kernel<TX>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+        CUDA_TRY(cudaFuncSetAttribute(compact_kernel<XS>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                       static_cast<int>(smem)));
         if (dev >= 0 && dev < kMaxDevices) optin[dev].store(true, std::memory_order_relaxed);
     }
     const unsigned grid2 = static_cast<unsigned>((L.n_dst + kCompactRows - 1) / kCompactRows);
     // bulk (TMA) copies of the slab rows need 16-byte aligned row pieces; SMM_COMPACT_BULK=0 forces element copies
     static const bool bulk_env = [] { const char *e = getenv("SMM_COMPACT_BULK"); return !(e && e[0] == '0'); }();
-    const int bulk = bulk_env && reinterpret_cast<uintptr_t>(sp.x) % 16 == 0 && (xbs * sizeof(TX)) % 16 == 0 &&
-                     (kCompactW * sizeof(TX)) % 16 == 0;
+    const int bulk = bulk_env && reinterpret_cast<uintptr_t>(sp.x) % 16 == 0 && (xbs * sizeof(XS)) % 16 == 0 &&
+                     (kCompactW * sizeof(XS)) % 16 == 0;
     // 8-byte elements: half the batch rows per pass keeps the pass-1 tile at the size that lets three
     // blocks share an SM (one block's transposition overlaps the others' copies)
     static const int rows64 = [] { const char *e = getenv("SMM_COMPACT_F64_ROWS"); return e ? atoi(e) : 32; }();
-    const int step = (sizeof(TX) == 8 && bulk && rows64 > 0 && rows64 < kCompactBC) ? rows64 : kCompactBC;
+    const int step = (sizeof(XS) == 8 && bulk && rows64 > 0 && rows64 < kCompactBC) ? rows64 : kCompactBC;
     for (int64_t b0 = 0; b0 < B; b0 += step) {
         const int bc = static_cast<int>(B - b0 < step ? B - b0 : step);
-        compact_kernel<TX><<<static_cast<unsigned>(L.compact_blocks), kCompactThreads,
-                             static_cast<size_t>(bc) * kCompactStride * sizeof(TX), st>>>(
-            static_cast<const TX *>(sp.x) + b0 * xbs, xbs, L.n_src, bc, L.tcols, L.blk_ptr, xt, bulk);
+        compact_kernel<XS><<<static_cast<unsigned>(L.compact_blocks), kCompactThreads,
+                             static_cast<size_t>(bc) * compact_stride(sizeof(XS)) * sizeof(XS), st>>>(
+            static_cast<const XS *>(sp.x) + b0 * xbs, xbs, L.n_src, bc, L.tcols, L.blk_ptr, xt, bulk);
         compact_apply_kernel<TX, TY><<<grid2, kCompactThreads, 0, st>>>(
             xt, bc, L.rowptr, L.rcol, L.val, L.imask, L.frac, sp.masked, area_min, L.n_dst,
-            static_cast<TY *>(sp.y) + b0 * ybs, ybs, L.nnz >= 2 * L.n_dst ? 1 : 0);
+            static_cast<TY *>(sp.y) + b0 * ybs, ybs, L.nnz >= 2 * L.n_dst ? 1 : 0, dec);
         const cudaError_t e = cudaGetLastError();
         if (e != cudaSuccess) return smm_fail(3, std::string("compact apply: ") + cudaGetErrorString(e));
         smm_count_launches(2);

@@ -143,6 +143,12 @@ class Variable:
             out += np.float64(offset)
         return out
 
+    def packing(self):
+        """``CFPacking`` of this variable (None when it is not packed), so that its raw values are
+        decoded inside the kernels: ``rg.regrid(var.read(), packing=var.packing())``."""
+        from .packing import CFPacking
+        return CFPacking.from_attrs(self.attrs, self.dtype)
+
     def __array__(self, dtype=None, copy=None):
         a = self.read()
         return a.astype(dtype) if dtype is not None else a

@@ -24,6 +24,10 @@ Data may be
 The numeric core always runs in the sm_100a kernels through the C ABI; there is no CPU path.
 Everything that varies per call (kernel family, the renormalising extension) travels as an
 argument of the C call (``smm_apply_opts``), never as state of the shared device handle.
+
+CF-packed 16-bit data (``packing=``, see ``packing.CFPacking``) reaches the kernels raw and is
+decoded there: a ``CFPacking`` for arrays and tensors, ``"cf"`` to take it from each variable's own
+attributes (as opened with ``mask_and_scale=False``).
 """
 from __future__ import annotations
 
@@ -35,6 +39,7 @@ from typing import Optional, Sequence
 import numpy as np
 
 from . import _lib
+from .packing import PACKING_ATTRS, RAW_DTYPES, CFPacking
 from .weights import (CdoWeights, WeightsMatrix, check_mask, compute_weights_matrix,
                       compute_weights_matrix3d, mask_weights, _device_index)
 
@@ -291,8 +296,12 @@ class Regridder(object):
 
     # ------------------------------------------------------------------ public API
 
-    def regrid(self, source_data, level_axis: Optional[int] = None, levels: Optional[Sequence[float]] = None):
-        """Regrid an array / DataArray / Dataset (reference: ``regrid.py:233-271``)."""
+    def regrid(self, source_data, level_axis: Optional[int] = None, levels: Optional[Sequence[float]] = None,
+               packing=None):
+        """Regrid an array / DataArray / Dataset (reference: ``regrid.py:233-271``).  ``packing``:
+        None, a ``CFPacking`` (raw int16 / uint16 data decoded in the kernels) or ``"cf"`` (each
+        DataArray / Dataset variable's packing from its own attributes; unpacked variables as
+        without it)."""
         if _is_dataset(source_data):
             # the reference refuses data on several grids when initialised from weights (regrid.py:253-259)
             grids = []
@@ -304,13 +313,19 @@ class Regridder(object):
                     grids.append(key)
             if len(grids) > 1 and self.init_mode == 'weights':
                 raise ValueError(f'Cannot process data with {len(grids)} GridType initializing from weights')
-            out = source_data.map(self.regrid_array, keep_attrs=True)
+            out = source_data.map(lambda v: self.regrid_array(v, packing=packing), keep_attrs=True)
             degen = [v for v in out.data_vars if out[v].dims == ()]      # regrid.py:265-266
-            return out.drop_vars(degen)
+            out = out.drop_vars(degen)
+            if packing is not None:           # (keep_attrs copies the packed variables' attributes back)
+                for name in out.data_vars:
+                    if _packing_of(source_data[name], packing) is not None:
+                        for k in PACKING_ATTRS:
+                            out[name].attrs.pop(k, None)
+            return out
         if _is_dataarray(source_data):
-            return self.regrid_array(source_data)
+            return self.regrid_array(source_data, packing=packing)
         if isinstance(source_data, np.ndarray) or _is_tensor(source_data):
-            return self.regrid_array(source_data, level_axis=level_axis, levels=levels)
+            return self.regrid_array(source_data, level_axis=level_axis, levels=levels, packing=packing)
         if isinstance(source_data, dict):
             # plain-array counterpart of Dataset.map (regrid.py:262): one entry per variable;
             # bounds variables are dropped except time bounds (regrid.py:482-490)
@@ -320,35 +335,36 @@ class Regridder(object):
                     if 'time' in str(name):
                         out[name] = arr
                     continue
-                out[name] = self.regrid_array(arr, level_axis=level_axis, levels=levels)
+                out[name] = self.regrid_array(arr, level_axis=level_axis, levels=levels, packing=packing)
             return out
         raise TypeError('The object provided is not a Xarray object!')
 
-    def regrid_array(self, source_data, level_axis=None, levels=None):
+    def regrid_array(self, source_data, level_axis=None, levels=None, packing=None):
         """2-D or 3-D dispatch on the presence of ``mask_dim`` (reference: ``regrid.py:273-312``)."""
         if _is_dataarray(source_data):
-            return self._regrid_dataarray(source_data)
+            return self._regrid_dataarray(source_data, packing)
         if self.mask_dim:
-            return self.regrid3d(source_data, level_axis=level_axis, levels=levels)
-        return self.regrid2d(source_data)
+            return self.regrid3d(source_data, level_axis=level_axis, levels=levels, packing=packing)
+        return self.regrid2d(source_data, packing=packing)
 
-    def regrid2d(self, source_data, datagridtype=None):
+    def regrid2d(self, source_data, datagridtype=None, packing=None):
         """Single apply with the 2-D operator (reference: ``regrid.py:429-456``)."""
         if _is_dataarray(source_data):
-            return self._regrid_dataarray(source_data)
+            return self._regrid_dataarray(source_data, packing)
         return self.apply_weights(source_data, self.weights, weights_matrix=self.weights_matrix,
-                                  masked=self.masked)
+                                  masked=self.masked, packing=packing)
 
-    def regrid3d(self, source_data, datagridtype=None, level_axis=None, levels=None, out=None, transpose=None):
+    def regrid3d(self, source_data, datagridtype=None, level_axis=None, levels=None, out=None, transpose=None,
+                 packing=None):
         """Per-level apply for level-varying masks (reference: ``regrid.py:339-427``), issued as
         one grouped launch that writes every level at its final position.  ``transpose``
         overrides ``self.transpose`` for this call; ``out`` (host data only): contiguous numpy
         array that receives the ``[kept..., L, tgt...]`` result."""
         if _is_dataarray(source_data):
-            return self._regrid_dataarray(source_data)
+            return self._regrid_dataarray(source_data, packing)
         torch = _torch()
         transpose = self.transpose if transpose is None else bool(transpose)
-        source_data = self._floating(source_data)
+        source_data, opts = self._source(source_data, packing)
         nh = self._n_horizontal_axes(source_data.shape)
         nkept = source_data.ndim - nh
         if nkept < 1:
@@ -366,7 +382,6 @@ class Regridder(object):
             raise ValueError("levels must have one value per data level")
         widx = np.array([select_level(wl, lev, self.mask_dim) for lev in levels], dtype=np.int32)
         masked = np.ascontiguousarray(np.asarray(self.masked)[widx], dtype=np.uint8)
-        opts = _lib.apply_opts(self.kernel, self.renormalize)
 
         was_numpy = isinstance(source_data, np.ndarray)
         x = torch.from_numpy(np.ascontiguousarray(source_data)) if was_numpy else source_data
@@ -391,7 +406,7 @@ class Regridder(object):
             stream = torch.cuda.current_stream(dev).cuda_stream
             _lib.check(lib.smm_apply_levels(
                 self.weights_matrix.handle, Ld, widx.ctypes.data_as(ctypes.c_void_p),
-                ctypes.c_void_p(x.data_ptr()), _np_dtype_code(_np_of(x.dtype)), T,
+                ctypes.c_void_p(x.data_ptr()), _x_code(x.dtype), T,
                 Ld * self.n_src, self.n_src,
                 ctypes.c_void_p(y.data_ptr()), _np_dtype_code(_np_of(y.dtype)), ybs, yls,
                 masked.ctypes.data_as(ctypes.c_void_p), self.remap_area_min, opts, ctypes.c_void_p(stream)))
@@ -421,7 +436,7 @@ class Regridder(object):
                 y = torch.from_numpy(_new_host_result((T, Ld, self.n_dst), self._out_np_dtype()))
         _lib.check(_lib.load().smm_apply_levels_host(
             self.weights_matrix.handle, Ld, widx.ctypes.data_as(ctypes.c_void_p),
-            ctypes.c_void_p(x.data_ptr()), _np_dtype_code(_np_of(x.dtype)), T,
+            ctypes.c_void_p(x.data_ptr()), _x_code(x.dtype), T,
             ctypes.c_void_p(y.data_ptr()), _np_dtype_code(_np_of(y.dtype)),
             masked.ctypes.data_as(ctypes.c_void_p), self.remap_area_min, opts, 0))
         if out is not None:
@@ -433,23 +448,23 @@ class Regridder(object):
         return y.numpy() if was_numpy else y
 
     def apply_weights(self, source_data, weights=None, weights_matrix=None, masked=True,
-                      horizontal_dims=None, level: int = 0, out=None):
+                      horizontal_dims=None, level: int = 0, out=None, packing=None):
         """Numeric core of the reference's ``apply_weights`` (``regrid.py:536-584``):
         reshape to ``[kept, n_src]``, non-finite -> 1e20, sparse matmul, destination mask,
         ``dst_grid_frac < remap_area_min``, ``> 1e19 -> NaN``, reshape to the target grid.
-        ``out`` (host data only): numpy array of the result's size to write into."""
+        ``out`` (host data only): numpy array of the result's size to write into.  ``packing``: a
+        ``CFPacking`` for raw int16 / uint16 data (decoded in the kernels)."""
         if _is_dataarray(source_data):
-            return self._regrid_dataarray(source_data)
+            return self._regrid_dataarray(source_data, packing)
         torch = _torch()
         wm = weights_matrix if weights_matrix is not None else self.weights_matrix
         parent, lvl = (wm.parent, wm.level) if hasattr(wm, "parent") else (wm, level)
-        source_data = self._floating(source_data)
+        source_data, opts = self._source(source_data, packing)
         nh = self._n_horizontal_axes(source_data.shape)
         kept_shape = tuple(source_data.shape[:source_data.ndim - nh])
         B = int(np.prod(kept_shape)) if kept_shape else 1
         lib = _lib.load()
         masked = 1 if bool(masked) else 0
-        opts = _lib.apply_opts(self.kernel, self.renormalize)
 
         if isinstance(source_data, np.ndarray) or not source_data.is_cuda:
             # host data: chunked H2D -> kernel -> D2H pipeline inside the library
@@ -468,7 +483,7 @@ class Regridder(object):
                 if y is None:
                     y = torch.from_numpy(_new_host_result((B, self.n_dst), self._out_np_dtype()))
             _lib.check(lib.smm_apply_host(
-                parent.handle, lvl, ctypes.c_void_p(xt.data_ptr()), _np_dtype_code(_np_of(xt.dtype)), B,
+                parent.handle, lvl, ctypes.c_void_p(xt.data_ptr()), _x_code(xt.dtype), B,
                 self.n_src, ctypes.c_void_p(y.data_ptr()), _np_dtype_code(_np_of(y.dtype)), self.n_dst,
                 masked, self.remap_area_min, opts, 0))
             if out is not None:
@@ -484,12 +499,30 @@ class Regridder(object):
         with torch.cuda.device(dev):
             stream = torch.cuda.current_stream(dev).cuda_stream
             _lib.check(lib.smm_apply(
-                parent.handle, lvl, ctypes.c_void_p(x.data_ptr()), _np_dtype_code(_np_of(x.dtype)), B,
+                parent.handle, lvl, ctypes.c_void_p(x.data_ptr()), _x_code(x.dtype), B,
                 self.n_src, ctypes.c_void_p(y.data_ptr()), _np_dtype_code(_np_of(y.dtype)), self.n_dst,
                 masked, self.remap_area_min, opts, ctypes.c_void_p(stream)))
         return y.reshape(kept_shape + self.tgt_shape)
 
     # ------------------------------------------------------------------ helpers
+
+    def _source(self, data, packing):
+        """The data as the kernels read it and the options of the call: floating-point data
+        (``_floating``), or with a ``CFPacking`` the raw 16 bits (as int16: the packing says how
+        they read) and the options that decode them."""
+        if packing is None:
+            return self._floating(data), _lib.apply_opts(self.kernel, self.renormalize)
+        if isinstance(packing, str):
+            raise ValueError('packing="cf" reads the attributes of a DataArray / Dataset variable; '
+                             'pass a CFPacking with array data')
+        if not isinstance(packing, CFPacking):
+            raise TypeError(f"packing must be None, 'cf' or a CFPacking, got {type(packing).__name__}")
+        if isinstance(data, np.ndarray) and data.dtype in RAW_DTYPES:
+            data = data.view(np.int16)
+        elif not (_is_tensor(data) and data.dtype == _torch().int16):
+            raise TypeError(f"packed data must be a numpy int16 / uint16 array or a torch int16 tensor, "
+                            f"got {getattr(data, 'dtype', type(data).__name__)}")
+        return data, _lib.apply_opts(self.kernel, self.renormalize, packing.to_c())
 
     def _floating(self, data):
         """The reference computes in ``result_type(data, float64 weights)``: integer and bool
@@ -547,9 +580,10 @@ class Regridder(object):
             raise ValueError(f'Only one masked dimension can be processed at the time: check {mask}')
         return frozenset(hor + mask)
 
-    def _regrid_dataarray(self, da):
+    def _regrid_dataarray(self, da, packing=None):
         """``regrid_array`` + ``regrid2d`` / ``regrid3d`` + the xarray side of ``apply_weights``
         (``regrid.py:273-312, 339-456, 476-626``) for one variable."""
+        packing = _packing_of(da, packing)
         name = "" if da.name is None else str(da.name)
         cls = type(da)
         scalars = [k for k, c in da.coords.items() if c.dims == ()]          # regrid.py:289-295
@@ -599,45 +633,48 @@ class Regridder(object):
         # `.chunks` is None unless the variable is dask-backed; `.data` of a lazily indexed backend
         # array would load the whole field, so it is only touched for dask
         if getattr(da, "chunks", None):
-            values = self._dask_apply(da.data, len(horizontal), levels, out_dt)
+            values = self._dask_apply(da.data, len(horizontal), levels, out_dt, packing)
         else:
-            values = self._stream_blocks(da, other, lev_dim, levels, kept_shape, out_dt)
+            values = self._stream_blocks(da, other, lev_dim, levels, kept_shape, out_dt, packing)
         out_dims = kept_canon
         if lev_dim and not self.transpose:             # level axis first, as xarray.concat leaves it (regrid.py:410)
             values = _moveaxis(values, len(other), 0)
             out_dims = [lev_dim] + other
-        return self._dress(cls, da, values, out_dims)
+        return self._dress(cls, da, values, out_dims, drop_packing=packing is not None)
 
-    def _block_apply(self, block, levels, out=None):
+    def _block_apply(self, block, levels, out=None, packing=None):
         """numeric core on one host block laid out ``[other..., (lev,) horizontal...]``; returns /
         fills ``[other..., (lev,) tgt...]``."""
-        block = self._floating(np.asarray(block))
+        block = np.asarray(block)
+        if packing is None:
+            block = self._floating(block)
         n_kept = block.ndim - self._n_horizontal_axes(block.shape)
         if levels is not None:     # level axis last among the kept ones; the caller moves it if asked to
-            res = self.regrid3d(block, level_axis=n_kept - 1, levels=levels, out=out, transpose=True)
+            res = self.regrid3d(block, level_axis=n_kept - 1, levels=levels, out=out, transpose=True, packing=packing)
         else:
-            res = self.apply_weights(block, self.weights, weights_matrix=self.weights_matrix, masked=self.masked, out=out)
+            res = self.apply_weights(block, self.weights, weights_matrix=self.weights_matrix, masked=self.masked, out=out,
+                                     packing=packing)
         if out is not None:
             return out
         return np.asarray(res).reshape(block.shape[:n_kept] + self.tgt_shape)
 
-    def _stream_blocks(self, da, other, lev_dim, levels, kept_shape, out_dt):
+    def _stream_blocks(self, da, other, lev_dim, levels, kept_shape, out_dt, packing=None):
         """Host-backed (numpy or lazily indexed) data: blocks of the leading kept dim are read,
         pushed through the device pipeline and written straight into the result, so no more than
         ``host_block_bytes`` of the source is ever held (``regrid.py:538-550`` keeps the field lazy)."""
         out = _new_host_result(kept_shape + self.tgt_shape, out_dt)
         if not other or da.shape[0] <= 1:
-            self._block_apply(da.values, levels, out=out)
+            self._block_apply(da.values, levels, out=out, packing=packing)
             return out
         lead, n_lead = other[0], da.shape[0]
         row_bytes = max(1, int(np.prod(da.shape[1:])) * np.dtype(da.dtype).itemsize)
         step = int(max(1, min(n_lead, self.host_block_bytes // row_bytes)))
         for a in range(0, n_lead, step):
             b = min(n_lead, a + step)
-            self._block_apply(da.isel({lead: slice(a, b)}).values, levels, out=out[a:b])
+            self._block_apply(da.isel({lead: slice(a, b)}).values, levels, out=out[a:b], packing=packing)
         return out
 
-    def _dask_apply(self, data, n_hor, levels, out_dt):
+    def _dask_apply(self, data, n_hor, levels, out_dt, packing=None):
         """dask-backed data stays lazy: one ``map_blocks`` task per chunk of the kept dims, each
         feeding the device pipeline (the handle is shared read-only by the worker threads)."""
         import dask.array as dka
@@ -647,14 +684,15 @@ class Regridder(object):
         hor_axes = list(range(nd - n_hor, nd))
         new_axes = list(range(nd - n_hor, nd - n_hor + len(self.tgt_shape)))
         chunks = tuple(data.chunks[:nd - n_hor]) + tuple((n,) for n in self.tgt_shape)
-        return dka.map_blocks(lambda blk: self._block_apply(blk, levels).astype(out_dt, copy=False), data,
+        return dka.map_blocks(lambda blk: self._block_apply(blk, levels, packing=packing).astype(out_dt, copy=False), data,
                               dtype=out_dt, chunks=chunks, drop_axis=hor_axes, new_axis=new_axes,
                               meta=np.empty((0,) * (nd - n_hor + len(self.tgt_shape)), dtype=out_dt))
 
-    def _dress(self, cls, da, values, kept_dims):
+    def _dress(self, cls, da, values, kept_dims, drop_packing=False):
         """Output DataArray of ``apply_weights`` (``regrid.py:586-626``): kept coordinates, target
         lat/lon (degrees, rounded; degenerate axes removed), ``i/j -> lat/lon`` for regular
-        targets, coordinate and variable attributes."""
+        targets, coordinate and variable attributes (``drop_packing``: without the CF packing
+        attributes, which xarray moves to ``.encoding`` when it decodes)."""
         w = self.weights
         tgt_dims = list(self.tgt_dims)
         coords = {k: v for k, v in da.coords.items() if set(v.dims).issubset(kept_dims)}
@@ -677,6 +715,9 @@ class Regridder(object):
             coords[key] = (tuple(dims), vals, attrs)
         attrs = dict(da.attrs)
         attrs.pop('CDI_grid_type', None)               # regrid.py:624
+        if drop_packing:
+            for k in PACKING_ATTRS:
+                attrs.pop(k, None)
         return cls(values, dims=list(kept_dims) + tgt_dims, coords=coords, name=da.name, attrs=attrs)
 
 
@@ -699,6 +740,23 @@ def _is_tensor(obj) -> bool:
         return isinstance(obj, _torch().Tensor)
     except ImportError:
         return False
+
+
+def _packing_of(da, packing):
+    """CFPacking of one DataArray: ``packing`` itself, or from its attributes for ``"cf"``."""
+    if isinstance(packing, str):
+        if packing != "cf":
+            raise ValueError(f"packing must be None, 'cf' or a CFPacking, got {packing!r}")
+        return CFPacking.from_attrs(da.attrs, da.dtype)
+    return packing
+
+
+def _x_code(torch_dtype) -> int:
+    """x_dtype code of the tensor handed to the library (int16: raw CF-packed values, which only
+    ``Regridder._source`` lets through)."""
+    if torch_dtype == _torch().int16:
+        return _lib.SMM_I16
+    return _np_dtype_code(_np_of(torch_dtype))
 
 
 def _np_of(torch_dtype):
