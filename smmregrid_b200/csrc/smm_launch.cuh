@@ -2,13 +2,37 @@
 // the eight smm_inst_*.cu translation units only, each of which instantiates one (x, y) type pair
 // (x: float, double, or packed 16-bit decoding to float / double; see XElem).
 #pragma once
+#include <algorithm>
 #include <atomic>
 #include <cstdlib>
+#include <mutex>
 
 #include "smm_internal.h"
 #include "smm_kernels.cuh"
 
 namespace smm {
+
+// The dynamic shared memory a kernel may use is process-wide state of the kernel on the current
+// device, shared by every thread that launches it, and launches of one kernel need different sizes
+// (the stage count and rows per stage follow B).  So the attribute is only ever raised, to the
+// largest size asked for so far, under a lock: a caller that set a smaller size after another had
+// raised it would make the other's launch fail.  optin[dev] is that high-water mark, read without
+// the lock by launches that need no more; devices beyond kMaxDevices go through the lock each time.
+template <typename Kernel>
+int raise_smem_optin(Kernel kfn, std::atomic<size_t> (&optin)[kMaxDevices], int dev, size_t smem)
+{
+    const bool tracked = dev >= 0 && dev < kMaxDevices;
+    if (tracked && optin[dev].load(std::memory_order_acquire) >= smem) return 0;
+    static std::mutex mu;
+    std::lock_guard<std::mutex> lock(mu);
+    cudaFuncAttributes fa;
+    CUDA_TRY(cudaFuncGetAttributes(&fa, kfn));
+    const size_t have = static_cast<size_t>(fa.maxDynamicSharedSizeBytes);
+    if (have < smem)
+        CUDA_TRY(cudaFuncSetAttribute(kfn, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
+    if (tracked) optin[dev].store(std::max(have, smem), std::memory_order_release);
+    return 0;
+}
 
 template <typename TX, typename TY>
 int launch_staged_t(int dev, int lpr, int kpl, int nct, bool packed, bool ord, dim3 grid, size_t smem,
@@ -17,13 +41,8 @@ int launch_staged_t(int dev, int lpr, int kpl, int nct, bool packed, bool ord, d
 #define SMM_CASE_PO(L_, K_, N_, P_, O_)                                                           \
     if (lpr == L_ && kpl == K_ && nct == N_ && packed == P_ && ord == O_) {                       \
         auto kfn = staged_kernel<TX, TY, L_, K_, N_, P_, O_>;                                     \
-        /* the opt-in is per kernel and device: raise it only when a launch needs more */         \
         static std::atomic<size_t> optin[kMaxDevices];                                            \
-        if (dev < 0 || dev >= kMaxDevices || optin[dev].load(std::memory_order_relaxed) < smem) { \
-            CUDA_TRY(cudaFuncSetAttribute(kfn, cudaFuncAttributeMaxDynamicSharedMemorySize,       \
-                                          static_cast<int>(smem)));                               \
-            if (dev >= 0 && dev < kMaxDevices) optin[dev].store(smem, std::memory_order_relaxed); \
-        }                                                                                         \
+        if (const int rc = raise_smem_optin(kfn, optin, dev, smem)) return rc;                    \
         kfn<<<grid, N_ + 32 * producer_warps(N_), smem, st>>>(jb, a);                             \
         CUDA_TRY(cudaGetLastError());                                                             \
         smm_count_launches(1);                                                                    \
@@ -49,11 +68,7 @@ int launch_ordered_t(int dev, int rows_per_tile, int threads_per_row, dim3 grid,
     if (rows_per_tile == R_ && threads_per_row == T_) {                                           \
         auto kfn = ordered_kernel<TX, TY, R_, T_>;                                                \
         static std::atomic<size_t> optin[kMaxDevices];                                            \
-        if (dev < 0 || dev >= kMaxDevices || optin[dev].load(std::memory_order_relaxed) < smem) { \
-            CUDA_TRY(cudaFuncSetAttribute(kfn, cudaFuncAttributeMaxDynamicSharedMemorySize,       \
-                                          static_cast<int>(smem)));                               \
-            if (dev >= 0 && dev < kMaxDevices) optin[dev].store(smem, std::memory_order_relaxed); \
-        }                                                                                         \
+        if (const int rc = raise_smem_optin(kfn, optin, dev, smem)) return rc;                    \
         kfn<<<grid, R_ * T_ + 32 * kOrderedProducerWarps, smem, st>>>(jb, a);                     \
         CUDA_TRY(cudaGetLastError());                                                             \
         smm_count_launches(1);                                                                    \
@@ -87,12 +102,8 @@ int launch_compact_t(int dev, const LevelDev &L, const JobSpec &sp, void *xt_raw
     using XS = xs_t<TX>;          // pass 1 copies what x holds: packed sources stay raw in XT
     XS *xt = static_cast<XS *>(xt_raw);
     const size_t smem = static_cast<size_t>(kCompactBC) * compact_stride(sizeof(XS)) * sizeof(XS);
-    static std::atomic<bool> optin[kMaxDevices];
-    if (dev < 0 || dev >= kMaxDevices || !optin[dev].load(std::memory_order_relaxed)) {
-        CUDA_TRY(cudaFuncSetAttribute(compact_kernel<XS>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                      static_cast<int>(smem)));
-        if (dev >= 0 && dev < kMaxDevices) optin[dev].store(true, std::memory_order_relaxed);
-    }
+    static std::atomic<size_t> optin[kMaxDevices];
+    if (const int rc = raise_smem_optin(compact_kernel<XS>, optin, dev, smem)) return rc;
     const unsigned grid2 = static_cast<unsigned>((L.n_dst + kCompactRows - 1) / kCompactRows);
     // bulk (TMA) copies of the slab rows need 16-byte aligned row pieces; SMM_COMPACT_BULK=0 forces element copies
     static const bool bulk_env = [] { const char *e = getenv("SMM_COMPACT_BULK"); return !(e && e[0] == '0'); }();

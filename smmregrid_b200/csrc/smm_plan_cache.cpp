@@ -5,11 +5,15 @@
 // 3.5 s for 75 ocean levels), repeated by every process that opens the same weight file.  The
 // cache stores the finished host structures under a key hashed from the link arrays themselves
 // (plus everything else the plan depends on), so a second process only reads and uploads them.
-// Files are written to a temporary name and renamed, so readers never see a partial file; any
-// mismatch (magic, version, sizes, truncated file) is treated as a miss.
+// Each writer fills a temporary file of its own (several threads or processes may build the same
+// operator at once) and renames it into place, so readers never see a partial file.  The file ends
+// with a hash of everything before it: any mismatch (magic, version, sizes, content, truncated file)
+// is treated as a miss, so a damaged payload never reaches the device.
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <functional>
+#include <thread>
 
 #include <sys/stat.h>
 #include <unistd.h>
@@ -20,7 +24,7 @@ namespace smm {
 
 namespace {
 
-constexpr char kMagic[8] = {'S', 'M', 'M', 'P', 'L', 'A', 'N', '6'};
+constexpr char kMagic[8] = {'S', 'M', 'M', 'P', 'L', 'A', 'N', '7'};
 
 // 4 interleaved 64-bit multiply-xorshift lanes over 8-byte words (a few GB/s on one core)
 struct Hasher {
@@ -60,7 +64,12 @@ struct Hasher {
 struct Writer {
     FILE *f;
     bool ok = true;
-    void raw(const void *p, size_t n) { if (ok && n && std::fwrite(p, 1, n, f) != n) ok = false; }
+    Hasher hs;                      // of every byte written
+    void raw(const void *p, size_t n)
+    {
+        if (ok && n && std::fwrite(p, 1, n, f) != n) ok = false;
+        hs.bytes(p, n);
+    }
     template <typename T> void pod(const T &v) { raw(&v, sizeof(T)); }
     template <typename T> void vec(const std::vector<T> &v)
     {
@@ -75,11 +84,13 @@ struct Reader {
     FILE *f;
     bool ok = true;
     uint64_t left;                  // bytes remaining in the file: bounds every vector length
+    Hasher hs;                      // of every byte read
     void raw(void *p, size_t n)
     {
         if (!ok) return;
         if (n > left || (n && std::fread(p, 1, n, f) != n)) { ok = false; return; }
         left -= n;
+        hs.bytes(p, n);
     }
     template <typename T> void pod(T &v) { raw(&v, sizeof(T)); }
     template <typename T> void vec(std::vector<T> &v)
@@ -183,9 +194,10 @@ bool plan_cache_load(const std::string &dir, const PlanCacheKey &key, int32_t n_
                           p.iplan.size() != p.wplan.size())))
                 rd.ok = false;
         }
-        uint64_t tail = 0;
+        uint64_t want[2], tail[2] = {0, 0};
+        rd.hs.finish(want);
         rd.pod(tail);
-        good = rd.ok && tail == (key.h[0] ^ key.h[1]);
+        good = rd.ok && rd.left == 0 && tail[0] == want[0] && tail[1] == want[1];
     }
     std::fclose(f);
     if (!good) { csrs.clear(); plans.clear(); }
@@ -198,7 +210,8 @@ bool plan_cache_store(const std::string &dir, const PlanCacheKey &key, std::vect
 {
     ::mkdir(dir.c_str(), 0777);            // best effort; an existing directory is fine
     const std::string path = cache_file(dir, key);
-    const std::string tmp = path + ".tmp" + std::to_string(static_cast<long long>(getpid()));
+    const std::string tmp = path + ".tmp" + std::to_string(static_cast<long long>(getpid())) + "." +
+                            std::to_string(std::hash<std::thread::id>{}(std::this_thread::get_id()));
     FILE *f = std::fopen(tmp.c_str(), "wb");
     if (!f) return false;
     Writer wr{f};
@@ -211,7 +224,8 @@ bool plan_cache_store(const std::string &dir, const PlanCacheKey &key, std::vect
         io_csr(wr, csrs[i]);
         io_plan(wr, plans[i]);
     }
-    const uint64_t tail = key.h[0] ^ key.h[1];
+    uint64_t tail[2];
+    wr.hs.finish(tail);
     wr.pod(tail);
     const bool ok = wr.ok && std::fclose(f) == 0;
     if (!wr.ok) std::fclose(f);
