@@ -10,10 +10,8 @@
 #include <cstring>
 #include <mutex>
 #include <string>
-#include <thread>
 #include <vector>
 
-#include <sched.h>
 #if defined(__x86_64__) || defined(_M_X64)
 #include <emmintrin.h>
 #endif
@@ -55,8 +53,6 @@ void smm_count_launches(int n) { g_launches.fetch_add(n, std::memory_order_relax
 namespace {
 
 int fail(int code, const std::string &msg) { return smm_fail(code, msg); }
-
-constexpr int kHostSlots = 4;
 
 struct HostSlot {
     void *dx = nullptr, *dy = nullptr;
@@ -186,10 +182,10 @@ inline size_t round_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 // the packed-rows layout (a thread owns up to 4 rows).
 struct PlanChoice {
     bool cfg = false, packed = false;
-    int32_t lpr = 0, kpl = 0, nct = 256;
+    int32_t lpr = 0, kpl = 0;
 };
 
-PlanChoice choose_plan(const std::vector<HostCsr> &csrs, int64_t n_dst, int sm_count, bool ref_order)
+PlanChoice choose_plan(const std::vector<HostCsr> &csrs, const PlanSettings &s)
 {
     PlanChoice pc;
     int32_t max_row = 0;
@@ -199,29 +195,9 @@ PlanChoice choose_plan(const std::vector<HostCsr> &csrs, int64_t n_dst, int sm_c
         const int64_t ps = packed_slots(c);
         pslots = (ps < 0 || pslots < 0) ? -1 : pslots + ps;
     }
-    pc.cfg = choose_lanes(max_row, pc.lpr, pc.kpl);
-    const int64_t nlev = static_cast<int64_t>(std::max<size_t>(csrs.size(), 1));
-    pc.packed = pc.cfg && prefer_packed(pslots);
-    // packed plans: always 256 consumer threads, two CTAs per SM (measured: bilinear 1440x721 ->
-    // 3600x1800 +4 %, 1:1 conservative +3 %, C3 +9 % over 512); n_dst = 0 leaves only the
-    // SMM_CONSUMER_THREADS override
-    pc.nct = pc.packed ? default_consumer_threads(0, 1, sm_count)
-                       : default_consumer_threads(n_dst, pc.cfg ? pc.lpr : 0, sm_count);
-    if (ref_order) pc.nct = 256;         // reference-order kernels exist for 256 consumer threads only
-    (void)nlev;
+    pc.cfg = choose_lanes(s, max_row, pc.lpr, pc.kpl);
+    pc.packed = pc.cfg && prefer_packed(s, pslots);
     return pc;
-}
-
-int host_threads_all()
-{
-    cpu_set_t set;
-    return sched_getaffinity(0, sizeof(set), &set) == 0 ? std::max(1, CPU_COUNT(&set)) : 1;
-}
-
-int env_int_plan(const char *name, int dflt)
-{
-    const char *e = std::getenv(name);
-    return e ? std::atoi(e) : dflt;
 }
 
 // Tile plans of all levels, one layout for the whole weight set so that a grouped launch runs a
@@ -236,9 +212,9 @@ int env_int_plan(const char *name, int dflt)
 // does: if any level's packed plan is unusable for that reason, all levels fall back to the next
 // candidate.
 void plan_levels(const std::vector<HostCsr> &csrs, int64_t n_dst, int sm_count, bool ref_order,
-                 std::vector<HostPlan> &plans)
+                 const PlanSettings &s, std::vector<HostPlan> &plans)
 {
-    PlanChoice pc = choose_plan(csrs, n_dst, sm_count, ref_order);
+    const PlanChoice pc = choose_plan(csrs, s);
     plans.assign(csrs.size(), HostPlan{});
     bool split = false;
     if (pc.cfg && !pc.packed) {
@@ -250,19 +226,19 @@ void plan_levels(const std::vector<HostCsr> &csrs, int64_t n_dst, int sm_count, 
                 if (n > 16) { ++rows_long; nnz_long += n; }
             }
         split = rows_long > 0 && rows_long * 8 <= rows && nnz_long * 5 <= nnz * 2;
-        if (const char *e = std::getenv("SMM_SPLIT")) split = rows_long > 0 && e[0] == '1';      // experiments: 0 | 1
+        if (s.split >= 0) split = rows_long > 0 && s.split == 1;
     }
     // levels are independent: a few host threads take them in turn (75 ocean levels: ~13 s -> ~1 s)
-    const int nthreads = std::max(1, std::min({host_threads_all(), 16, static_cast<int>(csrs.size())}));
+    const int nthreads = std::max(1, std::min({host_cpus(), 16, static_cast<int>(csrs.size())}));
     // reference-order sums for rows beyond the packed layout: a thread per row with the links in
     // shared memory (ordered_kernel) when an image of K = longest row links x R rows x 12 bytes fits
     // ~100 KB for some R in {256, 128, 64, 32}; else the lane-by-lane chain of staged_kernel<ORD>
     int32_t ord_k = 0, ord_rows = 0;
-    if (ref_order && pc.cfg && !pc.packed && env_int_plan("SMM_ORDLONG", 1) != 0) {
+    if (ref_order && pc.cfg && !pc.packed && s.ordlong) {
         for (const HostCsr &c : csrs) ord_k = std::max(ord_k, c.max_row_nnz);
         for (int32_t r : {256, 128, 64, 32})
             if (ord_rows == 0 && static_cast<int64_t>(ord_k) * r * 12 <= 100 * 1024) ord_rows = r;
-        if (const int forced = env_int_plan("SMM_ORD_ROWS", 0)) ord_rows = forced;
+        if (s.ord_rows) ord_rows = s.ord_rows;
     }
     enum Mode { kSplit, kPacked, kOrdLong, kLanes };
     std::vector<Mode> modes;
@@ -271,51 +247,42 @@ void plan_levels(const std::vector<HostCsr> &csrs, int64_t n_dst, int sm_count, 
     if (ord_rows > 0) modes.push_back(kOrdLong);
     modes.push_back(kLanes);
     for (Mode mode : modes) {
+        // packed plans: 256 consumer threads, two CTAs per SM (measured: bilinear 1440x721 -> 3600x1800
+        // +4 %, 1:1 conservative +3 %, C3 +9 % over 512), unless SMM_CONSUMER_THREADS overrides;
+        // reference-order kernels exist for 256 consumer threads only
         const int32_t nct = mode == kOrdLong ? ord_rows
-                            : mode == kLanes ? (ref_order ? 256 : default_consumer_threads(n_dst, pc.cfg ? pc.lpr : 0, sm_count))
-                                             : (ref_order ? 256 : default_consumer_threads(0, 1, sm_count));
-        std::atomic<size_t> next{0};
+                            : mode == kLanes ? (ref_order ? 256 : default_consumer_threads(s, n_dst, pc.cfg ? pc.lpr : 0, sm_count))
+                                             : (ref_order ? 256 : default_consumer_threads(s, 0, 1, sm_count));
         std::atomic<bool> retry{false};
-        auto work = [&]() {
-            for (size_t i = next.fetch_add(1); i < csrs.size() && !retry.load(); i = next.fetch_add(1)) {
-                plans[i] = HostPlan{};
-                plans[i].ref_order = ref_order;
-                if (!pc.cfg) { plans[i].why = "a destination row has more than 512 links"; continue; }
-                if (mode == kSplit) {
-                    std::vector<int32_t> lrows, srows;
-                    long_rows(csrs[i], lrows, srows);
-                    build_plan(csrs[i], -1, pc.kpl, nct, ref_order, plans[i], &srows);
-                    plans[i].gather_rows = std::move(lrows);
-                    if (!plans[i].ok) retry.store(true);           // any failure: the whole set takes the next layout
-                } else if (mode == kOrdLong) {
-                    build_plan(csrs[i], 1, ord_k, nct, true, plans[i]);
-                    plans[i].ordlong = plans[i].ok;
-                    if (!plans[i].ok && !csrs[i].col.empty()) retry.store(true);
-                } else {
-                    build_plan(csrs[i], mode == kPacked ? -1 : pc.lpr, pc.kpl, nct, ref_order, plans[i]);
-                    // only a footprint that is too large can be cured by smaller tiles
-                    if (mode == kPacked && !plans[i].ok && plans[i].why.rfind("tile footprint", 0) == 0) retry.store(true);
-                }
+        parallel_for(nthreads, static_cast<int64_t>(csrs.size()), [&](int64_t i) {
+            if (retry.load()) return;
+            plans[i] = HostPlan{};
+            plans[i].ref_order = ref_order;
+            if (!pc.cfg) { plans[i].why = "a destination row has more than 512 links"; return; }
+            if (mode == kSplit) {
+                std::vector<int32_t> lrows, srows;
+                long_rows(csrs[i], lrows, srows);
+                build_plan(csrs[i], -1, pc.kpl, nct, ref_order, s, plans[i], &srows);
+                plans[i].gather_rows = std::move(lrows);
+                if (!plans[i].ok) retry.store(true);           // any failure: the whole set takes the next layout
+            } else if (mode == kOrdLong) {
+                build_plan(csrs[i], 1, ord_k, nct, true, s, plans[i]);
+                plans[i].ordlong = plans[i].ok;
+                if (!plans[i].ok && !csrs[i].col.empty()) retry.store(true);
+            } else {
+                build_plan(csrs[i], mode == kPacked ? -1 : pc.lpr, pc.kpl, nct, ref_order, s, plans[i]);
+                // only a footprint that is too large can be cured by smaller tiles
+                if (mode == kPacked && !plans[i].ok && plans[i].why.rfind("tile footprint", 0) == 0) retry.store(true);
             }
-        };
-        if (nthreads == 1) {
-            work();
-        } else {
-            std::vector<std::thread> pool;
-            for (int t = 0; t < nthreads; ++t) pool.emplace_back(work);
-            for (auto &th : pool) th.join();
-        }
+        });
         if (!retry.load()) return;
     }
 }
 
 // SMM_SUM_AUTO: reference order when some weight is negative (the products of a row can cancel)
-bool resolve_ref_order(int32_t summation, const std::vector<HostCsr> &csrs)
+bool resolve_ref_order(int32_t summation, const PlanSettings &s, const std::vector<HostCsr> &csrs)
 {
-    if (const char *e = std::getenv("SMM_SUMMATION")) {          // experiments: fast | reference
-        if (e[0] == 'f') return false;
-        if (e[0] == 'r') return true;
-    }
+    if (s.summation != SMM_SUM_AUTO) summation = s.summation;
     if (summation == SMM_SUM_REFERENCE) return true;
     if (summation == SMM_SUM_FAST) return false;
     for (const HostCsr &c : csrs)
@@ -329,7 +296,7 @@ bool resolve_ref_order(int32_t summation, const std::vector<HostCsr> &csrs)
 int build_host_operator(int32_t n_levels, const int64_t *link_length, int64_t nl_max, int64_t n_src, int64_t n_dst,
                         const int32_t *src_address, const int32_t *dst_address, const double *remap_matrix,
                         int32_t num_wgts, int32_t index_base, const smm_create_opts *opts, int sm_count,
-                        std::vector<HostCsr> &csrs, std::vector<HostPlan> &plans, bool &ref_order, bool &cache_hit)
+                        const PlanSettings &s, std::vector<HostCsr> &csrs, std::vector<HostPlan> &plans, bool &ref_order, bool &cache_hit)
 {
     const int32_t summation = opts ? opts->summation : SMM_SUM_AUTO;
     if (summation != SMM_SUM_AUTO && summation != SMM_SUM_FAST && summation != SMM_SUM_REFERENCE)
@@ -345,7 +312,7 @@ int build_host_operator(int32_t n_levels, const int64_t *link_length, int64_t nl
     const bool use_cache = !cache_dir.empty() && usable_arrays && n_src > 0 && n_dst > 0 && num_wgts >= 1;
     if (use_cache) {
         cache_key = plan_cache_key(n_levels, link_length, nl_max, n_src, n_dst, src_address, dst_address,
-                                   remap_matrix, num_wgts, index_base, summation, sm_count);
+                                   remap_matrix, num_wgts, index_base, summation, sm_count, s);
         cache_hit = plan_cache_load(cache_dir, cache_key, n_levels, n_src, n_dst, csrs, plans, ref_order);
         if (cache_hit) return SMM_OK;
         csrs.assign(static_cast<size_t>(n_levels), HostCsr{});
@@ -354,40 +321,24 @@ int build_host_operator(int32_t n_levels, const int64_t *link_length, int64_t nl
         // levels are independent: built by a few host threads; the first failing level is reported
         std::vector<int> rcs(static_cast<size_t>(n_levels), SMM_OK);
         std::vector<std::string> errs(static_cast<size_t>(n_levels));
-        std::atomic<int32_t> next{0};
-        auto work = [&]() {
-            for (int32_t i = next.fetch_add(1); i < n_levels; i = next.fetch_add(1)) {
-                const int64_t o = static_cast<int64_t>(i) * nl_max;
-                rcs[i] = build_csr(n_src, n_dst, link_length[i], src_address ? src_address + o : nullptr,
-                                   dst_address ? dst_address + o : nullptr,
-                                   remap_matrix ? remap_matrix + o * num_wgts : nullptr, num_wgts, index_base,
-                                   csrs[i], errs[i]);
-            }
-        };
-        const int nthreads = std::max(1, std::min({host_threads_all(), 16, static_cast<int>(n_levels)}));
-        if (nthreads == 1) {
-            work();
-        } else {
-            std::vector<std::thread> pool;
-            for (int t = 0; t < nthreads; ++t) pool.emplace_back(work);
-            for (auto &th : pool) th.join();
-        }
+        const int nthreads = std::max(1, std::min({host_cpus(), 16, static_cast<int>(n_levels)}));
+        parallel_for(nthreads, n_levels, [&](int64_t i) {
+            const int64_t o = i * nl_max;
+            rcs[i] = build_csr(n_src, n_dst, link_length[i], src_address ? src_address + o : nullptr,
+                               dst_address ? dst_address + o : nullptr,
+                               remap_matrix ? remap_matrix + o * num_wgts : nullptr, num_wgts, index_base,
+                               csrs[i], errs[i]);
+        });
         for (int32_t i = 0; i < n_levels; ++i)
             if (rcs[i]) return fail(rcs[i], (n_levels > 1 ? "level " + std::to_string(i) + ": " : "") + errs[i]);
     }
-    ref_order = resolve_ref_order(summation, csrs);
-    plan_levels(csrs, n_dst, sm_count, ref_order, plans);
+    ref_order = resolve_ref_order(summation, s, csrs);
+    plan_levels(csrs, n_dst, sm_count, ref_order, s, plans);
     if (use_cache) plan_cache_store(cache_dir, cache_key, csrs, plans, ref_order);   // best effort
     return SMM_OK;
 }
 
 // ------------------------------------------------------------------ launch dispatch
-
-int env_int(const char *name, int dflt)
-{
-    const char *e = std::getenv(name);
-    return e ? std::atoi(e) : dflt;
-}
 
 // (packed 16-bit x: the element type follows the decoded dtype, opt.dec_dtype)
 #define SMM_DTYPE_DISPATCH(FN, ...)                                                                           \
@@ -411,14 +362,13 @@ size_t x_elem_bytes(int32_t x_dtype) { return x_dtype == SMM_I16 ? 2 : x_dtype =
 int64_t pick_chunks(int64_t B, int64_t blocks_total, int64_t slots, double bytes_per_row, double prologue_us,
                     int64_t multiple, int64_t &chunk)
 {
-    static const int k_min_rows = std::max(1, env_int("SMM_MIN_ROWS_PER_ITEM", 8));
-    static const int k_waves = env_int("SMM_WAVES", 0);                    // experiments: fixed wave count
+    const LaunchSettings &ls = launch_settings();
     const double t_us = static_cast<double>(B) * bytes_per_row / 6.5e6;     // at ~6.5 TB/s
-    double waves = k_waves > 0 ? k_waves : std::sqrt(t_us / (2.0 * prologue_us));
+    double waves = ls.waves > 0 ? ls.waves : std::sqrt(t_us / (2.0 * prologue_us));
     waves = std::min(32.0, std::max(1.0, waves));
     const double items = waves * static_cast<double>(slots);
     int64_t nchunks = static_cast<int64_t>(items / static_cast<double>(std::max<int64_t>(blocks_total, 1)) + 0.5);
-    const int64_t max_chunks = std::max<int64_t>(1, B / k_min_rows);
+    const int64_t max_chunks = std::max<int64_t>(1, B / ls.min_rows_per_item);
     nchunks = std::max<int64_t>(1, std::min<int64_t>({nchunks, max_chunks, 65535}));      // (grid.y of the staged launch)
     chunk = (B + nchunks - 1) / nchunks;
     chunk = (chunk + multiple - 1) / multiple * multiple;
@@ -556,10 +506,8 @@ int launch_jobs(const smm_handle *h, const std::vector<JobSpec> &specs, int32_t 
     a.B = B; a.x_bstride = xbs; a.y_bstride = ybs; a.remap_area_min = area_min;
     a.renorm_min_valid = opt.renorm_min_valid;
     a.dec = opt.dec;
-    // experiment switches are read once per process, not per launch
-    static const uint32_t k_debug_flags = static_cast<uint32_t>(env_int("SMM_DEBUG_STREAM_ONLY", 0)) & 3u;
-    static const int k_max_stages = std::max(2, env_int("SMM_MAX_STAGES", kMaxStages));
-    a.debug_flags = k_debug_flags;   // bit 0: staged consumers skip the arithmetic (profiling aid)
+    const LaunchSettings &ls = launch_settings();
+    a.debug_flags = ls.debug_flags;
 
     auto fill_job = [&](const JobSpec &s, LevelJob &j) {
         const LevelDev &L = h->levels[s.level];
@@ -600,8 +548,7 @@ int launch_jobs(const smm_handle *h, const std::vector<JobSpec> &specs, int32_t 
         const size_t row_bytes = std::max<size_t>(128, round_up(max_elems * sx, 128));
         // stage several batch rows together (up to 8, ~56 KB per stage) so that the per-stage
         // barrier and loop overhead of the consumers is amortised: C3 2156 -> 2671 GB/s, C2 5565 -> 6111
-        static const int k_rows_per_stage = env_int("SMM_ROWS_PER_STAGE", 0);
-        int nb_rows = k_rows_per_stage > 0 ? k_rows_per_stage : static_cast<int>((56u << 10) / row_bytes);
+        int nb_rows = ls.rows_per_stage > 0 ? ls.rows_per_stage : static_cast<int>((56u << 10) / row_bytes);
         const size_t half = (228u * 1024u - 2u * 1024u) / 2u - 1024u;   // two CTAs per SM (NCT = 256)
         {   // ...but never at the price of pipeline depth (>= 4 stages) or of the second CTA per SM
             const size_t budget = (nct == 256 ? half : h->smem_optin) - std::min(stage_off, half);
@@ -626,7 +573,7 @@ int launch_jobs(const smm_handle *h, const std::vector<JobSpec> &specs, int32_t 
         size_t S = (!ordl && nct == 256 && half > stage_off) ? (half - stage_off) / stage_bytes : 0;
         if (S < 3) S = (h->smem_optin - stage_off) / stage_bytes;        // one CTA per SM
         S = std::min<size_t>(S, kMaxStages);
-        S = std::min<size_t>(S, static_cast<size_t>(k_max_stages));
+        S = std::min<size_t>(S, static_cast<size_t>(ls.max_stages));
         if (S < 2) return fail(SMM_ERR_INVALID, "internal: staged footprint does not fit");
         a.nstages = static_cast<int32_t>(S);
         a.stage_bytes = static_cast<uint32_t>(stage_bytes);
@@ -651,8 +598,7 @@ int launch_jobs(const smm_handle *h, const std::vector<JobSpec> &specs, int32_t 
         const dim3 grid(static_cast<unsigned>(max_tiles), static_cast<unsigned>(nchunks), static_cast<unsigned>(jb.njobs));
         // two threads per row (one per batch row of a pair) while that leaves at most 8 consumer warps:
         // C4 (64 rows per tile) 3060 -> 3989 GB/s, C2 (256 rows: 16 warps re-reading the image) 4368 -> 3518
-        static const int k_ord_tpr = env_int("SMM_ORD_TPR", 0);
-        const int tpr = (ordl && nb_rows >= 2 && (k_ord_tpr == 2 || (k_ord_tpr == 0 && nct <= 128))) ? 2 : 1;
+        const int tpr = (ordl && nb_rows >= 2 && (ls.ord_tpr == 2 || (ls.ord_tpr == 0 && nct <= 128))) ? 2 : 1;
         const int rc = ordl ? SMM_DTYPE_DISPATCH(launch_ordered_t, h->device, nct, tpr, grid, smem, st, jb, a)
                             : SMM_DTYPE_DISPATCH(launch_staged_t, h->device, lpr, kpl, nct, packed, ord, grid, smem, st, jb, a);
         if (rc) return rc;
@@ -738,14 +684,6 @@ bool is_pinned(const void *p)
     return at.type == cudaMemoryTypeHost || at.type == cudaMemoryTypeManaged;
 }
 
-int host_threads()
-{
-    cpu_set_t set;
-    int n = 1;
-    if (sched_getaffinity(0, sizeof(set), &set) == 0) n = CPU_COUNT(&set);
-    return std::max(1, std::min(n, env_int("SMM_HOST_COPY_THREADS", 12)));
-}
-
 // Large host copy with non-temporal stores: the destination (a pinned bounce buffer the DMA engine
 // reads next) is written once and not read by the CPU again, so bypassing the cache saves the
 // read-for-ownership of every destination line (+18 % over memcpy, measured with 4-8 threads).
@@ -784,20 +722,16 @@ void parallel_copy_rows(char *dst, size_t dst_stride, const char *src, size_t sr
         return;
     }
     // split by bytes so a few huge rows still spread over all threads
-    std::vector<std::thread> pool;
-    for (int t = 0; t < nthreads; ++t) {
-        pool.emplace_back([=]() {
-            const size_t lo = total * t / nthreads, hi = total * (t + 1) / nthreads;
-            size_t pos = lo;
-            while (pos < hi) {
-                const size_t r = pos / row_bytes, o = pos % row_bytes;
-                const size_t n = std::min(row_bytes - o, hi - pos);
-                copy_streaming(dst + r * dst_stride + o, src + r * src_stride + o, n);
-                pos += n;
-            }
-        });
-    }
-    for (auto &th : pool) th.join();
+    parallel_for(nthreads, nthreads, [&](int64_t t) {
+        const size_t lo = total * t / nthreads, hi = total * (t + 1) / nthreads;
+        size_t pos = lo;
+        while (pos < hi) {
+            const size_t r = pos / row_bytes, o = pos % row_bytes;
+            const size_t n = std::min(row_bytes - o, hi - pos);
+            copy_streaming(dst + r * dst_stride + o, src + r * src_stride + o, n);
+            pos += n;
+        }
+    });
 }
 
 int check_dtypes(int32_t x_dtype, int32_t y_dtype)
@@ -839,7 +773,8 @@ template <typename Launch>
 int host_pipeline(smm_handle *h, const void *x, size_t row_x, size_t x_stride, void *y, size_t row_y,
                   size_t y_stride, int64_t B, int64_t chunk_rows, Launch launch)
 {
-    static const bool k_trace = env_int("SMM_HOST_TRACE", 0) != 0;      // diagnostics: phase times on stderr
+    const LaunchSettings &ls = launch_settings();
+    const HostCallSettings hs = host_call_settings();
     const auto t_enter = std::chrono::steady_clock::now();
     auto ms_since = [&](std::chrono::steady_clock::time_point t0) {
         return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
@@ -847,9 +782,8 @@ int host_pipeline(smm_handle *h, const void *x, size_t row_x, size_t x_stride, v
     const bool x_pinned = is_pinned(x), y_pinned = is_pinned(y);
     if (chunk_rows <= 0) {
         // ~128 MB of source per chunk for direct DMA (the fill of the pipeline -- the first chunk's
-        // copy -- is the only part that does not overlap), ~64 MB when staging; at least 4 rows;
-        // SMM_HOST_CHUNK_MB overrides
-        const int64_t mb = std::max(1, env_int("SMM_HOST_CHUNK_MB", x_pinned ? 128 : 64));
+        // copy -- is the only part that does not overlap), ~64 MB when staging; at least 4 rows
+        const int64_t mb = hs.chunk_mb > 0 ? hs.chunk_mb : (x_pinned ? 128 : 64);
         chunk_rows = std::max<int64_t>(4, (mb << 20) / std::max<int64_t>(1, static_cast<int64_t>(row_x)));
     }
     chunk_rows = std::min(chunk_rows, B);
@@ -859,9 +793,7 @@ int host_pipeline(smm_handle *h, const void *x, size_t row_x, size_t x_stride, v
     const size_t need_y = static_cast<size_t>(chunk_rows) * row_y;
     for (cudaStream_t *sp : {&h->s_in[0], &h->s_in[1], &h->s_k, &h->s_out})
         if (!*sp) CUDA_TRY(cudaStreamCreateWithFlags(sp, cudaStreamNonBlocking));
-    static const int k_in_streams = std::max(1, std::min(2, env_int("SMM_HOST_IN_STREAMS", 2)));
-    static const int k_slots = std::max(2, std::min(kHostSlots, env_int("SMM_HOST_SLOTS", kHostSlots)));
-    const int nslots = static_cast<int>(std::min<int64_t>(k_slots, (B + chunk_rows - 1) / chunk_rows));
+    const int nslots = static_cast<int>(std::min<int64_t>(ls.host_slots, (B + chunk_rows - 1) / chunk_rows));
     for (int s = 0; s < nslots; ++s) {
         HostSlot &sl = h->slots[s];
         for (cudaEvent_t *ev : {&sl.ev_in, &sl.ev_k, &sl.ev_out})
@@ -887,7 +819,7 @@ int host_pipeline(smm_handle *h, const void *x, size_t row_x, size_t x_stride, v
             sl.cap_py = need_y;
         }
     }
-    const int nthreads = host_threads();
+    const int nthreads = hs.copy_threads;
     struct Pending { char *ys = nullptr; int64_t nb = 0; bool used = false; };
     Pending pending[kHostSlots];
     // waits for the slot's last result copy and, when staging, hands the rows to the caller
@@ -908,7 +840,7 @@ int host_pipeline(smm_handle *h, const void *x, size_t row_x, size_t x_stride, v
         for (int64_t b0 = 0; b0 < B; b0 += chunk_rows, slot = (slot + 1) % nslots, ++ichunk) {
             const int64_t nb = std::min(chunk_rows, B - b0);
             HostSlot &sl = h->slots[slot];
-            cudaStream_t s_in = h->s_in[ichunk % k_in_streams];
+            cudaStream_t s_in = h->s_in[ichunk % ls.host_in_streams];
             const char *xs = static_cast<const char *>(x) + static_cast<size_t>(b0) * x_stride;
             char *ys = static_cast<char *>(y) + static_cast<size_t>(b0) * y_stride;
             const bool reused = pending[slot].used;
@@ -955,7 +887,7 @@ int host_pipeline(smm_handle *h, const void *x, size_t row_x, size_t x_stride, v
     };
     const double ms_setup = ms_since(t_enter);
     const int rc = run();
-    if (k_trace)
+    if (ls.host_trace)
         std::fprintf(stderr, "[smm host pipeline] B=%lld chunk_rows=%lld slots=%d pinned x/y=%d/%d setup %.3f ms total %.3f ms (%.2f GB/s in)\n",
                      static_cast<long long>(B), static_cast<long long>(chunk_rows), nslots, int(x_pinned), int(y_pinned), ms_setup,
                      ms_since(t_enter), static_cast<double>(B) * row_x / (ms_since(t_enter) * 1e6));
@@ -992,6 +924,7 @@ int smm_create_levels(int32_t n_levels, const int64_t *link_length, int64_t nl_m
                       const double *remap_matrix, int32_t num_wgts, int32_t index_base,
                       int32_t device, const smm_create_opts *opts, smm_handle **out)
 {
+    const PlanSettings settings = plan_settings();
     if (!out) return fail(SMM_ERR_INVALID, "null output handle pointer");
     *out = nullptr;
     if (n_levels < 1 || !link_length || nl_max < 0)
@@ -1008,7 +941,7 @@ int smm_create_levels(int32_t n_levels, const int64_t *link_length, int64_t nl_m
     std::vector<HostCsr> csrs;
     std::vector<HostPlan> plans;
     rc = build_host_operator(n_levels, link_length, nl_max, n_src, n_dst, src_address, dst_address, remap_matrix,
-                             num_wgts, index_base, opts, h->sm_count, csrs, plans, h->ref_order, h->cache_hit);
+                             num_wgts, index_base, opts, h->sm_count, settings, csrs, plans, h->ref_order, h->cache_hit);
     if (rc) { delete h; return rc; }
     h->levels.resize(static_cast<size_t>(n_levels));
     DeviceGuard g(device);              // the caller's current device is left as it was
@@ -1293,6 +1226,7 @@ int smm_host_plan_build(int64_t n_src, int64_t n_dst, int64_t nnz, const int32_t
                         const int32_t *dst_address, const double *remap_matrix, int32_t num_wgts,
                         int32_t index_base, const smm_create_opts *opts, smm_host_plan **out)
 {
+    const PlanSettings settings = plan_settings();
     if (!out) return fail(SMM_ERR_INVALID, "null output pointer");
     *out = nullptr;
     if (nnz < 0) return fail(SMM_ERR_INVALID, "smm_create: n_src, n_dst must be > 0, nnz >= 0, num_wgts >= 1");
@@ -1303,7 +1237,7 @@ int smm_host_plan_build(int64_t n_src, int64_t n_dst, int64_t nnz, const int32_t
     bool ref_order = false;
     const int64_t ll = nnz;
     const int rc = build_host_operator(1, &ll, nnz, n_src, n_dst, src_address, dst_address, remap_matrix, num_wgts,
-                                       index_base, opts, 148, csrs, plans, ref_order, p->cache_hit);
+                                       index_base, opts, 148, settings, csrs, plans, ref_order, p->cache_hit);
     if (rc) { delete p; return rc; }
     p->csr = std::move(csrs[0]);
     p->plan = std::move(plans[0]);

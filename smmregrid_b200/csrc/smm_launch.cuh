@@ -4,11 +4,11 @@
 #pragma once
 #include <algorithm>
 #include <atomic>
-#include <cstdlib>
 #include <mutex>
 
 #include "smm_internal.h"
 #include "smm_kernels.cuh"
+#include "smm_tuning.h"
 
 namespace smm {
 
@@ -105,13 +105,13 @@ int launch_compact_t(int dev, const LevelDev &L, const JobSpec &sp, void *xt_raw
     static std::atomic<size_t> optin[kMaxDevices];
     if (const int rc = raise_smem_optin(compact_kernel<XS>, optin, dev, smem)) return rc;
     const unsigned grid2 = static_cast<unsigned>((L.n_dst + kCompactRows - 1) / kCompactRows);
-    // bulk (TMA) copies of the slab rows need 16-byte aligned row pieces; SMM_COMPACT_BULK=0 forces element copies
-    static const bool bulk_env = [] { const char *e = getenv("SMM_COMPACT_BULK"); return !(e && e[0] == '0'); }();
-    const int bulk = bulk_env && reinterpret_cast<uintptr_t>(sp.x) % 16 == 0 && (xbs * sizeof(XS)) % 16 == 0 &&
+    const LaunchSettings &ls = launch_settings();
+    // bulk (TMA) copies of the slab rows need 16-byte aligned row pieces
+    const int bulk = ls.compact_bulk && reinterpret_cast<uintptr_t>(sp.x) % 16 == 0 && (xbs * sizeof(XS)) % 16 == 0 &&
                      (kCompactW * sizeof(XS)) % 16 == 0;
     // 8-byte elements: half the batch rows per pass keeps the pass-1 tile at the size that lets three
     // blocks share an SM (one block's transposition overlaps the others' copies)
-    static const int rows64 = [] { const char *e = getenv("SMM_COMPACT_F64_ROWS"); return e ? atoi(e) : 32; }();
+    const int rows64 = ls.compact_f64_rows;
     const int step = (sizeof(XS) == 8 && bulk && rows64 > 0 && rows64 < kCompactBC) ? rows64 : kCompactBC;
     for (int64_t b0 = 0; b0 < B; b0 += step) {
         const int bc = static_cast<int>(B - b0 < step ? B - b0 : step);

@@ -8,13 +8,9 @@
 #include "smm_plan.h"
 
 #include <algorithm>
-#include <cstdio>
-#include <cstdlib>
-#include <functional>
+#include <atomic>
 #include <numeric>
 #include <thread>
-
-#include <sched.h>
 
 #include "../../include/smmregrid_b200.h"
 
@@ -94,12 +90,9 @@ int build_csr(int64_t n_src, int64_t n_dst, int64_t nnz, const int32_t *src_addr
     return SMM_OK;
 }
 
-bool choose_lanes(int32_t m, int32_t &lpr, int32_t &kpl)
+bool choose_lanes(const PlanSettings &s, int32_t m, int32_t &lpr, int32_t &kpl)
 {
-    if (const char *e = std::getenv("SMM_FORCE_LANES")) {       // experiments: "lpr,kpl"
-        int a = 0, b = 0;
-        if (std::sscanf(e, "%d,%d", &a, &b) == 2 && a > 0 && b > 0 && m <= a * b) { lpr = a; kpl = b; return true; }
-    }
+    if (s.force_lpr > 0 && m <= s.force_lpr * s.force_kpl) { lpr = s.force_lpr; kpl = s.force_kpl; return true; }
     // (lanes per row, links per lane): fewest padded slots first -- every slot, padded or not,
     // costs an F2F conversion, and conversion throughput bounds link-dense operators
     if (m <= 4) { lpr = 1; kpl = 4; }
@@ -120,13 +113,9 @@ bool choose_lanes(int32_t m, int32_t &lpr, int32_t &kpl)
     return true;
 }
 
-int32_t default_consumer_threads(int64_t n_dst, int32_t lpr, int32_t sm_count)
+int32_t default_consumer_threads(const PlanSettings &s, int64_t n_dst, int32_t lpr, int32_t sm_count)
 {
-    const char *e = std::getenv("SMM_CONSUMER_THREADS");
-    if (e) {
-        const int v = std::atoi(e);
-        if (v == 256 || v == 512) return v;
-    }
+    if (s.consumer_threads) return s.consumer_threads;
     if (lpr <= 0) return 256;
     const int64_t tiles512 = (n_dst + 512 / lpr - 1) / (512 / lpr);
     return tiles512 >= sm_count ? 512 : 256;
@@ -139,7 +128,8 @@ int32_t default_consumer_threads(int64_t n_dst, int32_t lpr, int32_t sm_count)
 constexpr int kSubRows = 4, kSubLinks = 4;
 
 static void build_plan_rows(const HostCsr &csr, int32_t force_lpr, int32_t force_kpl, int32_t nct,
-                            const std::vector<int32_t> *order, bool packed, bool ref_order, HostPlan &plan)
+                            const std::vector<int32_t> *order, bool packed, bool ref_order, const PlanSettings &s,
+                            HostPlan &plan)
 {
     plan = HostPlan{};
     plan.ref_order = ref_order;
@@ -154,7 +144,7 @@ static void build_plan_rows(const HostCsr &csr, int32_t force_lpr, int32_t force
         if (max_row > kSubRows * kSubLinks) { plan.why = "row too long for the packed layout"; return; }
         lpr = 1; kpl = kSubRows * kSubLinks;
     } else if (lpr <= 0 || kpl <= 0) {
-        if (!choose_lanes(max_row, lpr, kpl)) {
+        if (!choose_lanes(s, max_row, lpr, kpl)) {
             plan.why = "a destination row has more than 512 links";
             return;
         }
@@ -594,25 +584,13 @@ static void build_plan_rows(const HostCsr &csr, int32_t force_lpr, int32_t force
     }
     };
 
-    int nthreads = 1;
-    {
-        cpu_set_t set;
-        if (sched_getaffinity(0, sizeof(set), &set) == 0) nthreads = CPU_COUNT(&set);
-        if (const char *e = std::getenv("SMM_PLAN_THREADS")) nthreads = std::atoi(e);
-        nthreads = static_cast<int>(std::max<int64_t>(1, std::min<int64_t>({nthreads, 16, ntiles / 32})));
-    }
+    const int nthreads = static_cast<int>(std::max<int64_t>(1, std::min<int64_t>({s.plan_threads, 16, ntiles / 32})));
     std::vector<Part> parts(static_cast<size_t>(nthreads));
     for (int i = 0; i < nthreads; ++i) {
         parts[i].t0 = ntiles * i / nthreads;
         parts[i].t1 = ntiles * (i + 1) / nthreads;
     }
-    if (nthreads == 1) {
-        work(parts[0]);
-    } else {
-        std::vector<std::thread> pool;
-        for (int i = 0; i < nthreads; ++i) pool.emplace_back(work, std::ref(parts[i]));
-        for (auto &th : pool) th.join();
-    }
+    parallel_for(nthreads, nthreads, [&](int64_t i) { work(parts[i]); });
     int64_t sum_blocks = 0;
     for (Part &pt : parts) {
         if (pt.too_big) { plan.why = "tile footprint exceeds 16-bit local indices"; return; }
@@ -664,20 +642,18 @@ int64_t packed_slots(const HostCsr &csr)
 // destination side, and four rows per thread amortise the per-row loop / barrier / epilogue
 // instructions that bound the lane-per-row layout there (measured on B200: bilinear
 // 1440x721 -> 3600x1800 2841 -> 5141 GB/s, 1:1 conservative 3845 -> 6096, 75 ocean levels
-// 2665 -> 5490; bilinear down-sampling within 2 %).  SMM_PACKED=0|1 overrides.
-bool prefer_packed(int64_t slots_packed)
+// 2665 -> 5490; bilinear down-sampling within 2 %).
+bool prefer_packed(const PlanSettings &s, int64_t slots_packed)
 {
-    if (slots_packed < 0) return false;
-    if (const char *e = std::getenv("SMM_PACKED")) return e[0] == '1';
-    return true;
+    return slots_packed >= 0 && s.packed != 0;
 }
 
-void build_plan(const HostCsr &csr, int32_t force_lpr, int32_t force_kpl, int32_t nct, bool ref_order, HostPlan &plan,
-                const std::vector<int32_t> *subset)
+void build_plan(const HostCsr &csr, int32_t force_lpr, int32_t force_kpl, int32_t nct, bool ref_order,
+                const PlanSettings &s, HostPlan &plan, const std::vector<int32_t> *subset)
 {
     const bool packed = force_lpr == -1;       // -1: packed layout requested (see smm_create_levels)
     if (packed) { force_lpr = 0; force_kpl = 0; }
-    build_plan_rows(csr, force_lpr, force_kpl, nct, subset, packed, ref_order, plan);
+    build_plan_rows(csr, force_lpr, force_kpl, nct, subset, packed, ref_order, s, plan);
     if (plan.lpr == 0 || csr.col.empty() || (subset && subset->empty())) return;
     // natural order good enough: footprints within 30 % of the columns actually touched
     if (plan.ok && plan_cost(plan) <= 1.3 * static_cast<double>(plan.sum_tile_cols)) return;
@@ -694,7 +670,7 @@ void build_plan(const HostCsr &csr, int32_t force_lpr, int32_t force_kpl, int32_
     }
     std::stable_sort(order.begin(), order.end(), [&](int32_t x, int32_t y) { return key[x] < key[y]; });
     HostPlan alt;
-    build_plan_rows(csr, force_lpr, force_kpl, nct, &order, packed, ref_order, alt);
+    build_plan_rows(csr, force_lpr, force_kpl, nct, &order, packed, ref_order, s, alt);
     if (alt.ok && (!plan.ok || plan_cost(alt) < 0.8 * plan_cost(plan))) plan = std::move(alt);
 }
 
@@ -705,6 +681,19 @@ void long_rows(const HostCsr &csr, std::vector<int32_t> &long_rows_out, std::vec
     short_rows_out.clear();
     for (int64_t r = 0; r < csr.n_dst; ++r)
         (csr.rowptr[r + 1] - csr.rowptr[r] > kSubRows * kSubLinks ? long_rows_out : short_rows_out).push_back(static_cast<int32_t>(r));
+}
+
+void parallel_for(int threads, int64_t n, const std::function<void(int64_t)> &fn)
+{
+    if (threads <= 1) {
+        for (int64_t i = 0; i < n; ++i) fn(i);
+        return;
+    }
+    std::atomic<int64_t> next{0};
+    std::vector<std::thread> pool;
+    for (int t = 0; t < threads; ++t)
+        pool.emplace_back([&]() { for (int64_t i = next.fetch_add(1); i < n; i = next.fetch_add(1)) fn(i); });
+    for (auto &th : pool) th.join();
 }
 
 void build_compact(const HostCsr &csr, int32_t block_cols, CompactPlan &out)

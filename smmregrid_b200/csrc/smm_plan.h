@@ -1,10 +1,12 @@
 // smm_plan.h -- host-side construction of the device operator from CDO link arrays.
 #pragma once
 #include <cstdint>
+#include <functional>
 #include <string>
 #include <vector>
 
 #include "smm_common.h"
+#include "smm_tuning.h"
 
 namespace smm {
 
@@ -66,7 +68,7 @@ struct HostPlan {
 
 // Picks (lanes per row, links per lane) for a maximum row length; false if no staged
 // configuration can hold it.
-bool choose_lanes(int32_t max_row_nnz, int32_t &lpr, int32_t &kpl);
+bool choose_lanes(const PlanSettings &s, int32_t max_row_nnz, int32_t &lpr, int32_t &kpl);
 
 // force_lpr/force_kpl > 0 impose a configuration shared by all levels of a 3-D weight set.
 // nct = consumer threads per CTA (256 or 512).
@@ -78,19 +80,22 @@ bool choose_lanes(int32_t max_row_nnz, int32_t &lpr, int32_t &kpl);
 // ref_order: place the links for the reference's summation order (see staged_kernel ORD) instead of
 // the bank-conflict-minimising free placement of the fast sums.
 // subset (ascending row ids): tile only these rows (one part of a split plan).
-void build_plan(const HostCsr &csr, int32_t force_lpr, int32_t force_kpl, int32_t nct, bool ref_order, HostPlan &plan,
-                const std::vector<int32_t> *subset = nullptr);
+void build_plan(const HostCsr &csr, int32_t force_lpr, int32_t force_kpl, int32_t nct, bool ref_order,
+                const PlanSettings &s, HostPlan &plan, const std::vector<int32_t> *subset = nullptr);
 void long_rows(const HostCsr &csr, std::vector<int32_t> &long_rows_out, std::vector<int32_t> &short_rows_out);
 
 // Packed-rows layout (one thread owns up to 4 short rows): link slots it would spend on `csr`
 // (-1: a row does not fit), and whether to use it.
 int64_t packed_slots(const HostCsr &csr);
-bool prefer_packed(int64_t slots_packed);
+bool prefer_packed(const PlanSettings &s, int64_t slots_packed);
 
 // Consumer threads per CTA for a weight set: 512 (one CTA per SM, tiles twice as long, longer TMA
 // segments: +4 % on C4, +5 % on C2) when that still leaves at least one tile per SM, else 256.
-// SMM_CONSUMER_THREADS=256|512 overrides.
-int32_t default_consumer_threads(int64_t n_dst, int32_t lpr, int32_t sm_count);
+int32_t default_consumer_threads(const PlanSettings &s, int64_t n_dst, int32_t lpr, int32_t sm_count);
+
+// Runs fn(0) .. fn(n - 1) on `threads` host threads, each taking the next index in turn (on the
+// calling thread alone when threads <= 1).
+void parallel_for(int threads, int64_t n, const std::function<void(int64_t)> &fn);
 
 // ---- on-disk cache of the operator construction (smm_plan_cache.cpp)
 struct PlanCacheKey { uint64_t h[2] = {0, 0}; };
@@ -98,7 +103,7 @@ struct PlanCacheKey { uint64_t h[2] = {0, 0}; };
 PlanCacheKey plan_cache_key(int32_t n_levels, const int64_t *link_length, int64_t nl_max, int64_t n_src,
                             int64_t n_dst, const int32_t *src_address, const int32_t *dst_address,
                             const double *remap_matrix, int32_t num_wgts, int32_t index_base,
-                            int32_t summation, int32_t sm_count);
+                            int32_t summation, int32_t sm_count, const PlanSettings &s);
 // false = miss (absent, stale or damaged file): build as usual.  ref_order = the summation order of
 // the weight set, stored in the file as the handle's own value
 bool plan_cache_load(const std::string &dir, const PlanCacheKey &key, int32_t n_levels, int64_t n_src,

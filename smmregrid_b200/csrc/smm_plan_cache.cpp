@@ -10,7 +10,6 @@
 // with a hash of everything before it: any mismatch (magic, version, sizes, content, truncated file)
 // is treated as a miss, so a damaged payload never reaches the device.
 #include <cstdio>
-#include <cstdlib>
 #include <cstring>
 #include <functional>
 #include <thread>
@@ -52,7 +51,6 @@ struct Hasher {
         }
     }
     template <typename T> void pod(const T &v) { bytes(&v, sizeof(T)); }
-    void str(const char *s) { const uint64_t l = s ? std::strlen(s) : 0; pod(l); if (l) bytes(s, l); }
     void finish(uint64_t out[2])
     {
         uint64_t a = mix(mix(h[0], h[1]), n), b = mix(mix(h[2], h[3]), ~n);
@@ -141,16 +139,15 @@ std::string cache_file(const std::string &dir, const PlanCacheKey &key)
 PlanCacheKey plan_cache_key(int32_t n_levels, const int64_t *link_length, int64_t nl_max, int64_t n_src,
                             int64_t n_dst, const int32_t *src_address, const int32_t *dst_address,
                             const double *remap_matrix, int32_t num_wgts, int32_t index_base,
-                            int32_t summation, int32_t sm_count)
+                            int32_t summation, int32_t sm_count, const PlanSettings &s)
 {
     Hasher hs;
     hs.bytes(kMagic, sizeof(kMagic));
     hs.pod(n_levels); hs.pod(nl_max); hs.pod(n_src); hs.pod(n_dst); hs.pod(num_wgts); hs.pod(index_base);
     hs.pod(summation); hs.pod(sm_count);
-    // plan-shaping experiment switches are part of the key
-    for (const char *env : {"SMM_CONSUMER_THREADS", "SMM_PACKED", "SMM_FORCE_LANES", "SMM_SPLIT", "SMM_ORDLONG",
-                            "SMM_ORD_ROWS", "SMM_SUMMATION"})
-        hs.str(std::getenv(env));
+    // the plan-shaping switches as the planner reads them (plan_threads does not change a plan)
+    hs.pod(s.force_lpr); hs.pod(s.force_kpl); hs.pod(s.consumer_threads); hs.pod(s.packed); hs.pod(s.split);
+    hs.pod(s.ordlong); hs.pod(s.ord_rows); hs.pod(s.summation);
     for (int32_t i = 0; i < n_levels; ++i) {
         const int64_t nl = link_length[i], o = static_cast<int64_t>(i) * nl_max;
         hs.pod(nl);

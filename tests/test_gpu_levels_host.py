@@ -635,7 +635,9 @@ def _host_plan_info(lib, op, cache_dir, env, summation=None):
 
 
 @pytest.mark.parametrize("switch,value", [("SMM_SPLIT", "0"), ("SMM_ORDLONG", "0"), ("SMM_ORD_ROWS", "64"),
-                                          ("SMM_SUMMATION", "fast"), ("SMM_SUMMATION", "reference")])
+                                          ("SMM_SUMMATION", "fast"), ("SMM_SUMMATION", "reference"),
+                                          ("SMM_FORCE_LANES", "8,16"), ("SMM_CONSUMER_THREADS", "512"),
+                                          ("SMM_PACKED", "0")])
 def test_plan_cache_key_covers_plan_switches(smm_lib, tmp_path, switch, value):
     """A switch that shapes the plan, changed between two builds, is a cache miss; the file
     written under it then serves exactly the plan a build without the cache gives."""

@@ -34,7 +34,7 @@ import pytest
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 LAUNCH_CUH = os.path.join(ROOT, "smmregrid_b200", "csrc", "smm_launch.cuh")
 
-# read by smm_create (per handle) | read once per process (static const in the launch code)
+# smm_tuning.h: PlanSettings, read by each smm_create | LaunchSettings, read once per process
 CREATE_ENV = ("SMM_FORCE_LANES", "SMM_PACKED", "SMM_CONSUMER_THREADS", "SMM_SUMMATION", "SMM_ORDLONG",
               "SMM_ORD_ROWS", "SMM_SPLIT")
 PROCESS_ENV = ("SMM_ROWS_PER_STAGE", "SMM_MAX_STAGES", "SMM_MIN_ROWS_PER_ITEM", "SMM_WAVES", "SMM_ORD_TPR",
