@@ -31,9 +31,11 @@ def nan_variation_count(field, axis: int, device=None) -> int:
         t = field if field.is_cuda else field.to(f"cuda:{0 if device is None else device}")
     else:
         a = np.asarray(field)
-        if a.dtype not in (np.float32, np.float64):
+        if a.dtype not in (np.float16, np.float32, np.float64):
             return 0                                        # integer data has no NaN (isnull is all False)
         t = torch.from_numpy(np.ascontiguousarray(a)).to(f"cuda:{0 if device is None else device}")
+    if t.dtype in (torch.float16, torch.bfloat16):
+        t = t.to(torch.float32)                             # widening keeps NaN-ness exactly; the kernel reads f32 / f64
     if t.dtype not in (torch.float32, torch.float64):
         return 0
     t = t.contiguous()

@@ -112,7 +112,9 @@ def test_named_configs(smm_lib, oracle, cuda, cfg, scale, B, nan_mode):
 
 
 def test_mask_sum_matches_oracle(smm_lib, oracle, cuda):
-    """mask_tensordot: bit-exact 0/1 destination mask, including sums that land on 0.5."""
+    """mask_tensordot: bit-exact 0/1 destination mask and any-masked flag on a conservative
+    operator.  (None of its row sums lands on 0.5: the boundary is tested in
+    test_gpu_init_kernels.py.)"""
     from smmregrid_b200 import _lib, synth
     w = synth.conservative_latlon(360, 180, 36, 18)
     n_src, n_dst = 360 * 180, 36 * 18
