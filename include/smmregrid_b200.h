@@ -39,6 +39,8 @@ extern "C" {
 #define SMM_F64 1
 #define SMM_I16 2           /* x_dtype only (smm_apply*): CF-packed 16-bit integers, decoded inside the */
                             /* kernels as smm_apply_opts.decode says (smm_decode)                       */
+#define SMM_F16 3           /* x_dtype only (smm_apply*): IEEE binary16, read as its float32 widening   */
+#define SMM_BF16 4          /* x_dtype only (smm_apply*): bfloat16, read as its float32 widening        */
 
 /* Which kernel family serves a level (smm_info.kernel). */
 #define SMM_KERNEL_STAGED 1 /* TMA-staged source footprint, register-resident weights     */
@@ -215,6 +217,27 @@ int smm_set_dst_mask(smm_handle *h, int32_t level, const int32_t *dst_grid_imask
  *   y [B, n_dst] row stride ldy, dtype y_dtype (SMM_F64 = the reference's result_type;
  *   SMM_F32 rounds the float64 result once at the store).
  * x and y are DEVICE pointers; the launch is asynchronous on `stream`.
+ *
+ * Half-precision sources (x_dtype SMM_F16 / SMM_BF16; y_dtype stays SMM_F32 or SMM_F64, a half
+ * y_dtype is SMM_ERR_DTYPE).  The kernels read the 2-byte values and widen each one exactly to
+ * float32; from there on the float32 semantics apply unchanged: non-finite -> 1e20 IN FLOAT32
+ * (1.00000002004e20 as a float64), float64 products and sums, the masks and the `> 1e19` rule,
+ * and the renormalising extension excludes non-finite sources.  Contract: every result of
+ * smm_apply, smm_apply_levels, smm_apply_host and smm_apply_levels_host with half data is
+ * bit-identical to the same call on the float32 widening of that data (same B, row strides and
+ * options; the float32 slab 16-byte aligned), for every summation order and kernel option.  The
+ * kernel family is the one float32 data would get; where that family is the staged kernel but the
+ * 2-byte rows cannot be staged (x not 16-byte aligned, a row stride or n_src that is not a
+ * multiple of 8), the rows are widened into float32 chunks from the handle's stream-ordered pool
+ * and applied there (SMM_ERR_ALLOC if the pool cannot provide a chunk).  Forced SMM_KERNEL_GATHER
+ * reads the 2-byte data directly, and so does forced SMM_KERNEL_COMPACT on gather-family levels;
+ * a level with a staged plan stays staged under SMM_KERNEL_COMPACT, as float32 data does, and so
+ * takes the float32 chunks like an automatic call when its 2-byte rows cannot be staged.  The
+ * chunks hold up to 256 MB of float32 rows; the pool keeps that memory for later calls (one chunk
+ * per stream applying at the same time) until the handle is destroyed.  One exception: when the pool cannot
+ * provide the compact path's transposed buffer, the path falls back to direct gathers; that
+ * buffer is half the size for 2-byte data, so under memory pressure half and float32 data may land
+ * on different sides of that fallback and then differ in the last bits of fast sums.
  */
 int smm_apply(const smm_handle *h, int32_t level,
               const void *x, int32_t x_dtype, int64_t B, int64_t ldx,
@@ -269,7 +292,9 @@ int smm_apply_levels_host(const smm_handle *h, int32_t n_sel, const int32_t *lev
  * positions whose NaN-ness changes somewhere along the axis -- the reference's
  * `isnull().astype("int8").diff(dim).astype(bool).any(dim).sum()`.  A dimension "has NaN
  * variation" (and becomes a mask dimension, regrid.py:630-653) when the count is > 0.
- * NaN only, as isnull: +-inf does not count.  Synchronous on `stream`.
+ * NaN only, as isnull: +-inf does not count.  Synchronous on `stream`.  x_dtype SMM_F32 or
+ * SMM_F64 only (anything else, SMM_F16 / SMM_BF16 included, is SMM_ERR_DTYPE: widen half data first,
+ * which keeps its NaN-ness exactly).
  */
 int smm_nan_variation(const void *x, int32_t x_dtype, int64_t outer, int64_t n_axis, int64_t inner,
                       int64_t *count_out, smm_stream_t stream);

@@ -16,7 +16,7 @@ import sys
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 OBJ = os.path.join(ROOT, "smmregrid_b200", "build")
 KERNELS = [
-    ("smm_inst_f32_f64.o", "ordered_kernel<float, double, 64>", "C4 with reference-order sums (thread per row)"),
+    ("smm_inst_f32_f64.o", "ordered_kernel<float, double, 64, 1>", "C4 with reference-order sums (thread per row)"),
     ("smm_inst_f32_f64.o", "staged_kernel<float, double, 8, 14, 512, false, false>", "C4 / bench headline"),
     ("smm_inst_f32_f64.o", "staged_kernel<float, double, 2, 14, 512, false, false>", "C2"),
     ("smm_inst_f32_f64.o", "staged_kernel<float, double, 1, 16, 256, true, false>", "C3 (packed rows)"),
@@ -30,16 +30,32 @@ KERNELS = [
     ("smm_inst_i16f32_f64.o", "staged_kernel<smm::I16F32, double, 8, 14, 512, false, false>", "C4, int16 -> float32"),
     ("smm_inst_i16f32_f64.o", "staged_kernel<smm::I16F32, double, 2, 14, 512, false, false>", "C2, int16 -> float32"),
     ("smm_inst_i16f32_f64.o", "staged_kernel<smm::I16F32, double, 1, 16, 256, true, false>", "C3, int16 -> float32"),
+    # float16 / bfloat16 sources (per link: LDS.U16 + F2F.F64.F16, or LDS.U16 + SHF + F2F.F64.F32)
+    ("smm_inst_f16_f64.o", "ordered_kernel<smm::F16, double, 64, 1>", "C4 reference order, float16"),
+    ("smm_inst_f16_f64.o", "staged_kernel<smm::F16, double, 8, 14, 512, false, false>", "C4, float16"),
+    ("smm_inst_f16_f64.o", "staged_kernel<smm::F16, double, 2, 14, 512, false, false>", "C2, float16"),
+    ("smm_inst_f16_f64.o", "staged_kernel<smm::F16, double, 1, 16, 256, true, false>", "C3, float16"),
+    ("smm_inst_f16_f64.o", "staged_kernel<smm::F16, double, 1, 16, 256, true, true>", "bicubic-like, float16"),
+    ("smm_inst_f32_f64.o", "staged_kernel<float, double, 8, 16, 256, false, true>", "reference-order lane chains"),
+    ("smm_inst_f16_f64.o", "staged_kernel<smm::F16, double, 8, 16, 256, false, true>", "the same, float16 (through float32)"),
+    ("smm_inst_f16_f64.o", "gather_kernel<smm::F16, double, 4, false>", "C5dis few batch rows, float16"),
+    ("smm_inst_f16_f64.o", "compact_apply_kernel<smm::F16, double>", "C5dis pass 2, float16"),
+    ("smm_inst_bf16_f64.o", "staged_kernel<smm::BF16, double, 8, 14, 512, false, false>", "C4, bfloat16"),
+    ("smm_inst_bf16_f64.o", "staged_kernel<smm::BF16, double, 2, 14, 512, false, false>", "C2, bfloat16"),
+    ("smm_inst_bf16_f64.o", "staged_kernel<smm::BF16, double, 1, 16, 256, true, false>", "C3, bfloat16"),
 ]
 MNEMONICS = ["UBLKCP", "UTMALDG", "UTMASTG", "SYNCS", "LDGSTS", "LDS", "F2F", "DFMA", "DMUL", "DADD", "IMAD", "LEA", "SHFL",
-             "STG", "LDG", "USETMAXREG", "FMUL", "FADD", "ISETP", "FSEL", "LOP3", "I2F"]
+             "STG", "LDG", "USETMAXREG", "FMUL", "FADD", "ISETP", "FSEL", "LOP3", "I2F", "SHF", "HADD2"]
+# full opcodes of the source conversions (a per-link F2F.F64.F16 and no HADD2.F32 for float16)
+FULL = ["F2F.F64.F32", "F2F.F64.F16", "HADD2.F32"]
 
 
 def main():
     print("# static SASS instruction counts per kernel instantiation (cuobjdump -sass, sm_100a)")
     print("# UBLKCP = cp.async.bulk (1-D TMA), UTMALDG/UTMASTG = tensor-map TMA, SYNCS = mbarrier ops,")
     print("# 'U*' = instructions on the uniform datapath (loop control, stage addressing)")
-    print(f"{'kernel':<66} " + " ".join(f"{m:>8}" for m in MNEMONICS) + f" {'U*':>6} {'total':>6}  use")
+    print(f"{'kernel':<66} " + " ".join(f"{m:>8}" for m in MNEMONICS) + f" {'U*':>6} {'total':>6} " +
+          " ".join(f"{m:>11}" for m in FULL) + "  use")
     for obj, name, use in KERNELS:
         out = subprocess.run(["cuobjdump", "-sass", os.path.join(OBJ, obj)], capture_output=True, text=True).stdout
         # split per function
@@ -61,7 +77,9 @@ def main():
             base = op.split(".")[0]
             cnt[base] += 1
         uni = sum(v for k, v in cnt.items() if k.startswith("U") and k not in ("UBLKCP", "UTMALDG", "UTMASTG", "USETMAXREG"))
-        print(f"{name:<66} " + " ".join(f"{cnt.get(m, 0):>8}" for m in MNEMONICS) + f" {uni:>6} {len(ops):>6}  {use}")
+        full = collections.Counter(ops)
+        print(f"{name:<66} " + " ".join(f"{cnt.get(m, 0):>8}" for m in MNEMONICS) + f" {uni:>6} {len(ops):>6} " +
+              " ".join(f"{full.get(m, 0):>11}" for m in FULL) + f"  {use}")
 
 
 if __name__ == "__main__":

@@ -11,7 +11,7 @@ import os
 from . import _build
 
 SMM_OK, SMM_ERR_INVALID, SMM_ERR_RANGE, SMM_ERR_CUDA, SMM_ERR_ALLOC, SMM_ERR_DTYPE = range(6)
-SMM_F32, SMM_F64, SMM_I16 = 0, 1, 2
+SMM_F32, SMM_F64, SMM_I16, SMM_F16, SMM_BF16 = 0, 1, 2, 3, 4
 SMM_KERNEL_STAGED, SMM_KERNEL_GATHER, SMM_KERNEL_COMPACT = 1, 2, 3
 KERNEL_NAMES = {SMM_KERNEL_STAGED: "staged", SMM_KERNEL_GATHER: "gather"}
 KERNEL_CODES = {None: 0, "auto": 0, "staged": SMM_KERNEL_STAGED, "gather": SMM_KERNEL_GATHER,

@@ -34,6 +34,10 @@ SMM_DECLARE_LAUNCHERS(extern, I16F32, float)
 SMM_DECLARE_LAUNCHERS(extern, I16F32, double)
 SMM_DECLARE_LAUNCHERS(extern, I16F64, float)
 SMM_DECLARE_LAUNCHERS(extern, I16F64, double)
+SMM_DECLARE_LAUNCHERS(extern, F16, float)
+SMM_DECLARE_LAUNCHERS(extern, F16, double)
+SMM_DECLARE_LAUNCHERS(extern, BF16, float)
+SMM_DECLARE_LAUNCHERS(extern, BF16, double)
 
 namespace {
 thread_local std::string g_err;
@@ -346,13 +350,20 @@ int build_host_operator(int32_t n_levels, const int64_t *link_length, int64_t nl
          ? ((opt.dec_dtype == SMM_F32)                                                                        \
                 ? (y_dtype == SMM_F32 ? FN<I16F32, float>(__VA_ARGS__) : FN<I16F32, double>(__VA_ARGS__))     \
                 : (y_dtype == SMM_F32 ? FN<I16F64, float>(__VA_ARGS__) : FN<I16F64, double>(__VA_ARGS__)))    \
+     : (x_dtype == SMM_F16) ? (y_dtype == SMM_F32 ? FN<F16, float>(__VA_ARGS__) : FN<F16, double>(__VA_ARGS__))    \
+     : (x_dtype == SMM_BF16) ? (y_dtype == SMM_F32 ? FN<BF16, float>(__VA_ARGS__) : FN<BF16, double>(__VA_ARGS__)) \
      : (x_dtype == SMM_F32 && y_dtype == SMM_F32) ? FN<float, float>(__VA_ARGS__)                             \
      : (x_dtype == SMM_F32 && y_dtype == SMM_F64) ? FN<float, double>(__VA_ARGS__)                            \
      : (x_dtype == SMM_F64 && y_dtype == SMM_F32) ? FN<double, float>(__VA_ARGS__)                            \
                                                   : FN<double, double>(__VA_ARGS__))
 
 // bytes of one x element as it sits in memory (SMM_I16: the raw 16 bits)
-size_t x_elem_bytes(int32_t x_dtype) { return x_dtype == SMM_I16 ? 2 : x_dtype == SMM_F32 ? 4 : 8; }
+size_t x_elem_bytes(int32_t x_dtype)
+{
+    return (x_dtype == SMM_I16 || x_dtype == SMM_F16 || x_dtype == SMM_BF16) ? 2 : x_dtype == SMM_F32 ? 4 : 8;
+}
+
+bool is_half(int32_t x_dtype) { return x_dtype == SMM_F16 || x_dtype == SMM_BF16; }
 
 // Batch rows per work item.  A work item pays a fixed prologue (its tile's register image,
 // barriers: `prologue_us`) and the launch pays about half an item of tail per wave, so with an
@@ -428,31 +439,37 @@ int resolve_opts(const smm_apply_opts *o, int32_t x_dtype, ApplyOpts &out)
     return SMM_OK;
 }
 
+// The handle's stream-ordered pool for transient device buffers (created on first use); null when
+// the device has no stream-ordered pools.
+cudaMemPool_t handle_pool(const smm_handle *h)
+{
+    std::lock_guard<std::mutex> lock(h->pool_mu);
+    if (!h->pool) {
+        cudaMemPoolProps props{};
+        props.allocType = cudaMemAllocationTypePinned;
+        props.location.type = cudaMemLocationTypeDevice;
+        props.location.id = h->device;
+        uint64_t keep = UINT64_MAX;
+        if (cudaMemPoolCreate(&h->pool, &props) != cudaSuccess ||
+            cudaMemPoolSetAttribute(h->pool, cudaMemPoolAttrReleaseThreshold, &keep) != cudaSuccess) {
+            cudaGetLastError();
+            if (h->pool) { cudaMemPoolDestroy(h->pool); h->pool = nullptr; }
+        }
+    }
+    return h->pool;
+}
+
 // Two-pass apply of one gather-family level (see compact_kernel).  The transposed buffer XT comes
 // from the handle's stream-ordered pool, so concurrent applies on other streams stay independent.
 int launch_compact(const smm_handle *h, const LevelDev &L, const JobSpec &sp, int32_t x_dtype, int32_t y_dtype,
                    int64_t B, int64_t xbs, int64_t ybs, double area_min, const ApplyOpts &opt, cudaStream_t st)
 {
-    {
-        std::lock_guard<std::mutex> lock(h->pool_mu);
-        if (!h->pool) {
-            cudaMemPoolProps props{};
-            props.allocType = cudaMemAllocationTypePinned;
-            props.location.type = cudaMemLocationTypeDevice;
-            props.location.id = h->device;
-            uint64_t keep = UINT64_MAX;
-            if (cudaMemPoolCreate(&h->pool, &props) != cudaSuccess ||
-                cudaMemPoolSetAttribute(h->pool, cudaMemPoolAttrReleaseThreshold, &keep) != cudaSuccess) {
-                cudaGetLastError();
-                if (h->pool) { cudaMemPoolDestroy(h->pool); h->pool = nullptr; }
-                return kCompactUnavailable;          // no stream-ordered pools here: direct gathers instead
-            }
-        }
-    }
+    cudaMemPool_t pool = handle_pool(h);
+    if (!pool) return kCompactUnavailable;           // no stream-ordered pools here: direct gathers instead
     void *xt = nullptr;
     const size_t sx = x_elem_bytes(x_dtype);
     const size_t xt_bytes = std::max<size_t>(static_cast<size_t>(L.touched), 1) * kCompactBC * sx;
-    if (cudaMallocFromPoolAsync(&xt, xt_bytes, h->pool, st) != cudaSuccess) {
+    if (cudaMallocFromPoolAsync(&xt, xt_bytes, pool, st) != cudaSuccess) {
         cudaGetLastError();
         return kCompactUnavailable;                  // not enough memory for the transposed buffer
     }
@@ -463,20 +480,65 @@ int launch_compact(const smm_handle *h, const LevelDev &L, const JobSpec &sp, in
 
 int launch_jobs(const smm_handle *h, const std::vector<JobSpec> &specs, int32_t x_dtype,
                 int32_t y_dtype, int64_t B, int64_t xbs, int64_t ybs, double area_min,
+                const ApplyOpts &opt, cudaStream_t st);
+
+constexpr int64_t kWidenBytes = int64_t{256} << 20;     // float32 rows widened per chunk (launch_widened)
+
+// The float32 path of one half-source level on float32 copies of its rows, widened exactly into a
+// buffer from the handle's pool, up to kWidenBytes at a time (see launch_jobs).
+int launch_widened(const smm_handle *h, const JobSpec &s, int32_t x_dtype, int32_t y_dtype, int64_t B, int64_t xbs,
+                   int64_t ybs, double area_min, const ApplyOpts &opt, cudaStream_t st)
+{
+    const int64_t n = h->levels[s.level].n_src;          // a multiple of 4 here: float32 rows stay 16-byte aligned
+    const int64_t rows = std::max<int64_t>(1, std::min<int64_t>({B, kWidenBytes / (4 * n), 65535}));
+    cudaMemPool_t pool = handle_pool(h);
+    float *buf = nullptr;
+    if (!pool || cudaMallocFromPoolAsync(reinterpret_cast<void **>(&buf), static_cast<size_t>(rows * n) * 4, pool, st) != cudaSuccess) {
+        cudaGetLastError();
+        return fail(SMM_ERR_ALLOC, "no device memory for the float32 copy of half-precision rows that cannot be staged");
+    }
+    const size_t sy = y_dtype == SMM_F32 ? 4 : 8;
+    int rc = SMM_OK;
+    for (int64_t b0 = 0; b0 < B && rc == SMM_OK; b0 += rows) {
+        const int64_t nb = std::min(rows, B - b0);
+        const uint16_t *x = static_cast<const uint16_t *>(s.x) + b0 * xbs;
+        const dim3 grid(static_cast<unsigned>(std::min<int64_t>((n + 255) / 256, 1024)), static_cast<unsigned>(nb));
+        if (x_dtype == SMM_BF16) widen16_kernel<true><<<grid, 256, 0, st>>>(x, xbs, n, buf, n);
+        else widen16_kernel<false><<<grid, 256, 0, st>>>(x, xbs, n, buf, n);
+        const cudaError_t e = cudaGetLastError();
+        if (e != cudaSuccess) { rc = fail(SMM_ERR_CUDA, std::string("widen16_kernel: ") + cudaGetErrorString(e)); break; }
+        smm_count_launches(1);
+        const std::vector<JobSpec> w{JobSpec{s.level, buf, static_cast<char *>(s.y) + static_cast<size_t>(b0 * ybs) * sy, s.masked}};
+        rc = launch_jobs(h, w, SMM_F32, y_dtype, nb, n, ybs, area_min, opt, st);
+    }
+    cudaFreeAsync(buf, st);
+    return rc;
+}
+
+int launch_jobs(const smm_handle *h, const std::vector<JobSpec> &specs, int32_t x_dtype,
+                int32_t y_dtype, int64_t B, int64_t xbs, int64_t ybs, double area_min,
                 const ApplyOpts &opt, cudaStream_t st)
 {
     if (B == 0 || specs.empty()) return SMM_OK;
     const size_t sx = x_elem_bytes(x_dtype);
+    // Half sources get the kernel family float32 data would get: their results are the float32 path's
+    // bit for bit, and the fast sums of the families differ in the last bits.  So every choice of a
+    // family is made with the element size `sd` of the float32 slab of the same B and ldx, at a
+    // 16-byte aligned address (plus the level's offset in the caller's x); stages, rows per stage and
+    // work items, which change no value, are sized with the real 2 bytes.
+    const bool half = is_half(x_dtype);
+    const size_t sd = half ? 4 : sx;
     const bool ord = h->ref_order;
     // shared memory a staged launch needs for `nstages` stages of one batch row each (`image` = the
     // link image of ordered-long plans: kpl x nct x (8 + 4) bytes)
     auto image_bytes = [](const LevelDev &L) -> size_t {
         return L.ordlong ? round_up(static_cast<size_t>(L.kpl) * L.nct * 12, 128) : 0;
     };
-    auto staged_smem = [&](size_t max_segs, size_t max_elems, size_t nstages, size_t image = 0) {
-        return kSmemHeader + round_up(max_segs * sizeof(Seg), 128) + image + nstages * round_up(max_elems * sx, 128);
+    auto staged_smem = [&](size_t max_segs, size_t max_elems, size_t nstages, size_t image, size_t es) {
+        return kSmemHeader + round_up(max_segs * sizeof(Seg), 128) + image + nstages * round_up(max_elems * es, 128);
     };
     std::vector<JobSpec> staged, gather, gather_lists;      // gather_lists: the long rows of split plans
+    std::vector<JobSpec> widened;                           // half sources staged through a float32 copy
     for (const JobSpec &s : specs) {
         const LevelDev &L = h->levels[s.level];
         if (s.masked && !L.has_imask)
@@ -489,18 +551,25 @@ int launch_jobs(const smm_handle *h, const std::vector<JobSpec> &specs, int32_t 
         // the renormalising extension is not implemented for packed-rows and ordered-long plans: gather kernel
         ok = ok && !((L.packed || L.ordlong) && opt.renorm_min_valid >= 0.0);
         // TMA bulk copies need 16-byte aligned rows and lengths
-        ok = ok && (reinterpret_cast<uintptr_t>(s.x) % 16 == 0) && ((xbs * sx) % 16 == 0) &&
-             ((L.n_src * sx) % 16 == 0);
+        const bool aligned = (reinterpret_cast<uintptr_t>(s.x) % 16 == 0) && ((xbs * sx) % 16 == 0) &&
+                             ((L.n_src * sx) % 16 == 0);
+        ok = ok && (half ? (s.x_off * 4) % 16 == 0 && (xbs * 4) % 16 == 0 && (L.n_src * 4) % 16 == 0 : aligned);
         // at least two stages must fit
-        ok = ok && staged_smem(L.max_segs, L.max_elems, 2, image_bytes(L)) <= h->smem_optin;
+        ok = ok && staged_smem(L.max_segs, L.max_elems, 2, image_bytes(L), sd) <= h->smem_optin;
         if (!ok && opt.kernel == SMM_KERNEL_STAGED)
             return fail(SMM_ERR_INVALID, "staged kernel forced but unavailable for level " +
                                              std::to_string(s.level) + ": " +
                                              (L.staged ? std::string("slab alignment / footprint size")
                                                        : L.why_not_staged));
+        // a half level that float32 would stage but whose 2-byte rows cannot be (x not 16-byte aligned,
+        // ldx or n_src not a multiple of 8) takes the float32 path on widened rows: rows never depend
+        // on the batching, so the chunked float32 applies give the float32 results
+        if (ok && !aligned) { widened.push_back(s); continue; }
         (ok ? staged : gather).push_back(s);
         if (ok && L.n_gather_rows > 0) gather_lists.push_back(s);
     }
+    for (const JobSpec &s : widened)
+        if (const int rc = launch_widened(h, s, x_dtype, y_dtype, B, xbs, ybs, area_min, opt, st)) return rc;
 
     ApplyArgs a{};
     a.B = B; a.x_bstride = xbs; a.y_bstride = ybs; a.remap_area_min = area_min;
@@ -533,7 +602,7 @@ int launch_jobs(const smm_handle *h, const std::vector<JobSpec> &specs, int32_t 
         for (; g1 < staged.size() && g1 - g0 < staged_per; ++g1) {
             const LevelDev &L = h->levels[staged[g1].level];
             const size_t ms = std::max<size_t>(max_segs, L.max_segs), me = std::max<size_t>(max_elems, L.max_elems);
-            if (g1 > g0 && staged_smem(ms, me, 2, image_bytes(L)) > h->smem_optin) break;
+            if (g1 > g0 && staged_smem(ms, me, 2, image_bytes(L), sx) > h->smem_optin) break;
             max_segs = ms; max_elems = me;
             tiles_total += L.ntiles;
             lpr = L.lpr; kpl = L.kpl; nct = L.nct; packed = L.packed; ordl = L.ordlong;
@@ -616,7 +685,7 @@ int launch_jobs(const smm_handle *h, const std::vector<JobSpec> &specs, int32_t 
             // bytes at the streaming rate.  Runs of fewer than 16 batch values are not worth it.
             const double gather_cost = static_cast<double>(L.nnz) * 120.0;
             const double compact_cost = 1.2 * (static_cast<double>(L.n_src) + static_cast<double>(L.touched) +
-                                               static_cast<double>(L.nnz)) * static_cast<double>(sx);
+                                               static_cast<double>(L.nnz)) * static_cast<double>(sd);
             bool use = L.rcol && opt.renorm_min_valid < 0.0 && opt.kernel != SMM_KERNEL_GATHER;
             if (opt.kernel != SMM_KERNEL_COMPACT) use = use && B >= 16 && gather_cost > compact_cost;
             if (!use) { plain.push_back(sp); continue; }
@@ -736,8 +805,10 @@ void parallel_copy_rows(char *dst, size_t dst_stride, const char *src, size_t sr
 
 int check_dtypes(int32_t x_dtype, int32_t y_dtype)
 {
-    if ((x_dtype != SMM_F32 && x_dtype != SMM_F64 && x_dtype != SMM_I16) || (y_dtype != SMM_F32 && y_dtype != SMM_F64))
-        return fail(SMM_ERR_DTYPE, "x_dtype must be SMM_F32 (0), SMM_F64 (1) or SMM_I16 (2), y_dtype SMM_F32 or SMM_F64");
+    if ((x_dtype != SMM_F32 && x_dtype != SMM_F64 && x_dtype != SMM_I16 && !is_half(x_dtype)) ||
+        (y_dtype != SMM_F32 && y_dtype != SMM_F64))
+        return fail(SMM_ERR_DTYPE, "x_dtype must be SMM_F32 (0), SMM_F64 (1), SMM_I16 (2), SMM_F16 (3) or SMM_BF16 (4), "
+                                   "y_dtype SMM_F32 or SMM_F64");
     return SMM_OK;
 }
 
@@ -1148,6 +1219,7 @@ int smm_apply_levels(const smm_handle *h, int32_t n_sel, const int32_t *level_in
         s.x = static_cast<const char *>(x) + static_cast<int64_t>(i) * x_level_stride * static_cast<int64_t>(sx);
         s.y = static_cast<char *>(y) + static_cast<int64_t>(i) * y_level_stride * static_cast<int64_t>(sy);
         s.masked = masked ? (masked[i] ? 1 : 0) : 0;
+        s.x_off = static_cast<int64_t>(i) * x_level_stride;
         specs.push_back(s);
     }
     DeviceGuard g(h->device);
@@ -1208,7 +1280,7 @@ int smm_apply_levels_host(const smm_handle *hc, int32_t n_sel, const int32_t *le
                                  specs.push_back(JobSpec{level_index[i],
                                                          static_cast<const char *>(dx) + static_cast<size_t>(i) * n_src * sx,
                                                          static_cast<char *>(dy) + static_cast<size_t>(i) * n_dst * sy,
-                                                         masked ? (masked[i] ? 1 : 0) : 0});
+                                                         masked ? (masked[i] ? 1 : 0) : 0, static_cast<int64_t>(i) * n_src});
                              return launch_jobs(h, specs, x_dtype, y_dtype, nb, static_cast<int64_t>(n_sel) * n_src,
                                                 static_cast<int64_t>(n_sel) * n_dst, remap_area_min, opt, st);
                          });

@@ -1,6 +1,8 @@
-// smm_aux_kernels.cuh -- the two init-time kernels (included by smm_api.cu only):
+// smm_aux_kernels.cuh -- the kernels outside the weight application (included by smm_api.cu only):
 //   mask_sum_kernel       mask_tensordot (weights.py:47-52): sequential ascending-src sum per row.
 //   nan_variation_kernel  detect_nan_variation_dims (util.py:57-85) for one axis.
+//   widen16_kernel        exact float16 / bfloat16 -> float32 copy of a slab (the float32 path of
+//                         half sources whose 2-byte rows cannot be staged).
 #pragma once
 #include <cuda_runtime.h>
 
@@ -49,6 +51,22 @@ __global__ void nan_variation_kernel(const TX *__restrict__ x, int64_t outer, in
     }
     const unsigned n = __popc(__ballot_sync(0xffffffffu, varies));
     if ((threadIdx.x & 31) == 0 && n) atomicAdd(count, static_cast<unsigned long long>(n));
+}
+
+// y[b][i] = x[b][i] widened exactly to float32, i < n, b < blockIdx.y's rows (one grid row per batch row).
+template <bool BF16>
+__global__ void widen16_kernel(const uint16_t *__restrict__ x, int64_t ldx, int64_t n, float *__restrict__ y, int64_t ldy)
+{
+    const uint16_t *xr = x + static_cast<int64_t>(blockIdx.y) * ldx;
+    float *yr = y + static_cast<int64_t>(blockIdx.y) * ldy;
+    for (int64_t i = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x; i < n;
+         i += static_cast<int64_t>(gridDim.x) * blockDim.x) {
+        const uint16_t r = xr[i];
+        float v;
+        if constexpr (BF16) v = __uint_as_float(static_cast<uint32_t>(r) << 16);
+        else asm("cvt.f32.f16 %0, %1;" : "=f"(v) : "h"(r));
+        yr[i] = v;
+    }
 }
 
 }  // namespace smm

@@ -1,0 +1,7 @@
+// smm_inst_bf16_f32.cu -- kernel launchers for x = bfloat16 (float32 semantics), y = float
+// (one translation unit per type pair so that the library builds in parallel; see smm_internal.h).
+#include "smm_launch.cuh"
+
+namespace smm {
+SMM_DECLARE_LAUNCHERS(, BF16, float)
+}  // namespace smm

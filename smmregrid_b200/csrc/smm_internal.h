@@ -1,7 +1,7 @@
 // smm_internal.h -- declarations shared by the translation units of the library (not part of
-// the ABI).  The kernel launchers are templates over the (x, y) element types; each of the eight
-// type pairs (x: float, double, I16F32, I16F64; y: float, double) is instantiated in its own
-// translation unit (smm_inst_*.cu) so the library builds in parallel.
+// the ABI).  The kernel launchers are templates over the (x, y) element types; each of the twelve
+// type pairs (x: float, double, I16F32, I16F64, F16, BF16; y: float, double) is instantiated in its
+// own translation unit (smm_inst_*.cu) so the library builds in parallel.
 #pragma once
 #include <cuda_runtime.h>
 
@@ -57,12 +57,16 @@ struct LevelDev {
 // packed element types (smm_kernels.cuh): raw 16-bit sources decoding to float / double
 struct I16F32;
 struct I16F64;
+// half element types (smm_kernels.cuh): IEEE binary16 / bfloat16 sources with float32 semantics
+struct F16;
+struct BF16;
 
 struct JobSpec {
     int32_t level;
     const void *x;
     void *y;
     int32_t masked;
+    int64_t x_off = 0;      // elements from the caller's x to this level's x (half sources: the float32 model's alignment)
 };
 
 // staged_kernel<TX, TY, lpr, kpl, nct, packed, ord> on `grid` work items

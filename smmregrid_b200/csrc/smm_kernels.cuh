@@ -104,17 +104,60 @@ __device__ __forceinline__ double fill_invalid(double v) { return (fabs(v) <= 1.
 
 // ------------------------------------------------------------------ source element types
 //
-// TX is float, double, or a PACKED type: raw 16-bit CF-packed values (smm_decode) that every read
-// of x decodes to float (I16F32) or double (I16F64).  xs_t<TX> is what x holds in memory (staged,
-// gathered, transposed into XT), xv_t<TX> what the arithmetic sees.  For float / double every
-// helper below is exactly the plain load.
+// TX is float, double, a PACKED type: raw 16-bit CF-packed values (smm_decode) that every read
+// of x decodes to float (I16F32) or double (I16F64), or a HALF type: IEEE binary16 (F16) or
+// bfloat16 (BF16) values, widened exactly on every read.  xs_t<TX> is what x holds in memory
+// (staged, gathered, transposed into XT), xv_t<TX> what the arithmetic sees.  For float / double
+// every helper below is exactly the plain load.
+//
+// Half values have float32 semantics (their float32 widening is exact), but the arithmetic sees
+// them as double: the products are float64 anyway, and binary16 converts straight to float64 in
+// one instruction (cvt.f64.f16) where a detour through float32 costs a second.  What differs from
+// a float32 source is the non-finite fill, which must be float32's 1e20 (fill_x).
 struct I16F32 {};
 struct I16F64 {};
-template <typename TX> struct XElem { using S = TX; using V = TX; static constexpr bool kPacked = false; };
-template <> struct XElem<I16F32> { using S = uint16_t; using V = float; static constexpr bool kPacked = true; };
-template <> struct XElem<I16F64> { using S = uint16_t; using V = double; static constexpr bool kPacked = true; };
+struct F16 {};
+struct BF16 {};
+template <typename TX> struct XElem {
+    using S = TX; using V = TX; static constexpr bool kPacked = false; static constexpr bool kHalf = false;
+};
+template <> struct XElem<I16F32> {
+    using S = uint16_t; using V = float; static constexpr bool kPacked = true; static constexpr bool kHalf = false;
+};
+template <> struct XElem<I16F64> {
+    using S = uint16_t; using V = double; static constexpr bool kPacked = true; static constexpr bool kHalf = false;
+};
+template <> struct XElem<F16> {
+    using S = uint16_t; using V = double; static constexpr bool kPacked = false; static constexpr bool kHalf = true;
+};
+template <> struct XElem<BF16> {
+    using S = uint16_t; using V = double; static constexpr bool kPacked = false; static constexpr bool kHalf = true;
+};
 template <typename TX> using xs_t = typename XElem<TX>::S;
 template <typename TX> using xv_t = typename XElem<TX>::V;
+
+// Exact widening of a half value (no ftz: subnormals keep their value).  binary16: one F2F.F64.F16;
+// bfloat16: its bits are the high half of the float32 with the same value.
+template <typename TX>
+__device__ __forceinline__ double widen16(uint16_t r)
+{
+    if constexpr (cuda::std::is_same<TX, F16>::value) {
+        double v;
+        asm("cvt.f64.f16 %0, %1;" : "=d"(v) : "h"(r));
+        return v;
+    } else {
+        return static_cast<double>(__uint_as_float(static_cast<uint32_t>(r) << 16));
+    }
+}
+
+// the 1e20 fill of a source value in the arithmetic's type: half sources fill as float32 does
+// (1e20f = 1.00000002004e20, not the float64 1e20)
+template <typename TX>
+__device__ __forceinline__ xv_t<TX> fill_x(xv_t<TX> v)
+{
+    if constexpr (XElem<TX>::kHalf) return (fabs(v) <= 1.7976931348623157e+308) ? v : static_cast<double>(1e20f);
+    else return fill_invalid(v);
+}
 
 // CF decode of one raw value (see Decode): fill values -> NaN, else (v * scale) + offset in V, each
 // operation rounded once (no FMA contraction), as numpy does it in the decoded dtype.
@@ -136,12 +179,16 @@ __device__ __forceinline__ V decode16(uint32_t r, const Decode &d)
 
 // plain (generic) read of one source element; packed types pass their Decode
 template <typename TX>
-__device__ __forceinline__ xv_t<TX> ldx_g(const xs_t<TX> *p) { return *p; }
+__device__ __forceinline__ xv_t<TX> ldx_g(const xs_t<TX> *p)
+{
+    if constexpr (XElem<TX>::kHalf) return widen16<TX>(*p);
+    else return *p;
+}
 template <typename TX>
 __device__ __forceinline__ xv_t<TX> ldx_g(const xs_t<TX> *p, const Decode &d)
 {
     if constexpr (XElem<TX>::kPacked) return decode16<xv_t<TX>>(*p, d);
-    else return *p;
+    else return ldx_g<TX>(p);
 }
 
 // Gather load of one source element, with the smallest L2 prefetch-size hint (SASS LDG.E.LTC64B):
@@ -189,11 +236,12 @@ template <> __device__ __forceinline__ uint16_t ld_nc<uint16_t>(const uint16_t *
 #endif
 }
 
-// gather read of one source element, decoded for packed types
+// gather read of one source element, decoded for packed types, widened for half types
 template <typename TX>
 __device__ __forceinline__ xv_t<TX> ld_nc_x(const xs_t<TX> *p, const Decode &d)
 {
     if constexpr (XElem<TX>::kPacked) return decode16<xv_t<TX>>(ld_nc(p), d);
+    else if constexpr (XElem<TX>::kHalf) return widen16<TX>(ld_nc(p));
     else return ld_nc(p);
 }
 
@@ -209,7 +257,7 @@ __device__ __noinline__ double replay_row(const int32_t *__restrict__ rowptr,
     double acc = 0.0;
     const int j1 = rowptr[row + 1];
     for (int j = rowptr[row]; j < j1; ++j) {
-        const xv_t<TX> v = fill_invalid(ldx_g<TX>(xrow + col[j], d...));
+        const xv_t<TX> v = fill_x<TX>(ldx_g<TX>(xrow + col[j], d...));
         acc = __dadd_rn(acc, __dmul_rn(static_cast<double>(v), val[j]));
     }
     return acc;
@@ -290,24 +338,42 @@ template <> __device__ __forceinline__ uint16_t lds<uint16_t>(uint32_t addr)
     asm volatile("ld.shared.u16 %0, [%1];" : "=h"(v) : "r"(addr));
     return v;
 }
-// an already loaded source element, decoded for packed types
+// an already loaded source element, decoded for packed types, widened for half types -- binary16
+// through float32 here (one HADD2.F32 more than F2F.F64.F16): the value stays in one register until
+// its product.  Used where registers are short: the compact path's pass 2 (40 registers) and the
+// reference-order lane chains (16-link lanes), both of which spill with the double at the load.
 template <typename TX>
-__device__ __forceinline__ xv_t<TX> ldx_v(xs_t<TX> v) { return v; }
+__device__ __forceinline__ xv_t<TX> ldx_v(xs_t<TX> v)
+{
+    if constexpr (cuda::std::is_same<TX, F16>::value) {
+        float f;
+        asm("cvt.f32.f16 %0, %1;" : "=f"(f) : "h"(v));
+        return static_cast<double>(f);
+    } else if constexpr (XElem<TX>::kHalf) {
+        return widen16<TX>(v);
+    } else {
+        return v;
+    }
+}
 template <typename TX>
 __device__ __forceinline__ xv_t<TX> ldx_v(xs_t<TX> v, const Decode &d)
 {
     if constexpr (XElem<TX>::kPacked) return decode16<xv_t<TX>>(v, d);
-    else return v;
+    else return ldx_v<TX>(v);
 }
 
-// shared-memory read of one staged source element, decoded for packed types
+// shared-memory read of one staged source element, decoded for packed types, widened for half types
 template <typename TX>
-__device__ __forceinline__ xv_t<TX> ldx_s(uint32_t addr) { return lds<TX>(addr); }
+__device__ __forceinline__ xv_t<TX> ldx_s(uint32_t addr)
+{
+    if constexpr (XElem<TX>::kHalf) return widen16<TX>(lds<uint16_t>(addr));
+    else return lds<TX>(addr);
+}
 template <typename TX>
 __device__ __forceinline__ xv_t<TX> ldx_s(uint32_t addr, const Decode &d)
 {
     if constexpr (XElem<TX>::kPacked) return decode16<xv_t<TX>>(lds<uint16_t>(addr), d);
-    else return lds<TX>(addr);
+    else return ldx_s<TX>(addr);
 }
 
 // Sum of one lane's register-resident links against the staged footprint at shared address
@@ -341,7 +407,7 @@ __device__ __forceinline__ double lane_sum(uint32_t sb, const uint32_t (&off)[KP
     for (int k = 0; k < KPL; k += 2) {
         xv_t<TX> v0 = ldx_s<TX>(sb + off[k + 0], d);
         xv_t<TX> v1 = ldx_s<TX>(sb + off[k + 1], d);
-        if (kFill) { v0 = fill_invalid(v0); v1 = fill_invalid(v1); }
+        if (kFill) { v0 = fill_x<TX>(v0); v1 = fill_x<TX>(v1); }
         acc[k % 4 + 0] = fma(static_cast<double>(v0), w[k + 0], acc[k % 4 + 0]);
         acc[k % 4 + 1] = fma(static_cast<double>(v1), w[k + 1], acc[k % 4 + 1]);
     }
@@ -359,7 +425,7 @@ __device__ __forceinline__ void lane_sum4(uint32_t sb, const uint32_t (&off)[16]
         xv_t<TX> v1 = ldx_s<TX>(sb + off[4 * u + 1], d);
         xv_t<TX> v2 = ldx_s<TX>(sb + off[4 * u + 2], d);
         xv_t<TX> v3 = ldx_s<TX>(sb + off[4 * u + 3], d);
-        if (kFill) { v0 = fill_invalid(v0); v1 = fill_invalid(v1); v2 = fill_invalid(v2); v3 = fill_invalid(v3); }
+        if (kFill) { v0 = fill_x<TX>(v0); v1 = fill_x<TX>(v1); v2 = fill_x<TX>(v2); v3 = fill_x<TX>(v3); }
         const double e = fma(static_cast<double>(v1), w[4 * u + 1], static_cast<double>(v0) * w[4 * u + 0]);
         const double o = fma(static_cast<double>(v3), w[4 * u + 3], static_cast<double>(v2) * w[4 * u + 2]);
         s4[u] = e + o;
@@ -376,8 +442,12 @@ __device__ __forceinline__ void lane_products(uint32_t sb, const uint32_t (&off)
 {
 #pragma unroll
     for (int k = 0; k < KPL; ++k) {
-        xv_t<TX> v = ldx_s<TX>(sb + off[k], d);
-        if (kFill) v = fill_invalid(v);
+        // half sources: ldx_v, which keeps a float16 value in 32 bits until its product (with the
+        // double at the load, the 16-link lanes of these chains spill where float32's do not)
+        xv_t<TX> v;
+        if constexpr (XElem<TX>::kHalf) v = ldx_v<TX>(lds<uint16_t>(sb + off[k]));
+        else v = ldx_s<TX>(sb + off[k], d);
+        if (kFill) v = fill_x<TX>(v);
         p[k] = __dmul_rn(static_cast<double>(v), w[k]);
     }
 }
@@ -428,7 +498,7 @@ __device__ __forceinline__ void lane_chain4(uint32_t sb, const uint32_t (&off)[1
 #pragma unroll
         for (int j = 0; j < 4; ++j) {
             xv_t<TX> v = ldx_s<TX>(sb + off[4 * u + j], d);
-            if (kFill) v = fill_invalid(v);
+            if (kFill) v = fill_x<TX>(v);
             c = __dadd_rn(c, __dmul_rn(static_cast<double>(v), w[4 * u + j]));
         }
         s4[u] = c;
@@ -452,7 +522,7 @@ __device__ __noinline__ void lane_sum_valid(const double *__restrict__ wplan, co
                            static_cast<uint32_t>(sizeof(xs_t<TX>));
         const xv_t<TX> v = ldx_s<TX>(sb + o, d...);
         wa += wk;
-        if (fill_invalid(v) == v) { wx = fma(static_cast<double>(v), wk, wx); wv += wk; }   // false for NaN, +-inf
+        if (fill_x<TX>(v) == v) { wx = fma(static_cast<double>(v), wk, wx); wv += wk; }   // false for NaN, +-inf
     }
     out3[0] = wx; out3[1] = wv; out3[2] = wa;
 }
@@ -829,7 +899,7 @@ __device__ __forceinline__ void chain_pair(uint32_t wa, uint32_t oa, int K, uint
         const uint32_t o = lds_u32(oa);
         xv_t<TX> v0 = ldx_s<TX>(s0 + o, d);
         xv_t<TX> v1 = ldx_s<TX>(s1 + o, d);
-        if (kFill) { v0 = fill_invalid(v0); v1 = fill_invalid(v1); }
+        if (kFill) { v0 = fill_x<TX>(v0); v1 = fill_x<TX>(v1); }
         a0 = __dadd_rn(a0, __dmul_rn(static_cast<double>(v0), w));
         a1 = __dadd_rn(a1, __dmul_rn(static_cast<double>(v1), w));
     }
@@ -843,7 +913,7 @@ __device__ __forceinline__ double chain_one(uint32_t wa, uint32_t oa, int K, uin
     for (int k = 0; k < K; ++k, wa += R * 8, oa += R * 4) {
         const double w = lds_f64(wa);
         xv_t<TX> v = ldx_s<TX>(s0 + lds_u32(oa), d);
-        if (kFill) v = fill_invalid(v);
+        if (kFill) v = fill_x<TX>(v);
         acc = __dadd_rn(acc, __dmul_rn(static_cast<double>(v), w));
     }
     return acc;
@@ -1085,7 +1155,7 @@ gather_kernel(const __grid_constant__ JobBatch jb, const __grid_constant__ Apply
             for (int t = 0; t < BT; ++t) v[t] = ld_nc_x<TX>(xr[t] + c, a.dec);
 #pragma unroll
             for (int t = 0; t < BT; ++t) {  // renormalising mode keeps raw values: a non-finite sum flags the row
-                const double xv = static_cast<double>(do_fill ? fill_invalid(v[t]) : v[t]);
+                const double xv = static_cast<double>(do_fill ? fill_x<TX>(v[t]) : v[t]);
                 if constexpr (ORD) acc[t] = __dadd_rn(acc[t], __dmul_rn(xv, wv));
                 else acc[t] = fma(xv, wv, acc[t]);
             }
@@ -1109,7 +1179,7 @@ gather_kernel(const __grid_constant__ JobBatch jb, const __grid_constant__ Apply
                             const xv_t<TX> v = ldx_g<TX>(xr[t] + job.col[j], a.dec);
                             const double wj = job.val[j];
                             wa += wj;
-                            if (fill_invalid(v) == v) { wx = fma(static_cast<double>(v), wj, wx); wv += wj; }
+                            if (fill_x<TX>(v) == v) { wx = fma(static_cast<double>(v), wj, wx); wv += wj; }
                         }
                         r = renormalise(wx, wv, wa, a.renorm_min_valid);
                     }
@@ -1266,8 +1336,8 @@ __device__ __noinline__ double2 compact_row_filled(const xs_t<TX> *__restrict__ 
 #pragma unroll
         for (int u = 0; u < 4; ++u) {
             if (j + u < j1) {
-                a0 = __dadd_rn(a0, __dmul_rn(static_cast<double>(fill_invalid(v0[u])), w[u]));
-                a1 = __dadd_rn(a1, __dmul_rn(static_cast<double>(fill_invalid(v1[u])), w[u]));
+                a0 = __dadd_rn(a0, __dmul_rn(static_cast<double>(fill_x<TX>(v0[u])), w[u]));
+                a1 = __dadd_rn(a1, __dmul_rn(static_cast<double>(fill_x<TX>(v1[u])), w[u]));
             }
         }
     }
@@ -1295,7 +1365,7 @@ __device__ __forceinline__ void compact_rows(const xs_t<TX> *__restrict__ xt, in
                 v0 = ldx_v<TX>(lane < bc ? __ldg(src) : XS(0), d);
                 v1 = ldx_v<TX>(lane + 32 < bc ? __ldg(src + 32) : XS(0), d);
             }
-            if (!RAW) { v0 = fill_invalid(v0); v1 = fill_invalid(v1); }
+            if (!RAW) { v0 = fill_x<TX>(v0); v1 = fill_x<TX>(v1); }
             a0 = __dadd_rn(a0, __dmul_rn(static_cast<double>(v0), wj));      // reference order, no FMA
             a1 = __dadd_rn(a1, __dmul_rn(static_cast<double>(v1), wj));
         }

@@ -1,6 +1,6 @@
 // smm_launch.cuh -- definitions of the kernel launchers declared in smm_internal.h.  Included by
-// the eight smm_inst_*.cu translation units only, each of which instantiates one (x, y) type pair
-// (x: float, double, or packed 16-bit decoding to float / double; see XElem).
+// the twelve smm_inst_*.cu translation units only, each of which instantiates one (x, y) type pair
+// (x: float, double, packed 16-bit decoding to float / double, float16 or bfloat16; see XElem).
 #pragma once
 #include <algorithm>
 #include <atomic>

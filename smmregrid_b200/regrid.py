@@ -526,21 +526,18 @@ class Regridder(object):
 
     def _floating(self, data):
         """The reference computes in ``result_type(data, float64 weights)``: integer and bool
-        data are promoted to float64 (they hold no missing values), float16 is widened to
-        float32 before the 1e20 fill."""
+        data are promoted to float64 (they hold no missing values).  float16 and bfloat16 pass
+        unchanged: the kernels widen them to float32 (exactly) as they read them, with float32's
+        1e20 fill, so the results are those of the float32 widening at half its source bytes."""
         if isinstance(data, np.ndarray):
-            if data.dtype in (np.float32, np.float64):
+            if data.dtype in (np.float16, np.float32, np.float64):
                 return data
-            if data.dtype == np.float16:
-                return data.astype(np.float32)
             if data.dtype.kind in "iub":
                 return data.astype(np.float64)
             raise TypeError(f"cannot regrid data of dtype {data.dtype}")
         torch = _torch()
-        if data.dtype in (torch.float32, torch.float64):
+        if data.dtype in (torch.float16, torch.bfloat16, torch.float32, torch.float64):
             return data
-        if data.dtype in (torch.float16, torch.bfloat16):
-            return data.to(torch.float32)
         if not data.dtype.is_floating_point and not data.dtype.is_complex:
             return data.to(torch.float64)
         raise TypeError(f"cannot regrid data of dtype {data.dtype}")
@@ -753,9 +750,15 @@ def _packing_of(da, packing):
 
 def _x_code(torch_dtype) -> int:
     """x_dtype code of the tensor handed to the library (int16: raw CF-packed values, which only
-    ``Regridder._source`` lets through)."""
-    if torch_dtype == _torch().int16:
+    ``Regridder._source`` lets through; float16 / bfloat16: read by the kernels as their float32
+    widening)."""
+    torch = _torch()
+    if torch_dtype == torch.int16:
         return _lib.SMM_I16
+    if torch_dtype == torch.float16:
+        return _lib.SMM_F16
+    if torch_dtype == torch.bfloat16:
+        return _lib.SMM_BF16
     return _np_dtype_code(_np_of(torch_dtype))
 
 
