@@ -485,7 +485,7 @@ int launch_jobs(const smm_handle *h, const std::vector<JobSpec> &specs, int32_t 
 constexpr int64_t kWidenBytes = int64_t{256} << 20;     // float32 rows widened per chunk (launch_widened)
 
 // The float32 path of one half-source level on float32 copies of its rows, widened exactly into a
-// buffer from the handle's pool, up to kWidenBytes at a time (see launch_jobs).
+// buffer from the handle's pool, up to kWidenBytes at a time (see route_jobs).
 int launch_widened(const smm_handle *h, const JobSpec &s, int32_t x_dtype, int32_t y_dtype, int64_t B, int64_t xbs,
                    int64_t ybs, double area_min, const ApplyOpts &opt, cudaStream_t st)
 {
@@ -515,47 +515,39 @@ int launch_widened(const smm_handle *h, const JobSpec &s, int32_t x_dtype, int32
     return rc;
 }
 
-int launch_jobs(const smm_handle *h, const std::vector<JobSpec> &specs, int32_t x_dtype,
-                int32_t y_dtype, int64_t B, int64_t xbs, int64_t ybs, double area_min,
-                const ApplyOpts &opt, cudaStream_t st)
+// shared memory of the link image of ordered-long plans: kpl x nct x (8 + 4) bytes
+size_t image_bytes(const LevelDev &L) { return L.ordlong ? round_up(static_cast<size_t>(L.kpl) * L.nct * 12, 128) : 0; }
+
+// shared memory a staged launch needs for two stages of one batch row each
+size_t two_stage_smem(size_t max_segs, size_t max_elems, size_t image, size_t es)
 {
-    if (B == 0 || specs.empty()) return SMM_OK;
-    const size_t sx = x_elem_bytes(x_dtype);
-    // Half sources get the kernel family float32 data would get: their results are the float32 path's
-    // bit for bit, and the fast sums of the families differ in the last bits.  So every choice of a
-    // family is made with the element size `sd` of the float32 slab of the same B and ldx, at a
-    // 16-byte aligned address (plus the level's offset in the caller's x); stages, rows per stage and
-    // work items, which change no value, are sized with the real 2 bytes.
-    const bool half = is_half(x_dtype);
-    const size_t sd = half ? 4 : sx;
-    const bool ord = h->ref_order;
-    // shared memory a staged launch needs for `nstages` stages of one batch row each (`image` = the
-    // link image of ordered-long plans: kpl x nct x (8 + 4) bytes)
-    auto image_bytes = [](const LevelDev &L) -> size_t {
-        return L.ordlong ? round_up(static_cast<size_t>(L.kpl) * L.nct * 12, 128) : 0;
-    };
-    auto staged_smem = [&](size_t max_segs, size_t max_elems, size_t nstages, size_t image, size_t es) {
-        return kSmemHeader + round_up(max_segs * sizeof(Seg), 128) + image + nstages * round_up(max_elems * es, 128);
-    };
-    std::vector<JobSpec> staged, gather, gather_lists;      // gather_lists: the long rows of split plans
-    std::vector<JobSpec> widened;                           // half sources staged through a float32 copy
+    return kSmemHeader + round_up(max_segs * sizeof(Seg), 128) + image + 2 * round_up(max_elems * es, 128);
+}
+
+// The kernel family that applies one level of a call.
+enum Route { kWidened, kStaged, kCompact, kGather };
+
+// Appends the route of every spec.  Half sources get the kernel family float32 data would get: their
+// results are the float32 path's bit for bit, and the fast sums of the families differ in the last
+// bits.  So every choice of a family is made with the element size `sd` of the float32 slab of the
+// same B and ldx, at a 16-byte aligned address (plus the level's offset in the caller's x); stages,
+// rows per stage and work items, which change no value, are sized with the real 2 bytes.
+int route_jobs(const smm_handle *h, const std::vector<JobSpec> &specs, int32_t x_dtype, int64_t B, int64_t xbs,
+               const ApplyOpts &opt, std::vector<Route> &route)
+{
+    const bool half_x = is_half(x_dtype);
+    const size_t sx = x_elem_bytes(x_dtype), sd = half_x ? 4 : sx;
     for (const JobSpec &s : specs) {
         const LevelDev &L = h->levels[s.level];
-        if (s.masked && !L.has_imask)
-            return fail(SMM_ERR_INVALID, "masked apply but dst_grid_imask was never set for level " +
-                                             std::to_string(s.level));
-        if (area_min > 0.0 && !L.has_frac)
-            return fail(SMM_ERR_INVALID, "remap_area_min > 0 but dst_grid_frac was never set for level " +
-                                             std::to_string(s.level));
         bool ok = L.staged && opt.kernel != SMM_KERNEL_GATHER;
         // the renormalising extension is not implemented for packed-rows and ordered-long plans: gather kernel
         ok = ok && !((L.packed || L.ordlong) && opt.renorm_min_valid >= 0.0);
         // TMA bulk copies need 16-byte aligned rows and lengths
         const bool aligned = (reinterpret_cast<uintptr_t>(s.x) % 16 == 0) && ((xbs * sx) % 16 == 0) &&
                              ((L.n_src * sx) % 16 == 0);
-        ok = ok && (half ? (s.x_off * 4) % 16 == 0 && (xbs * 4) % 16 == 0 && (L.n_src * 4) % 16 == 0 : aligned);
+        ok = ok && (half_x ? (s.x_off * 4) % 16 == 0 && (xbs * 4) % 16 == 0 && (L.n_src * 4) % 16 == 0 : aligned);
         // at least two stages must fit
-        ok = ok && staged_smem(L.max_segs, L.max_elems, 2, image_bytes(L), sd) <= h->smem_optin;
+        ok = ok && two_stage_smem(L.max_segs, L.max_elems, image_bytes(L), sd) <= h->smem_optin;
         if (!ok && opt.kernel == SMM_KERNEL_STAGED)
             return fail(SMM_ERR_INVALID, "staged kernel forced but unavailable for level " +
                                              std::to_string(s.level) + ": " +
@@ -564,176 +556,162 @@ int launch_jobs(const smm_handle *h, const std::vector<JobSpec> &specs, int32_t 
         // a half level that float32 would stage but whose 2-byte rows cannot be (x not 16-byte aligned,
         // ldx or n_src not a multiple of 8) takes the float32 path on widened rows: rows never depend
         // on the batching, so the chunked float32 applies give the float32 results
-        if (ok && !aligned) { widened.push_back(s); continue; }
-        (ok ? staged : gather).push_back(s);
-        if (ok && L.n_gather_rows > 0) gather_lists.push_back(s);
+        if (ok) { route.push_back(aligned ? kStaged : kWidened); continue; }
+        // The two-pass compact path for scattered sources with enough batch rows.  Cost per batch row
+        // in HBM-byte equivalents, calibrated on B200 (C5nn / C5dis, f32 and f64): a random gather
+        // costs ~120 bytes (a 64-byte sector at about half the streaming rate); the two passes move
+        // the slab (at the streaming rate: TMA bulk copies), the touched columns twice-ish and the
+        // links (random 256-byte runs), together ~1.2x the bytes at the streaming rate.  Runs of
+        // fewer than 16 batch values are not worth it.
+        const double gather_cost = static_cast<double>(L.nnz) * 120.0;
+        const double compact_cost = 1.2 * (static_cast<double>(L.n_src) + static_cast<double>(L.touched) +
+                                           static_cast<double>(L.nnz)) * static_cast<double>(sd);
+        bool compact = L.rcol && opt.renorm_min_valid < 0.0 && opt.kernel != SMM_KERNEL_GATHER;
+        if (opt.kernel != SMM_KERNEL_COMPACT) compact = compact && B >= 16 && gather_cost > compact_cost;
+        route.push_back(compact ? kCompact : kGather);
     }
-    for (const JobSpec &s : widened)
-        if (const int rc = launch_widened(h, s, x_dtype, y_dtype, B, xbs, ybs, area_min, opt, st)) return rc;
+    return SMM_OK;
+}
 
-    ApplyArgs a{};
-    a.B = B; a.x_bstride = xbs; a.y_bstride = ybs; a.remap_area_min = area_min;
-    a.renorm_min_valid = opt.renorm_min_valid;
-    a.dec = opt.dec;
+// The job of one level in a grouped launch, `nblocks` blocks of it (the launcher sets its first work item)
+LevelJob level_job(const LevelDev &L, const JobSpec &s, int64_t nblocks)
+{
+    LevelJob j{};
+    j.nblocks = static_cast<int32_t>(nblocks);
+    j.tiles = L.tiles; j.segs = L.segs; j.wplan = L.wplan; j.iplan = L.iplan; j.rowmap = L.rowmap;
+    j.rowptr = L.rowptr; j.col = L.col; j.val = L.val;
+    j.imask = L.imask; j.frac = L.frac;
+    j.x = s.x; j.y = s.y; j.masked = s.masked;
+    return j;
+}
+
+// Shared-memory layout and batch split of a staged launch of `njobs` levels in the plan layout of `L`
+// (the last of them): fills the staged fields of `a`, the dynamic shared memory and threads per row.
+int size_staged(const smm_handle *h, const LevelDev &L, size_t max_segs, size_t max_elems, int64_t tiles,
+                size_t njobs, size_t sx, size_t sy, ApplyArgs &a, size_t &smem, int &tpr)
+{
     const LaunchSettings &ls = launch_settings();
-    a.debug_flags = ls.debug_flags;
+    const size_t segs_off = kSmemHeader + round_up(max_segs * sizeof(Seg), 128);
+    const size_t stage_off = segs_off + image_bytes(L);
+    a.n_src = L.n_src; a.n_dst = L.n_dst;
+    a.ord_k = L.kpl;
+    a.wimg_off = static_cast<uint32_t>(segs_off);
+    a.oimg_off = static_cast<uint32_t>(segs_off + static_cast<size_t>(L.kpl) * L.nct * 8);
+    const size_t row_bytes = std::max<size_t>(128, round_up(max_elems * sx, 128));
+    // stage several batch rows together (up to 8, ~56 KB per stage) so that the per-stage
+    // barrier and loop overhead of the consumers is amortised: C3 2156 -> 2671 GB/s, C2 5565 -> 6111
+    int nb_rows = ls.rows_per_stage > 0 ? ls.rows_per_stage : static_cast<int>((56u << 10) / row_bytes);
+    const size_t smem_half = (228u * 1024u - 2u * 1024u) / 2u - 1024u;   // two CTAs per SM (NCT = 256)
+    {   // ...but never at the price of pipeline depth (>= 4 stages) or of the second CTA per SM
+        const size_t budget = (L.nct == 256 ? smem_half : h->smem_optin) - std::min(stage_off, smem_half);
+        nb_rows = static_cast<int>(std::min<size_t>(nb_rows, std::max<size_t>(1, budget / (4 * row_bytes))));
+    }
+    nb_rows = static_cast<int>(std::max<int64_t>(1, std::min<int64_t>({nb_rows, 8, a.B})));
+    if (L.ordlong) {    // ordered kernel: one CTA per SM, batch rows chained in pairs: an even number of
+                        // rows per stage, as many as leave three stages
+        nb_rows = (a.B >= 2 && stage_off + 4 * row_bytes <= h->smem_optin) ? 2 : 1;
+        while (nb_rows >= 2 && nb_rows + 2 <= 8 && nb_rows + 2 <= a.B &&
+               stage_off + 3 * static_cast<size_t>(nb_rows + 2) * row_bytes <= h->smem_optin)
+            nb_rows += 2;
+    }
+    const size_t stage_bytes = row_bytes * nb_rows;
+    int64_t chunk = 0;             // batch rows per work item: whole stages
+    const double row_bytes_hbm = static_cast<double>(njobs) *
+                                 (static_cast<double>(a.n_src) * sx + static_cast<double>(a.n_dst) * sy);
+    const int ctas_per_sm = (!L.ordlong && L.nct == 256) ? 2 : 1;
+    const int64_t nchunks = pick_chunks(a.B, tiles, static_cast<int64_t>(h->sm_count) * ctas_per_sm,
+                                        row_bytes_hbm, L.ordlong ? 6.0 : (L.nct == 256 ? 2.5 : 4.0), nb_rows, chunk);
+    a.chunk = chunk; a.nchunks = static_cast<int32_t>(nchunks);
+    size_t S = (!L.ordlong && L.nct == 256 && smem_half > stage_off) ? (smem_half - stage_off) / stage_bytes : 0;
+    if (S < 3) S = (h->smem_optin - stage_off) / stage_bytes;        // one CTA per SM
+    S = std::min<size_t>(S, kMaxStages);
+    S = std::min<size_t>(S, static_cast<size_t>(ls.max_stages));
+    if (S < 2) return fail(SMM_ERR_INVALID, "internal: staged footprint does not fit");
+    a.nstages = static_cast<int32_t>(S);
+    a.stage_bytes = static_cast<uint32_t>(stage_bytes);
+    a.row_bytes = static_cast<uint32_t>(row_bytes);
+    a.rows_per_stage = nb_rows;
+    a.stage_off = static_cast<uint32_t>(stage_off);
+    smem = stage_off + S * stage_bytes;
+    // two threads per row (one per batch row of a pair) while that leaves at most 8 consumer warps:
+    // C4 (64 rows per tile) 3060 -> 3989 GB/s, C2 (256 rows: 16 warps re-reading the image) 4368 -> 3518
+    tpr = (L.ordlong && nb_rows >= 2 && (ls.ord_tpr == 2 || (ls.ord_tpr == 0 && L.nct <= 128))) ? 2 : 1;
+    return SMM_OK;
+}
 
-    auto fill_job = [&](const JobSpec &s, LevelJob &j) {
-        const LevelDev &L = h->levels[s.level];
-        j.tiles = L.tiles; j.segs = L.segs; j.wplan = L.wplan; j.iplan = L.iplan; j.rowmap = L.rowmap;
-        j.rowptr = L.rowptr; j.col = L.col; j.val = L.val;
-        j.imask = L.imask; j.frac = L.frac;
-        j.x = s.x; j.y = s.y; j.masked = s.masked; j.nrows = 0;
-    };
-
-    // ---- staged launches: up to kMaxJobs levels at a time (balanced when there are more), and a
-    // group is closed early when the segment table of one level and the footprint of another would
-    // not fit two stages TOGETHER (each level fits on its own, see above)
-    const size_t staged_groups = (staged.size() + kMaxJobs - 1) / kMaxJobs;
-    const size_t staged_per = staged_groups ? (staged.size() + staged_groups - 1) / staged_groups : 1;   // balanced
+// Staged launches: up to kMaxJobs levels at a time (balanced when there are more), and a group is
+// closed early when the segment table of one level and the footprint of another would not fit two
+// stages TOGETHER (each level fits on its own, see route_jobs).
+int launch_staged(const smm_handle *h, const std::vector<JobSpec> &staged, int32_t x_dtype, int32_t y_dtype,
+                  const ApplyOpts &opt, ApplyArgs a, cudaStream_t st)
+{
+    const size_t sx = x_elem_bytes(x_dtype), sy = y_dtype == SMM_F32 ? 4 : 8;
+    const size_t groups = (staged.size() + kMaxJobs - 1) / kMaxJobs;
+    const size_t per_group = groups ? (staged.size() + groups - 1) / groups : 1;   // balanced
     for (size_t g0 = 0; g0 < staged.size();) {
-        size_t g1 = g0;
         JobBatch jb{};
-        int64_t tiles_total = 0;
-        size_t max_segs = 0, max_elems = 0;
-        int lpr = 0, kpl = 0, nct = 256;
-        bool packed = false, ordl = false;
-        size_t image = 0;
-        for (; g1 < staged.size() && g1 - g0 < staged_per; ++g1) {
+        int64_t tiles = 0, max_tiles = 0;
+        size_t max_segs = 0, max_elems = 0, g1 = g0;
+        for (; g1 < staged.size() && g1 - g0 < per_group; ++g1) {
             const LevelDev &L = h->levels[staged[g1].level];
             const size_t ms = std::max<size_t>(max_segs, L.max_segs), me = std::max<size_t>(max_elems, L.max_elems);
-            if (g1 > g0 && staged_smem(ms, me, 2, image_bytes(L), sx) > h->smem_optin) break;
+            if (g1 > g0 && two_stage_smem(ms, me, image_bytes(L), sx) > h->smem_optin) break;
             max_segs = ms; max_elems = me;
-            tiles_total += L.ntiles;
-            lpr = L.lpr; kpl = L.kpl; nct = L.nct; packed = L.packed; ordl = L.ordlong;
-            image = image_bytes(L);
-            a.n_src = L.n_src; a.n_dst = L.n_dst;
+            tiles += L.ntiles;
+            max_tiles = std::max<int64_t>(max_tiles, L.ntiles);
+            jb.jobs[g1 - g0] = level_job(L, staged[g1], L.ntiles);
         }
-        const size_t segs_off = kSmemHeader + round_up(max_segs * sizeof(Seg), 128);
-        const size_t stage_off = segs_off + image;
-        a.ord_k = kpl;
-        a.wimg_off = static_cast<uint32_t>(segs_off);
-        a.oimg_off = static_cast<uint32_t>(segs_off + static_cast<size_t>(kpl) * nct * 8);
-        const size_t row_bytes = std::max<size_t>(128, round_up(max_elems * sx, 128));
-        // stage several batch rows together (up to 8, ~56 KB per stage) so that the per-stage
-        // barrier and loop overhead of the consumers is amortised: C3 2156 -> 2671 GB/s, C2 5565 -> 6111
-        int nb_rows = ls.rows_per_stage > 0 ? ls.rows_per_stage : static_cast<int>((56u << 10) / row_bytes);
-        const size_t half = (228u * 1024u - 2u * 1024u) / 2u - 1024u;   // two CTAs per SM (NCT = 256)
-        {   // ...but never at the price of pipeline depth (>= 4 stages) or of the second CTA per SM
-            const size_t budget = (nct == 256 ? half : h->smem_optin) - std::min(stage_off, half);
-            nb_rows = static_cast<int>(std::min<size_t>(nb_rows, std::max<size_t>(1, budget / (4 * row_bytes))));
-        }
-        nb_rows = static_cast<int>(std::max<int64_t>(1, std::min<int64_t>({nb_rows, 8, B})));
-        if (ordl) {     // ordered kernel: one CTA per SM, batch rows chained in pairs: an even number of rows
-                        // per stage, as many as leave three stages
-            nb_rows = (B >= 2 && stage_off + 4 * row_bytes <= h->smem_optin) ? 2 : 1;
-            while (nb_rows >= 2 && nb_rows + 2 <= 8 && nb_rows + 2 <= B &&
-                   stage_off + 3 * static_cast<size_t>(nb_rows + 2) * row_bytes <= h->smem_optin)
-                nb_rows += 2;
-        }
-        const size_t stage_bytes = row_bytes * nb_rows;
-        int64_t chunk = 0;             // batch rows per work item: whole stages
-        const double row_bytes_hbm = static_cast<double>(g1 - g0) *
-                                     (static_cast<double>(a.n_src) * sx + static_cast<double>(a.n_dst) * (y_dtype == SMM_F32 ? 4 : 8));
-        const int ctas_per_sm = (!ordl && nct == 256) ? 2 : 1;
-        const int64_t nchunks = pick_chunks(B, tiles_total, static_cast<int64_t>(h->sm_count) * ctas_per_sm,
-                                            row_bytes_hbm, ordl ? 6.0 : (nct == 256 ? 2.5 : 4.0), nb_rows, chunk);
-        a.chunk = chunk; a.nchunks = static_cast<int32_t>(nchunks);
-        size_t S = (!ordl && nct == 256 && half > stage_off) ? (half - stage_off) / stage_bytes : 0;
-        if (S < 3) S = (h->smem_optin - stage_off) / stage_bytes;        // one CTA per SM
-        S = std::min<size_t>(S, kMaxStages);
-        S = std::min<size_t>(S, static_cast<size_t>(ls.max_stages));
-        if (S < 2) return fail(SMM_ERR_INVALID, "internal: staged footprint does not fit");
-        a.nstages = static_cast<int32_t>(S);
-        a.stage_bytes = static_cast<uint32_t>(stage_bytes);
-        a.row_bytes = static_cast<uint32_t>(row_bytes);
-        a.rows_per_stage = nb_rows;
-        a.stage_off = static_cast<uint32_t>(stage_off);
-        const size_t smem = stage_off + S * stage_bytes;
+        const LevelDev &L = h->levels[staged[g1 - 1].level];
+        jb.njobs = static_cast<int32_t>(g1 - g0);
+        g0 = g1;
+        size_t smem = 0;
+        int tpr = 1;
+        if (const int rc = size_staged(h, L, max_segs, max_elems, tiles, jb.njobs, sx, sy, a, smem, tpr)) return rc;
+        if (max_tiles == 0) continue;
         // grid: x = tile, y = batch chunk, z = level of the group (blocks beyond a level's tile
         // count exit at once).  No index arithmetic in the kernel: what steers its batch loop stays
         // in uniform registers.
-        int64_t max_tiles = 0;
-        jb.njobs = static_cast<int32_t>(g1 - g0);
-        for (size_t g = g0; g < g1; ++g) {
-            LevelJob &j = jb.jobs[g - g0];
-            fill_job(staged[g], j);
-            j.nblocks = h->levels[staged[g].level].ntiles;
-            j.item0 = 0;
-            max_tiles = std::max<int64_t>(max_tiles, j.nblocks);
-        }
-        g0 = g1;
-        if (max_tiles == 0) continue;
-        const dim3 grid(static_cast<unsigned>(max_tiles), static_cast<unsigned>(nchunks), static_cast<unsigned>(jb.njobs));
-        // two threads per row (one per batch row of a pair) while that leaves at most 8 consumer warps:
-        // C4 (64 rows per tile) 3060 -> 3989 GB/s, C2 (256 rows: 16 warps re-reading the image) 4368 -> 3518
-        const int tpr = (ordl && nb_rows >= 2 && (ls.ord_tpr == 2 || (ls.ord_tpr == 0 && nct <= 128))) ? 2 : 1;
-        const int rc = ordl ? SMM_DTYPE_DISPATCH(launch_ordered_t, h->device, nct, tpr, grid, smem, st, jb, a)
-                            : SMM_DTYPE_DISPATCH(launch_staged_t, h->device, lpr, kpl, nct, packed, ord, grid, smem, st, jb, a);
+        const dim3 grid(static_cast<unsigned>(max_tiles), static_cast<unsigned>(a.nchunks), static_cast<unsigned>(jb.njobs));
+        const int rc = L.ordlong ? SMM_DTYPE_DISPATCH(launch_ordered_t, h->device, L.nct, tpr, grid, smem, st, jb, a)
+                                 : SMM_DTYPE_DISPATCH(launch_staged_t, h->device, L.lpr, L.kpl, L.nct, L.packed,
+                                                      h->ref_order, grid, smem, st, jb, a);
         if (rc) return rc;
     }
+    return SMM_OK;
+}
 
-    // ---- compact (two-pass) launches: scattered sources with enough batch rows, one level at a time
-    {
-        std::vector<JobSpec> plain;
-        for (const JobSpec &sp : gather) {
-            const LevelDev &L = h->levels[sp.level];
-            // Cost per batch row in HBM-byte equivalents, calibrated on B200 (C5nn / C5dis, f32 and
-            // f64): a random gather costs ~120 bytes (a 64-byte sector at about half the streaming
-            // rate); the two passes move the slab (at the streaming rate: TMA bulk copies), the
-            // touched columns twice-ish and the links (random 256-byte runs), together ~1.2x the
-            // bytes at the streaming rate.  Runs of fewer than 16 batch values are not worth it.
-            const double gather_cost = static_cast<double>(L.nnz) * 120.0;
-            const double compact_cost = 1.2 * (static_cast<double>(L.n_src) + static_cast<double>(L.touched) +
-                                               static_cast<double>(L.nnz)) * static_cast<double>(sd);
-            bool use = L.rcol && opt.renorm_min_valid < 0.0 && opt.kernel != SMM_KERNEL_GATHER;
-            if (opt.kernel != SMM_KERNEL_COMPACT) use = use && B >= 16 && gather_cost > compact_cost;
-            if (!use) { plain.push_back(sp); continue; }
-            const int rc = launch_compact(h, L, sp, x_dtype, y_dtype, B, xbs, ybs, area_min, opt, st);
-            if (rc == kCompactUnavailable) { plain.push_back(sp); continue; }
-            if (rc) return rc;
-        }
-        gather.swap(plain);
-    }
-
-    // ---- gather launches: whole levels, then the row lists of split plans
-    for (int pass = 0; pass < 2; ++pass) {
-    const std::vector<JobSpec> &list = pass == 0 ? gather : gather_lists;
-    const bool lists = pass == 1;
-    // reference order: one thread walks a row's links in sequence
-    const int lpr = ord ? 1 : h->gather_lanes[pass];
+// Gather launches of whole levels, or (`lists`) of the long rows of split plans, kMaxJobs levels at a time
+int launch_gather(const smm_handle *h, const std::vector<JobSpec> &list, bool lists, int32_t x_dtype,
+                  int32_t y_dtype, const ApplyOpts &opt, ApplyArgs a, cudaStream_t st)
+{
+    const bool ord = h->ref_order;     // reference order: one thread walks a row's links in sequence
+    const int lpr = ord ? 1 : h->gather_lanes[lists ? 1 : 0];
+    const int rpb = kGatherThreads / lpr;
     for (size_t g0 = 0; g0 < list.size(); g0 += kMaxJobs) {
         const size_t g1 = std::min(list.size(), g0 + kMaxJobs);
         JobBatch jb{};
-        int64_t nnz = 0, rows = 0;
+        jb.njobs = static_cast<int32_t>(g1 - g0);
+        int64_t nnz = 0, rows = 0, blocks_total = 0;
         for (size_t g = g0; g < g1; ++g) {
             const LevelDev &L = h->levels[list[g].level];
+            const int64_t nrows = lists ? L.n_gather_rows : L.n_dst, nblocks = (nrows + rpb - 1) / rpb;
+            LevelJob &j = jb.jobs[g - g0] = level_job(L, list[g], nblocks);
+            if (lists) { j.rowmap = L.gather_rows; j.nrows = L.n_gather_rows; }
             nnz += lists ? L.gather_nnz : L.nnz;
-            rows += lists ? L.n_gather_rows : L.n_dst;
+            rows += nrows;
+            blocks_total += nblocks;
             a.n_src = L.n_src; a.n_dst = L.n_dst;
         }
-        const int rpb = kGatherThreads / lpr;
-        auto rows_of = [&](const LevelDev &L) -> int64_t { return lists ? L.n_gather_rows : L.n_dst; };
-        int64_t blocks_total = 0;
-        for (size_t g = g0; g < g1; ++g)
-            blocks_total += (rows_of(h->levels[list[g].level]) + rpb - 1) / rpb;
         int64_t chunk = 0;
         // gather kernel: up to 8 CTAs of 256 threads per SM, a light prologue, traffic dominated by the gathers
         const double row_bytes_hbm = static_cast<double>(nnz) * 64.0 + static_cast<double>(rows) * (y_dtype == SMM_F32 ? 4 : 8);
-        const int64_t nchunks = pick_chunks(B, blocks_total, static_cast<int64_t>(h->sm_count) * 8, row_bytes_hbm, 1.0,
+        const int64_t nchunks = pick_chunks(a.B, blocks_total, static_cast<int64_t>(h->sm_count) * 8, row_bytes_hbm, 1.0,
                                             kGatherBT, chunk);
         a.chunk = chunk; a.nchunks = static_cast<int32_t>(nchunks);
-        a.nstages = 0; a.stage_bytes = 0; a.stage_off = 0; a.row_bytes = 0; a.rows_per_stage = 1;
         int64_t item = 0;
-        jb.njobs = static_cast<int32_t>(g1 - g0);
-        for (size_t g = g0; g < g1; ++g) {
-            const LevelDev &L = h->levels[list[g].level];
-            LevelJob &j = jb.jobs[g - g0];
-            fill_job(list[g], j);
-            if (lists) { j.rowmap = L.gather_rows; j.nrows = L.n_gather_rows; }
-            j.nblocks = static_cast<int32_t>((rows_of(L) + rpb - 1) / rpb);
-            j.item0 = static_cast<int32_t>(item);
-            item += static_cast<int64_t>(j.nblocks) * nchunks;
+        for (int32_t k = 0; k < jb.njobs; ++k) {
+            jb.jobs[k].item0 = static_cast<int32_t>(item);
+            item += static_cast<int64_t>(jb.jobs[k].nblocks) * nchunks;
         }
         if (item > INT32_MAX) return fail(SMM_ERR_INVALID, "too many work items in one launch");
         if (item == 0) continue;
@@ -741,8 +719,40 @@ int launch_jobs(const smm_handle *h, const std::vector<JobSpec> &specs, int32_t 
         const int rc = SMM_DTYPE_DISPATCH(launch_gather_t, lpr, ord, grid, st, jb, a);
         if (rc) return rc;
     }
-    }
     return SMM_OK;
+}
+
+// One apply of the specs' levels to B batch rows, in this order: widened levels, staged groups,
+// compact levels, gathers of whole levels, gathers of the split plans' row lists.
+int launch_jobs(const smm_handle *h, const std::vector<JobSpec> &specs, int32_t x_dtype,
+                int32_t y_dtype, int64_t B, int64_t xbs, int64_t ybs, double area_min,
+                const ApplyOpts &opt, cudaStream_t st)
+{
+    std::vector<Route> route;
+    if (const int rc = route_jobs(h, specs, x_dtype, B, xbs, opt, route)) return rc;
+    // the specs of one route, or (split plans) the staged ones whose long rows are listed for gathers
+    auto select = [&](Route r, bool lists = false) {
+        std::vector<JobSpec> out;
+        for (size_t i = 0; i < specs.size(); ++i)
+            if (route[i] == r && (!lists || h->levels[specs[i].level].n_gather_rows > 0)) out.push_back(specs[i]);
+        return out;
+    };
+    for (const JobSpec &s : select(kWidened))
+        if (const int rc = launch_widened(h, s, x_dtype, y_dtype, B, xbs, ybs, area_min, opt, st)) return rc;
+    ApplyArgs a{};
+    a.B = B; a.x_bstride = xbs; a.y_bstride = ybs; a.remap_area_min = area_min;
+    a.renorm_min_valid = opt.renorm_min_valid;
+    a.dec = opt.dec;
+    a.debug_flags = launch_settings().debug_flags;
+    if (const int rc = launch_staged(h, select(kStaged), x_dtype, y_dtype, opt, a, st)) return rc;
+    for (size_t i = 0; i < specs.size(); ++i) {
+        if (route[i] != kCompact) continue;
+        const int rc = launch_compact(h, h->levels[specs[i].level], specs[i], x_dtype, y_dtype, B, xbs, ybs, area_min, opt, st);
+        if (rc == kCompactUnavailable) route[i] = kGather;        // the level takes the gather kernel instead
+        else if (rc) return rc;
+    }
+    if (const int rc = launch_gather(h, select(kGather), false, x_dtype, y_dtype, opt, a, st)) return rc;
+    return launch_gather(h, select(kStaged, true), true, x_dtype, y_dtype, opt, a, st);
 }
 
 // true when cudaMemcpyAsync can DMA straight from/to the pointer (pinned or registered)
@@ -803,21 +813,38 @@ void parallel_copy_rows(char *dst, size_t dst_stride, const char *src, size_t sr
     });
 }
 
-int check_dtypes(int32_t x_dtype, int32_t y_dtype)
-{
-    if ((x_dtype != SMM_F32 && x_dtype != SMM_F64 && x_dtype != SMM_I16 && !is_half(x_dtype)) ||
-        (y_dtype != SMM_F32 && y_dtype != SMM_F64))
-        return fail(SMM_ERR_DTYPE, "x_dtype must be SMM_F32 (0), SMM_F64 (1), SMM_I16 (2), SMM_F16 (3) or SMM_BF16 (4), "
-                                   "y_dtype SMM_F32 or SMM_F64");
-    return SMM_OK;
-}
-
 int check_level(const smm_handle *h, int32_t level)
 {
     if (!h) return fail(SMM_ERR_INVALID, "null handle");
     if (level < 0 || level >= static_cast<int32_t>(h->levels.size()))
         return fail(SMM_ERR_INVALID, "level " + std::to_string(level) + " out of range [0, " +
                                          std::to_string(h->levels.size()) + ")");
+    return SMM_OK;
+}
+
+// Checks the four apply entry points share: dtypes, options, B (and n_sel of the grouped calls,
+// which pass it) and remap_area_min.  `empty`: nothing to apply, SMM_OK before any pointer is read.
+int check_apply(int32_t x_dtype, int32_t y_dtype, const smm_apply_opts *opts, int64_t B, const int32_t *n_sel,
+                double area_min, ApplyOpts &opt, bool &empty)
+{
+    if ((x_dtype != SMM_F32 && x_dtype != SMM_F64 && x_dtype != SMM_I16 && !is_half(x_dtype)) ||
+        (y_dtype != SMM_F32 && y_dtype != SMM_F64))
+        return fail(SMM_ERR_DTYPE, "x_dtype must be SMM_F32 (0), SMM_F64 (1), SMM_I16 (2), SMM_F16 (3) or SMM_BF16 (4), "
+                                   "y_dtype SMM_F32 or SMM_F64");
+    if (int rc = resolve_opts(opts, x_dtype, opt)) return rc;
+    if (B < 0 || (n_sel && *n_sel < 0)) return fail(SMM_ERR_INVALID, n_sel ? "n_sel and B must be >= 0" : "B must be >= 0");
+    if ((empty = B == 0 || (n_sel && *n_sel == 0)) || (area_min >= 0.0 && area_min <= 1.0)) return SMM_OK;
+    return fail(SMM_ERR_INVALID, "The remap_area_min provided must be between 0.0 and 1.0");
+}
+
+// A masked apply needs the level's dst_grid_imask, a remap_area_min > 0 its dst_grid_frac.
+int check_dst_arrays(const smm_handle *h, int32_t level, bool masked, double area_min)
+{
+    const LevelDev &L = h->levels[level];
+    if (masked && !L.has_imask)
+        return fail(SMM_ERR_INVALID, "masked apply but dst_grid_imask was never set for level " + std::to_string(level));
+    if (area_min > 0.0 && !L.has_frac)
+        return fail(SMM_ERR_INVALID, "remap_area_min > 0 but dst_grid_frac was never set for level " + std::to_string(level));
     return SMM_OK;
 }
 
@@ -1175,18 +1202,14 @@ int smm_apply(const smm_handle *h, int32_t level, const void *x, int32_t x_dtype
               int64_t ldx, void *y, int32_t y_dtype, int64_t ldy, int32_t masked,
               double remap_area_min, const smm_apply_opts *opts, smm_stream_t stream)
 {
-    int rc = check_level(h, level);
-    if (rc) return rc;
-    if ((rc = check_dtypes(x_dtype, y_dtype))) return rc;
     ApplyOpts opt;
-    if ((rc = resolve_opts(opts, x_dtype, opt))) return rc;
-    if (B < 0) return fail(SMM_ERR_INVALID, "B must be >= 0");
-    if (B == 0) return SMM_OK;
+    bool empty;
+    int rc = check_level(h, level);
+    if (rc || (rc = check_apply(x_dtype, y_dtype, opts, B, nullptr, remap_area_min, opt, empty)) || empty) return rc;
     const LevelDev &L = h->levels[level];
     if (!x || !y) return fail(SMM_ERR_INVALID, "null x or y");
     if (ldx < L.n_src || ldy < L.n_dst) return fail(SMM_ERR_INVALID, "ldx < n_src or ldy < n_dst");
-    if (!(remap_area_min >= 0.0 && remap_area_min <= 1.0))
-        return fail(SMM_ERR_INVALID, "The remap_area_min provided must be between 0.0 and 1.0");
+    if ((rc = check_dst_arrays(h, level, masked, remap_area_min))) return rc;
     DeviceGuard g(h->device);
     std::vector<JobSpec> specs{JobSpec{level, x, y, masked ? 1 : 0}};
     return launch_jobs(h, specs, x_dtype, y_dtype, B, ldx, ldy, remap_area_min, opt,
@@ -1200,26 +1223,22 @@ int smm_apply_levels(const smm_handle *h, int32_t n_sel, const int32_t *level_in
                      smm_stream_t stream)
 {
     if (!h) return fail(SMM_ERR_INVALID, "null handle");
-    int rc;
-    if ((rc = check_dtypes(x_dtype, y_dtype))) return rc;
     ApplyOpts opt;
-    if ((rc = resolve_opts(opts, x_dtype, opt))) return rc;
-    if (n_sel < 0 || B < 0) return fail(SMM_ERR_INVALID, "n_sel and B must be >= 0");
-    if (n_sel == 0 || B == 0) return SMM_OK;
+    bool empty;
+    int rc = check_apply(x_dtype, y_dtype, opts, B, &n_sel, remap_area_min, opt, empty);
+    if (rc || empty) return rc;
     if (!level_index || !x || !y) return fail(SMM_ERR_INVALID, "null level_index, x or y");
-    if (!(remap_area_min >= 0.0 && remap_area_min <= 1.0))
-        return fail(SMM_ERR_INVALID, "The remap_area_min provided must be between 0.0 and 1.0");
     const size_t sx = x_elem_bytes(x_dtype), sy = y_dtype == SMM_F32 ? 4 : 8;
     std::vector<JobSpec> specs;
     specs.reserve(static_cast<size_t>(n_sel));
     for (int32_t i = 0; i < n_sel; ++i) {
-        if ((rc = check_level(h, level_index[i]))) return rc;
         JobSpec s;
         s.level = level_index[i];
         s.x = static_cast<const char *>(x) + static_cast<int64_t>(i) * x_level_stride * static_cast<int64_t>(sx);
         s.y = static_cast<char *>(y) + static_cast<int64_t>(i) * y_level_stride * static_cast<int64_t>(sy);
         s.masked = masked ? (masked[i] ? 1 : 0) : 0;
         s.x_off = static_cast<int64_t>(i) * x_level_stride;
+        if ((rc = check_level(h, s.level)) || (rc = check_dst_arrays(h, s.level, s.masked, remap_area_min))) return rc;
         specs.push_back(s);
     }
     DeviceGuard g(h->device);
@@ -1231,19 +1250,15 @@ int smm_apply_host(const smm_handle *hc, int32_t level, const void *x, int32_t x
                    int64_t ldx, void *y, int32_t y_dtype, int64_t ldy, int32_t masked,
                    double remap_area_min, const smm_apply_opts *opts, int64_t chunk_rows)
 {
-    int rc = check_level(hc, level);
-    if (rc) return rc;
-    if ((rc = check_dtypes(x_dtype, y_dtype))) return rc;
     ApplyOpts opt;
-    if ((rc = resolve_opts(opts, x_dtype, opt))) return rc;
-    if (B < 0) return fail(SMM_ERR_INVALID, "B must be >= 0");
-    if (B == 0) return SMM_OK;
+    bool empty;
+    int rc = check_level(hc, level);
+    if (rc || (rc = check_apply(x_dtype, y_dtype, opts, B, nullptr, remap_area_min, opt, empty)) || empty) return rc;
     if (!x || !y) return fail(SMM_ERR_INVALID, "null x or y");
-    if (!(remap_area_min >= 0.0 && remap_area_min <= 1.0))
-        return fail(SMM_ERR_INVALID, "The remap_area_min provided must be between 0.0 and 1.0");
     smm_handle *h = const_cast<smm_handle *>(hc);
     const LevelDev &L = h->levels[level];
     if (ldx < L.n_src || ldy < L.n_dst) return fail(SMM_ERR_INVALID, "ldx < n_src or ldy < n_dst");
+    if ((rc = check_dst_arrays(h, level, masked, remap_area_min))) return rc;
     const size_t sx = x_elem_bytes(x_dtype), sy = y_dtype == SMM_F32 ? 4 : 8;
     return host_pipeline(h, x, L.n_src * sx, ldx * sx, y, L.n_dst * sy, ldy * sy, B, chunk_rows,
                          [&](void *dx, void *dy, int64_t nb, cudaStream_t st) -> int {
@@ -1257,17 +1272,14 @@ int smm_apply_levels_host(const smm_handle *hc, int32_t n_sel, const int32_t *le
                           double remap_area_min, const smm_apply_opts *opts, int64_t chunk_rows)
 {
     if (!hc) return fail(SMM_ERR_INVALID, "null handle");
-    int rc;
-    if ((rc = check_dtypes(x_dtype, y_dtype))) return rc;
     ApplyOpts opt;
-    if ((rc = resolve_opts(opts, x_dtype, opt))) return rc;
-    if (n_sel < 0 || B < 0) return fail(SMM_ERR_INVALID, "n_sel and B must be >= 0");
-    if (n_sel == 0 || B == 0) return SMM_OK;
+    bool empty;
+    int rc = check_apply(x_dtype, y_dtype, opts, B, &n_sel, remap_area_min, opt, empty);
+    if (rc || empty) return rc;
     if (!level_index || !x || !y) return fail(SMM_ERR_INVALID, "null level_index, x or y");
-    if (!(remap_area_min >= 0.0 && remap_area_min <= 1.0))
-        return fail(SMM_ERR_INVALID, "The remap_area_min provided must be between 0.0 and 1.0");
     for (int32_t i = 0; i < n_sel; ++i)
-        if ((rc = check_level(hc, level_index[i]))) return rc;
+        if ((rc = check_level(hc, level_index[i])) || (rc = check_dst_arrays(hc, level_index[i], masked && masked[i], remap_area_min)))
+            return rc;
     smm_handle *h = const_cast<smm_handle *>(hc);
     const int64_t n_src = h->levels[0].n_src, n_dst = h->levels[0].n_dst;
     const size_t sx = x_elem_bytes(x_dtype), sy = y_dtype == SMM_F32 ? 4 : 8;

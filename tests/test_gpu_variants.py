@@ -139,7 +139,7 @@ assert len(BY_ID) == len(VARIANTS)
 
 
 def ordered_threads_per_row(R, B, tpr_env):
-    """What launch_jobs picks for an ordered-kernel plan of R rows per tile (two batch rows per
+    """What size_staged picks for an ordered-kernel plan of R rows per tile (two batch rows per
     stage fit whenever B >= 2 for these operators)."""
     return 2 if B >= 2 and (tpr_env == 2 or (tpr_env == 0 and R <= 128)) else 1
 
